@@ -230,12 +230,13 @@ def run_ours(args):
         return ops[name]()
 
     def step(marks=None):
-        """One pass of the hot path, device-resident."""
+        """One pass of the hot path, device-resident. Returns the DCN output and gradients (the FAC results land in
+        out_f, gi_f, gk_f)."""
         def mark():
             if marks is not None:
                 e = ev(); e.record(); marks.append(e)
         mark()
-        run("dcn_fwd")
+        out_d = run("dcn_fwd")
         mark()
         grads = run("dcn_bwd")
         # data-parallel weight-gradient all-reduce (the only collective on the path): ONE flat bucket, issued
@@ -253,6 +254,7 @@ def run_ours(args):
         elif pending is not None:
             pending.wait()
         mark()
+        return out_d, grads
 
     for _ in range(args.warmup):
         step()
@@ -273,12 +275,16 @@ def run_ours(args):
     with ClockSampler(local, _gpu_uuid(torch, dev)) as clk:
         t0.record()
         for _ in range(args.steps):
-            step(marks)
+            out_d, grads_d = step(marks)
         t1.record()
         torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, dict(
+            zip(["dcn_out", "dcn_grad_input", "dcn_grad_offset", "dcn_grad_mask", "dcn_grad_weight", "dcn_grad_bias",
+                 "fac_out", "fac_grad_input", "fac_grad_kernel"], [out_d, *grads_d, out_f, gi_f, gk_f])))
     ms_total = t0.elapsed_time(t1)
     if world > 1:
         tt = torch.tensor([ms_total], device=dev)
@@ -530,6 +536,23 @@ def run_ours(args):
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_ELEMENTS = 1 << 21       # 8 MB of float32 per array; the nine arrays of a step stay under 64 MB
+
+
+def dump_outputs(torch, out_dir, arrays):
+    """--dump-outputs: write each array as out_dir/<name>.npy in float32, flattened. An array of more than
+    DUMP_MAX_ELEMENTS elements is written as its values at DUMP_MAX_ELEMENTS positions drawn from a fixed seed, so
+    two runs (or two builds) with the same arguments can be compared element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        flat = t.detach().reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMENTS:
+            idx = torch.randint(0, flat.numel(), (DUMP_MAX_ELEMENTS,), generator=torch.Generator().manual_seed(0))
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), flat.float().cpu().numpy())
 
 
 def widening_numbers(torch, dev, d, timed):
@@ -786,7 +809,14 @@ def main():
     ap.add_argument("--no-model", action="store_true", help="skip the full-model legs (BASELINE configs[3], configs[4])")
     ap.add_argument("--kernels-only", action="store_true",
                     help="profiling runs: skip the e2e, cold-breakdown and CPU-baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the DCN and FAC outputs and gradients of the last timed step to DIR/<name>.npy "
+                         "(float32; arrays over 2M elements as a fixed seeded sample of 2M elements)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs: it needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         # torchrun exports OMP_NUM_THREADS=1; the reference arm uses all the host threads it can

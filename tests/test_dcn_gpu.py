@@ -1,5 +1,5 @@
 """GPU parity of DCNv2: CUDA path (through the C ABI / autograd Function) vs the CPU oracle, the
-reference-generated golden vectors and the reference's own CUDA kernels (oracle/_ref/dcn_cuda).
+reference-generated golden vectors and the stored results of the reference's own CUDA kernels (tests/golden/ref_dcn_*).
 Gates (BASELINE.json north_star): forward 1e-5, gradients 1e-4, relative to max|ref| per tensor."""
 import numpy as np
 import pytest
@@ -273,32 +273,17 @@ def test_reductions_are_bit_reproducible(dcn):
 
 
 def test_matches_reference_cuda_kernels(dcn):
-    """The reference's own dcn_v2_im2col_cuda.cu kernels compiled unmodified for sm_100a."""
-    from gpu_util import dev, load_ref_ext
-    ref = load_ref_ext("dcn_cuda", "_ext_cuda_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref/dcn_cuda not built (needs /root/reference at build time)")
-    torch.manual_seed(2)
-    B, C, Co, H, W, dg = 2, 64, 64, 40, 40, 8
-    x = torch.randn(B, C, H, W, device=dev())
-    off = 2 * torch.randn(B, 2 * dg * 9, H, W, device=dev())
-    msk = torch.sigmoid(torch.randn(B, dg * 9, H, W, device=dev()))
-    w = (torch.rand(Co, C, 3, 3, device=dev()) * 2 - 1) / 24
-    b = torch.randn(Co, device=dev())
-    go = torch.randn(B, Co, H, W, device=dev())
-    allow = torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cuda.matmul.allow_tf32 = False
-    try:
-        r_out = ref.dcn_v2_forward(x, w, b, off, msk, 3, 3, 1, 1, 1, 1, 1, 1, dg)
-        r_grads = ref.dcn_v2_backward(x, w, b, off, msk, go, 3, 3, 1, 1, 1, 1, 1, 1, dg)
-    finally:
-        torch.backends.cuda.matmul.allow_tf32 = allow
-    ts = [v.clone().requires_grad_() for v in (x, off, msk, w, b)]
-    out = dcn.dcn_v2_conv(*ts, 1, 1, 1, dg)
-    out.backward(go)
-    assert rel_err(out.detach().cpu().numpy(), r_out.cpu().numpy()) < FWD_TOL
-    for name, v, r in zip(GRADS, ts, r_grads):
-        assert rel_err(v.grad.cpu().numpy(), r.cpu().numpy()) < GRAD_TOL, name
+    """The reference's own dcn_v2_im2col_cuda.cu kernels compiled unmodified for sm_100a, through their stored
+    results (tests/golden/ref_dcn_b2_40x40.npz, see make_golden_ref.py)."""
+    from gpu_util import RefGolden, ref_dcn_inputs
+    d = ref_dcn_inputs()
+    ref = RefGolden("ref_dcn_b2_40x40", d)
+    ts = [d[k].clone().requires_grad_() for k in ("x", "off", "msk", "w", "b")]
+    out = dcn.dcn_v2_conv(*ts, 1, 1, 1, 8)
+    out.backward(d["go"])
+    assert ref.rel_err("out", out) < FWD_TOL
+    for name, v in zip(GRADS, ts):
+        assert ref.rel_err(name, v.grad) < GRAD_TOL, name
 
 
 def test_modules_forward_backward(dcn):

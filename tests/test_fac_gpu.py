@@ -1,5 +1,5 @@
 """GPU parity of FAC KernelConv2D: CUDA path (through the C ABI) vs the CPU oracle, the golden
-vectors, and the reference's own CUDA kernels compiled for sm_100a (oracle/_ref/fac_cuda)."""
+vectors, and the stored results of the reference's own CUDA kernels compiled for sm_100a (tests/golden/ref_fac_*)."""
 import os
 
 import numpy as np
@@ -87,26 +87,17 @@ def test_backward_is_bit_reproducible(fac):
 
 
 def test_matches_reference_cuda_kernels(fac):
-    """The reference's own KernelConv2D_kernel.cu, compiled unmodified for sm_100a."""
-    from gpu_util import dev, load_ref_ext
-    ref = load_ref_ext("fac_cuda", "kernelconv2d_cuda")
-    if ref is None:
-        pytest.skip("oracle/_ref/fac_cuda not built (needs /root/reference at build time)")
-    torch.manual_seed(0)
-    for (B, C, K, H, W) in [(2, 4, 5, 64, 64), (1, 3, 3, 30, 22), (1, 2, 5, 19, 21)]:
-        x = torch.randn(B, C, H + K - 1, W + K - 1, device=dev())
-        ker = torch.randn(B, C * K * K, H, W, device=dev())
-        go = torch.randn(B, C, H, W, device=dev())
-        r_out = torch.zeros(B, C, H, W, device=dev())
-        r_gi, r_gk = torch.zeros_like(x), torch.zeros_like(ker)
-        ref.forward(x, ker, K, r_out)
-        ref.backward(x, ker, K, go, r_gi, r_gk)
-        xg, kg = x.clone().requires_grad_(), ker.clone().requires_grad_()
+    """The reference's own KernelConv2D_kernel.cu, compiled unmodified for sm_100a, through its stored results
+    (tests/golden/ref_fac_case*.npz, see make_golden_ref.py)."""
+    from gpu_util import RefGolden, ref_fac_inputs
+    for i, (K, f) in enumerate(ref_fac_inputs()):
+        ref = RefGolden(f"ref_fac_case{i}", f)
+        xg, kg = f["x"].clone().requires_grad_(), f["ker"].clone().requires_grad_()
         out = fac.KernelConv2DFunction.apply(xg, kg, K)
-        out.backward(go)
-        assert torch.equal(out, r_out), "forward uses the reference's tap order: expected bit-equality"
-        assert torch.equal(kg.grad, r_gk), "grad_kernel is one product per element: expected bit-equality"
-        assert rel_err(xg.grad.cpu().numpy(), r_gi.cpu().numpy()) < GRAD_TOL
+        out.backward(f["go"])
+        assert ref.equal("out", out), "forward uses the reference's tap order: expected bit-equality"
+        assert ref.equal("grad_kernel", kg.grad), "grad_kernel is one product per element: expected bit-equality"
+        assert ref.rel_err("grad_input", xg.grad) < GRAD_TOL
 
 
 def test_module_pads_like_the_reference(fac, oracle):

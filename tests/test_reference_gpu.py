@@ -2,7 +2,7 @@
 staged by tools/refmodel.py into the git-ignored baseline/_ref/ebfi_be) executed on the GPU through this repo's `_ext` /
 `kernelconv2d_cuda` shims, bit-compared with the host-side mirrors in ebfi_be_b200.
 (2) Element-wise parity AT THE BENCHMARKED SHAPES (BASELINE configs[0], configs[1], and the 720p FAC of configs[3])
-against the reference's own CUDA kernels compiled unmodified for sm_100a (oracle/_ref/{dcn,fac}_cuda).
+against the stored results of the reference's own CUDA kernels compiled unmodified for sm_100a (tests/golden/ref_*).
 (3) The reference's full model (models/Ours/model_singleframe.py) forward + backward on the shims.
 """
 import os
@@ -13,7 +13,7 @@ import pytest
 import torch
 
 from conftest import FWD_TOL, GRAD_TOL, ROOT
-from gpu_util import dev, load_ref_ext
+from gpu_util import DCN_GEOM, RefGolden, cfg1_inputs, cfg2_inputs, dev
 
 pytestmark = pytest.mark.gpu
 
@@ -105,56 +105,34 @@ def test_reference_fac_wrapper_runs_on_shims_bit_equal_to_mirror(staged):
 
 # ------------------------------------------------------------------ (2) exact benchmark shapes vs the reference CUDA kernels
 def test_cfg1_exact_shape_vs_reference_cuda():
-    """BASELINE configs[0]: DCNv2 3x3 C=64 dg=8 B=1 256x256, same seeded inputs as bench.py."""
-    ref = load_ref_ext("dcn_cuda", "_ext_cuda_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref/dcn_cuda not built")
+    """BASELINE configs[0]: DCNv2 3x3 C=64 dg=8 B=1 256x256, same seeded inputs as bench.py; the reference kernels'
+    results are stored in tests/golden/ref_cfg1_dcn.npz (see make_golden_ref.py)."""
     from ebfi_be_b200.shims import _ext
-    g = torch.Generator(device="cpu").manual_seed(1234)
-    r = lambda *s: torch.randn(*s, generator=g)
-    x, off, msk = r(1, 64, 256, 256), 2 * r(1, 144, 256, 256), torch.sigmoid(r(1, 72, 256, 256))
-    w, b, go = (torch.rand(64, 64, 3, 3, generator=g) * 2 - 1) / 24, r(64), r(1, 64, 256, 256)
-    x, off, msk, w, b, go = (v.to(dev()) for v in (x, off, msk, w, b, go))
-    geom = (3, 3, 1, 1, 1, 1, 1, 1, 8)
-    allow = torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cuda.matmul.allow_tf32 = False          # the reference's GEMMs are fp32 SGEMMs
-    try:
-        o_ref = ref.dcn_v2_forward(x, w, b, off, msk, *geom)
-        g_ref = ref.dcn_v2_backward(x, w, b, off, msk, go, *geom)
-    finally:
-        torch.backends.cuda.matmul.allow_tf32 = allow
-    o = _ext.dcn_v2_forward(x, w, b, off, msk, *geom)
-    gr = _ext.dcn_v2_backward(x, w, b, off, msk, go, *geom)
-    assert trel(o, o_ref) < FWD_TOL
-    for name, a, c in zip(("grad_input", "grad_offset", "grad_mask", "grad_weight", "grad_bias"), gr, g_ref):
-        assert trel(a, c) < GRAD_TOL, name
+    d = cfg1_inputs()
+    ref = RefGolden("ref_cfg1_dcn", d)
+    args = [d[k] for k in ("x", "w", "b", "off", "msk")]
+    o = _ext.dcn_v2_forward(*args, *DCN_GEOM)
+    gr = _ext.dcn_v2_backward(*args, d["go"], *DCN_GEOM)
+    assert ref.rel_err("out", o) < FWD_TOL
+    for name, a in zip(("grad_input", "grad_offset", "grad_mask", "grad_weight", "grad_bias"), gr):
+        assert ref.rel_err(name, a) < GRAD_TOL, name
 
 
 @pytest.mark.parametrize("shape", [(4, 64, 256, 256), (1, 64, 360, 640)], ids=["cfg2_B4_256", "cfg4_720p_half_res"])
-def test_cfg2_exact_shape_vs_reference_cuda(shape):
-    """BASELINE configs[1] (FAC K=5 C=64 B=4 256x256) and the FAC call of the 720p model (configs[3])."""
-    ref = load_ref_ext("fac_cuda", "kernelconv2d_cuda")
-    if ref is None:
-        pytest.skip("oracle/_ref/fac_cuda not built")
+def test_cfg2_exact_shape_vs_reference_cuda(shape, request):
+    """BASELINE configs[1] (FAC K=5 C=64 B=4 256x256) and the FAC call of the 720p model (configs[3]); the reference
+    kernels' results are stored in tests/golden/ref_<id>.npz (see make_golden_ref.py)."""
     from ebfi_be_b200.shims import kernelconv2d_cuda as kc
-    B, C, H, W = shape
-    K = 5
-    g = torch.Generator(device="cpu").manual_seed(1234)
-    xi = torch.randn(B, C, H + 4, W + 4, generator=g).to(dev())
-    ker = (0.1 * torch.randn(B, C * 25, H, W, generator=g)).to(dev())
-    go = torch.randn(B, C, H, W, generator=g).to(dev())
-    out_r, out = torch.zeros(B, C, H, W, device=dev()), torch.empty(B, C, H, W, device=dev())
-    ref.forward(xi, ker, K, out_r)
-    kc.forward(xi, ker, K, out)
-    assert torch.equal(out, out_r)                          # same tap order -> bit-identical
-    gi_r = torch.zeros_like(xi)
-    gk_r = torch.zeros_like(ker)
-    ref.backward(xi, ker, K, go, gi_r, gk_r)
-    gi, gk = torch.empty_like(xi), torch.empty_like(ker)
-    kc.backward(xi, ker, K, go, gi, gk)
-    assert torch.equal(gk, gk_r)
-    del gk, gk_r
-    assert trel(gi, gi_r) < GRAD_TOL
+    f = cfg2_inputs(shape)
+    ref = RefGolden("ref_" + request.node.callspec.id, f)
+    out = torch.empty_like(f["go"])
+    kc.forward(f["xi"], f["ker"], 5, out)
+    assert ref.equal("out", out)                            # same tap order -> bit-identical
+    gi, gk = torch.empty_like(f["xi"]), torch.empty_like(f["ker"])
+    kc.backward(f["xi"], f["ker"], 5, f["go"], gi, gk)
+    assert ref.equal("grad_kernel", gk)
+    del gk
+    assert ref.rel_err("grad_input", gi) < GRAD_TOL
 
 
 # ------------------------------------------------------------------ (3) the reference model on the shims
