@@ -35,6 +35,18 @@
 // Precision: tensors are fp32 at the boundary (like the reference); the conv operands are rounded to bf16
 // for the tensor cores, accumulation and the whole FAC part are fp32. Stated tolerance 1e-2 of max|out|
 // against the fp32/fp64 op sequence; 1e-5 against the same sequence with bf16-rounded conv operands.
+//
+// Backward (ebfi_kpn_fused_backward): the same kernel with BWD = true recomputes the pre-activation P in TMEM
+// through the identical main loop (same operands, same MMA chain -> bit-identical P, so forward and backward take
+// the same LeakyReLU branch everywhere) and replaces the FAC epilogue by its gradient. Thread = (pixel, channel):
+//   gP[c*KK+t, p]  = G[c,p] * Epad[c,p+t] * (P > 0 ? 1 : slope)      written fp32 NCHW = cuDNN's dgrad/wgrad input
+//   gEpad[c, q]   += LeakyReLU(P)[c*KK+t, q-t] * G[c, q-t]            per-warp box in unclamped Epad coordinates
+//   grad_bias      = per-lane running column sums of gP over the CTA's items of a slice
+// gEpad: a warp holds 4 x 8 pixels, i.e. an (4+K-1) x (8+K-1) box of Epad cells, <= 3 per lane. For a fixed tap every
+// cell has at most one source pixel, so its owner lane pulls the value with one shuffle: 3 shuffles per tap, summed
+// in tap order. The boxes go to the workspace (every cell is covered by <= 4 boxes); kpn_gev_collect sums the boxes
+// of a cell in a fixed order and folds the replication border. kpn_bias_collect sums the column partials of the
+// CTAs of a slice in CTA order. No float atomics anywhere: the outputs are bit-reproducible for a given grid.
 #include "common.cuh"
 #include "tma.cuh"
 #include "umma.cuh"
@@ -54,6 +66,8 @@ constexpr int NTHR = NEPI + 64;                  // + 1 TMA producer warp + 1 MM
 constexpr int PART_CH = 32;                      // channels per halo part = two K = 16 MMA steps per tap
 constexpr int PART_BYTES = (PART_CH / 8) * HPIX * 16;
 constexpr int TMEM_COLS = 256;                   // two accumulators at columns 0 and 128
+constexpr int WR = 4;                            // pixel rows per epilogue warp (32 lanes = WR x TW pixels)
+constexpr int BWD_MAX_GRID = 1024;               // backward grid cap: sizes the bias partials without a device query
 
 struct KpnDims {
     int B, Ce, Cin, H, W, K, KK;
@@ -63,6 +77,14 @@ struct KpnDims {
     int npart;                   // Cin / 32 halo parts
     int w_bytes;
     float slope;
+};
+
+// Backward-only operands of the fused kernel (unused by the forward instantiation).
+struct KpnBwdArgs {
+    const float *gout;      // (B, Ce, H, W) dL/dout
+    float *gpre;            // (B, Ce*KK, H, W) dL/dP
+    float *gbox;            // [B][Ce][tiles_y*TH/WR][tiles_x][WR+K-1][TW+K-1] per-warp dL/dEpad boxes
+    float *bias_part;       // [CTA + slice][NEPI/32 warps][KK] column sums of dL/dP
 };
 
 // (ev | fr) NCHW fp32 -> [b][chunk of 8 channels][y][x][8] bf16: one thread per (b, chunk, y, x)
@@ -176,12 +198,138 @@ __device__ __forceinline__ void kpn_epilogue(uint32_t tmem, uint64_t *acc_full, 
     }
 }
 
-// K: FAC kernel size; NPART: halo parts = Cin / 32
-template <int K, int NPART>
+// Backward epilogue of warpgroup G (see the header comment): gP, the warp's dL/dEpad box, bias column sums.
+template <int K, int G>
+__device__ __forceinline__ void kpn_bwd_epilogue(uint32_t tmem, uint64_t *acc_full, uint64_t *acc_free,
+                                                 const float *__restrict__ bias, const float *__restrict__ ev,
+                                                 const KpnBwdArgs &a, const KpnDims &d, int item0, int item1)
+{
+    constexpr int KK = K * K, R = (K - 1) / 2;
+    constexpr int COL0 = (G * KK / 8) * 8, OFF = G * KK - COL0, NLD = (OFF + KK + 7) / 8;
+    constexpr int BH = WR + K - 1, BW = TW + K - 1, BOX = BH * BW, NCELL = (BOX + 31) / 32;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wq = warp & 3;
+    const int p = wq * 32 + lane, py = p / TW, px = p % TW;
+    const uint32_t lane_base = (uint32_t)wq * 32u;
+    const size_t plane = (size_t)d.H * d.W;
+    const int tiles_per_sample = d.tiles_x * d.tiles_y;
+    const int wrows = d.tiles_y * (TH / WR);
+    // owned box cell j = lane + 32 j at (cy, cx): for tap (ky, kx) its source pixel is lane (cy - ky) * TW + (cx - kx)
+    // = cbase[j] - (ky * TW + kx), if that pixel lies in the warp's WR x TW block: bit q of cmask[j]
+    int cbase[NCELL];
+    uint32_t cmask[NCELL];
+#pragma unroll
+    for (int j = 0; j < NCELL; ++j) {
+        const int cy = (lane + 32 * j) / BW, cx = (lane + 32 * j) % BW;
+        cbase[j] = cy * TW + cx;
+        cmask[j] = 0;
+        for (int q = 0; q < KK; ++q) {
+            const int sy = cy - q / K, sx = cx - q % K;
+            if (lane + 32 * j < BOX && sy >= 0 && sy < WR && sx >= 0 && sx < TW) cmask[j] |= 1u << q;
+        }
+    }
+    // the slice's bias column of this warp in shared memory (broadcast reads): registers are the scarce resource
+    // here, the epilogue already holds the Event window, the accumulators and the bias column sums
+    __shared__ float bias_s[4][KK];
+    float bsum[KK];
+    int cur_slice = -1;
+    auto flush = [&](int s) {                                // warp column sums -> bias_part[CTA + slice][warp]
+#pragma unroll
+        for (int q = 0; q < KK; ++q) {
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) bsum[q] += __shfl_xor_sync(0xffffffffu, bsum[q], o);
+        }
+        if (lane == 0) {
+            float *dst = a.bias_part + ((size_t)(blockIdx.x + s) * (NEPI / 32) + warp) * KK;
+#pragma unroll
+            for (int q = 0; q < KK; ++q) dst[q] = bsum[q];
+        }
+    };
+    for (int item = item0, n = 0; item < item1; ++item, ++n) {
+        const int s = item / d.ntile, t = item % d.ntile;
+        const int b = t / tiles_per_sample, tt = t % tiles_per_sample;
+        const int tyi = tt / d.tiles_x, txi = tt % d.tiles_x;
+        const int y = tyi * TH + py, x = txi * TW + px;
+        const int c = s * CPS + G;
+        const bool active = c < d.Ce;                        // warp-uniform
+        const bool valid = active && y < d.H && x < d.W;
+        if (s != cur_slice) {
+            if (cur_slice >= 0 && cur_slice * CPS + G < d.Ce) flush(cur_slice);
+            cur_slice = s;
+            if (active) {
+                __syncwarp();
+                if (lane < KK) bias_s[wq][lane] = __ldg(bias + c * KK + lane);
+                __syncwarp();
+#pragma unroll
+                for (int q = 0; q < KK; ++q) bsum[q] = 0.f;
+            }
+        }
+        float e[KK], g = 0.f;
+        if (valid) {
+            const float *evc = ev + ((size_t)b * d.Ce + c) * plane;
+            int xo[K];
+#pragma unroll
+            for (int kx = 0; kx < K; ++kx) xo[kx] = min(max(x + kx - R, 0), d.W - 1);
+#pragma unroll
+            for (int ky = 0; ky < K; ++ky) {
+                const float *row = evc + (size_t)min(max(y + ky - R, 0), d.H - 1) * d.W;
+#pragma unroll
+                for (int kx = 0; kx < K; ++kx) e[ky * K + kx] = __ldg(row + xo[kx]);
+            }
+            g = __ldg(a.gout + ((size_t)b * d.Ce + c) * plane + (size_t)y * d.W + x);
+        }
+        const int buf = n & 1;
+        umma::mbar_wait_warp(&acc_full[buf], (uint32_t)((n >> 1) & 1));
+        umma::fence_after_sync();
+        float v[NLD * 8];
+        if (active) {
+#pragma unroll
+            for (int q = 0; q < NLD; ++q) {
+                float (&vq)[8] = *reinterpret_cast<float (*)[8]>(&v[q * 8]);
+                umma::tmem_ld8(umma::tmem_addr(tmem, lane_base, buf * 128 + COL0 + q * 8), vq);
+            }
+            umma::tmem_ld_wait();
+        }
+        umma::fence_before_sync();
+        __syncwarp();
+        if (lane == 0) umma::mbar_arrive(&acc_free[buf]);
+        if (active) {
+            float box[NCELL];
+#pragma unroll
+            for (int j = 0; j < NCELL; ++j) box[j] = 0.f;
+            float *gp = a.gpre + ((size_t)b * d.Ce * KK + (size_t)c * KK) * plane + (size_t)y * d.W + x;
+#pragma unroll
+            for (int q = 0; q < KK; ++q) {
+                const float pre = v[OFF + q] + bias_s[wq][q];   // bit-identical to the forward's accumulator + bias
+                const bool pos = pre > 0.f;
+                float kg = 0.f;                              // LeakyReLU(P) * G: this pixel's dL/dEpad term of tap q
+                if (valid) {
+                    const float ge = g * e[q];               // dL/dKernel (KernelConv2D backward)
+                    const float gpq = pos ? ge : ge * d.slope;   // leaky_relu_backward: P == 0 takes the slope
+                    __stcs(gp + (size_t)q * plane, gpq);
+                    bsum[q] += gpq;
+                    kg = (pos ? pre : pre * d.slope) * g;
+                }
+#pragma unroll
+                for (int j = 0; j < NCELL; ++j) {        // the lane index wraps mod 32 where the cell has no source
+                    const float pulled = __shfl_sync(0xffffffffu, kg, cbase[j] - ((q / K) * TW + q % K));
+                    if ((cmask[j] >> q) & 1u) box[j] += pulled;
+                }
+            }
+            float *dst = a.gbox + ((((size_t)b * d.Ce + c) * wrows + tyi * (TH / WR) + wq) * d.tiles_x + txi) * BOX;
+#pragma unroll
+            for (int j = 0; j < NCELL; ++j)
+                if (lane + 32 * j < BOX) dst[lane + 32 * j] = box[j];
+        }
+    }
+    if (cur_slice >= 0 && cur_slice * CPS + G < d.Ce) flush(cur_slice);
+}
+
+// K: FAC kernel size; NPART: halo parts = Cin / 32; BWD: backward epilogue (bw) instead of the FAC one (out)
+template <int K, int NPART, bool BWD>
 __global__ void __launch_bounds__(NTHR, 1)
 kpn_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat16 *__restrict__ wimg,
                  const float *__restrict__ bias, const float *__restrict__ ev, float *__restrict__ out,
-                 KpnDims d, int items_per_cta)
+                 KpnBwdArgs bw, KpnDims d, int items_per_cta)
 {
     constexpr int KK = K * K, R = (K - 1) / 2;
     extern __shared__ __align__(128) unsigned char smem[];
@@ -282,13 +430,61 @@ kpn_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat16 *
     } else {
         // ===================== epilogue warpgroups: thread = (pixel = TMEM lane, FAC channel G of the slice) ==========
         const int g = warp >> 2;
-        if (g == 0) kpn_epilogue<K, 0>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
-        else if (g == 1) kpn_epilogue<K, 1>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
-        else kpn_epilogue<K, 2>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
+        if constexpr (BWD) {
+            if (g == 0) kpn_bwd_epilogue<K, 0>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
+            else if (g == 1) kpn_bwd_epilogue<K, 1>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
+            else kpn_bwd_epilogue<K, 2>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
+        } else {
+            if (g == 0) kpn_epilogue<K, 0>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
+            else if (g == 1) kpn_epilogue<K, 1>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
+            else kpn_epilogue<K, 2>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
+        }
     }
     umma::fence_before_sync();
     __syncthreads();
     if (warp == 0) umma::tmem_dealloc<TMEM_COLS>(tmem);
+}
+
+// dL/dEvent (FAC + ReplicationPad part): thread = one event cell (b, c, y, x). It sums the Epad cells that the
+// replication pad maps onto it (one in the interior, up to (R+1)^2 in a corner), each from the <= 2 x 2 warp boxes
+// that cover it, in a fixed order.
+__global__ void kpn_gev_collect(const float *__restrict__ gbox, float *__restrict__ gev, KpnDims d)
+{
+    const int R = (d.K - 1) / 2, BH = WR + d.K - 1, BW = TW + d.K - 1, box = BH * BW;
+    const int wrows = d.tiles_y * (TH / WR);
+    const size_t plane = (size_t)d.H * d.W, n = (size_t)d.B * d.Ce * plane;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const int x = (int)(i % d.W), y = (int)((i / d.W) % d.H);
+        const size_t bc = i / plane;
+        const int y0 = y == 0 ? 0 : y + R, y1 = y == d.H - 1 ? d.H - 1 + 2 * R : y + R;   // Epad rows folding onto y
+        const int x0 = x == 0 ? 0 : x + R, x1 = x == d.W - 1 ? d.W - 1 + 2 * R : x + R;
+        const float *base = gbox + bc * wrows * d.tiles_x * box;
+        float acc = 0.f;
+        for (int Y = y0; Y <= y1; ++Y) {
+            const int r0 = Y >= BH ? (Y - BH + WR) / WR : 0, r1 = min(Y / WR, wrows - 1);
+            for (int X = x0; X <= x1; ++X) {
+                const int c0 = X >= BW ? (X - BW + TW) / TW : 0, c1 = min(X / TW, d.tiles_x - 1);
+                for (int r = r0; r <= r1; ++r)
+                    for (int cc = c0; cc <= c1; ++cc)
+                        acc += __ldg(base + ((size_t)r * d.tiles_x + cc) * box + (Y - r * WR) * BW + (X - cc * TW));
+            }
+        }
+        gev[i] = acc;
+    }
+}
+
+// grad_bias[c*KK+q]: the warp partials of slice c / CPS, CTA by CTA (the CTAs whose item range meets the slice), then
+// warp by warp.
+__global__ void kpn_bias_collect(const float *__restrict__ part, float *__restrict__ gbias, KpnDims d, int per)
+{
+    const int col = blockIdx.x * blockDim.x + threadIdx.x;
+    if (col >= d.Ce * d.KK) return;
+    const int c = col / d.KK, q = col % d.KK, s = c / CPS, g = c % CPS;
+    const long k0 = (long)s * d.ntile / per, k1 = ((long)(s + 1) * d.ntile - 1) / per;
+    float acc = 0.f;
+    for (long k = k0; k <= k1; ++k)
+        for (int w = 0; w < 4; ++w) acc += part[((size_t)(k + s) * (NEPI / 32) + g * 4 + w) * d.KK + q];
+    gbias[col] = acc;
 }
 
 // featb [B*kchunks][H][W*8] bf16, box = one halo part: [4 chunks][18 rows][10 pixels * 8 channels]
@@ -319,6 +515,55 @@ int fill(KpnDims &d, int B, int Ce, int Cf, int H, int W, int K, float slope)
 
 size_t ws_weights(const KpnDims &d) { return ebfi::round_up((size_t)d.nslice * d.w_bytes, (size_t)256); }
 size_t ws_input(const KpnDims &d) { return (size_t)d.B * d.Cin * d.H * d.W * 2; }
+size_t ws_gbox(const KpnDims &d)
+{
+    return ebfi::round_up((size_t)d.B * d.Ce * d.tiles_y * (TH / WR) * d.tiles_x * (WR + d.K - 1) * (TW + d.K - 1) * 4, (size_t)256);
+}
+// bias partials are indexed by CTA + slice (injective: CTA ranges are contiguous and slice-major)
+size_t ws_bias_part(const KpnDims &d) { return (size_t)(BWD_MAX_GRID + d.nslice) * (NEPI / 32) * d.KK * 4; }
+
+// bf16 operand images for the main loop (weights per slice, channel-chunked input) and the input's tensor map
+int prep_operands(const KpnDims &d, cudaStream_t st, const float *ev, const float *fr, const float *w, void *workspace,
+                  CUtensorMap &tmap)
+{
+    __nv_bfloat16 *wimg = static_cast<__nv_bfloat16 *>(workspace);
+    __nv_bfloat16 *featb = reinterpret_cast<__nv_bfloat16 *>(static_cast<char *>(workspace) + ws_weights(d));
+    kpn_prep_weights<<<ebfi::sm_count() * 4, 256, 0, st>>>(w, wimg, d);
+    EBFI_LAUNCH_OK("kpn_prep_weights");
+    kpn_prep_input<<<ebfi::sm_count() * 8, 256, 0, st>>>(ev, fr, featb, d);
+    EBFI_LAUNCH_OK("kpn_prep_input");
+    return make_tmap(tmap, d, featb);
+}
+
+template <bool BWD>
+int launch_fused(const KpnDims &d, cudaStream_t st, const CUtensorMap &tmap, const void *workspace, const float *bias,
+                 const float *ev, float *out, const KpnBwdArgs &bw, int per)
+{
+    const __nv_bfloat16 *wimg = static_cast<const __nv_bfloat16 *>(workspace);
+    const int smem = d.w_bytes + d.npart * PART_BYTES;
+    const int total = d.nslice * d.ntile;
+#define EBFI_KPN(KS, ST)                                                                                      \
+    do {                                                                                                      \
+        EBFI_CUDA_OK(cudaFuncSetAttribute(kpn_fused_kernel<KS, ST, BWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+        kpn_fused_kernel<KS, ST, BWD><<<ceil_div(total, per), NTHR, smem, st>>>(tmap, wimg, bias, ev, out, bw, d, per); \
+    } while (0)
+#define EBFI_KPN_K(KS)                                                                                        \
+    switch (d.Cin / 32) {                                                                                     \
+    case 1: EBFI_KPN(KS, 1); break;                                                                           \
+    case 2: EBFI_KPN(KS, 2); break;                                                                           \
+    case 3: EBFI_KPN(KS, 3); break;                                                                           \
+    default: EBFI_KPN(KS, 4); break;                                                                          \
+    }
+    switch (d.K) {
+    case 1: EBFI_KPN_K(1); break;
+    case 3: EBFI_KPN_K(3); break;
+    default: EBFI_KPN_K(5); break;
+    }
+#undef EBFI_KPN_K
+#undef EBFI_KPN
+    EBFI_LAUNCH_OK("kpn_fused_kernel");
+    return EBFI_OK;
+}
 
 }  // namespace
 
@@ -346,38 +591,52 @@ int ebfi_kpn_fused_forward(void *stream, const float *event_feat, const float *f
         return ebfi::fail(EBFI_ERR_WORKSPACE, "kpn_fused: workspace %zu < %zu bytes", workspace_bytes, need);
     EBFI_REQUIRE(ebfi::aligned16(workspace), "kpn_fused: workspace must be 16-byte aligned");
     cudaStream_t st = ebfi::as_stream(stream);
-    __nv_bfloat16 *wimg = static_cast<__nv_bfloat16 *>(workspace);
-    __nv_bfloat16 *featb = reinterpret_cast<__nv_bfloat16 *>(static_cast<char *>(workspace) + ws_weights(d));
-    kpn_prep_weights<<<ebfi::sm_count() * 4, 256, 0, st>>>(conv_weight, wimg, d);
-    EBFI_LAUNCH_OK("kpn_prep_weights");
-    kpn_prep_input<<<ebfi::sm_count() * 8, 256, 0, st>>>(event_feat, frame_feat, featb, d);
-    EBFI_LAUNCH_OK("kpn_prep_input");
-    const int smem = d.w_bytes + d.npart * PART_BYTES;
     CUtensorMap tmap;
-    if (int rc = make_tmap(tmap, d, featb)) return rc;
+    if (int rc = prep_operands(d, st, event_feat, frame_feat, conv_weight, workspace, tmap)) return rc;
     const int total = d.nslice * d.ntile;
     const int grid = std::min(total, ebfi::sm_count());
+    return launch_fused<false>(d, st, tmap, workspace, conv_bias, event_feat, output, KpnBwdArgs{}, ceil_div(total, grid));
+}
+
+size_t ebfi_kpn_fused_backward_workspace_bytes(int batch, int channels_event, int channels_frame, int height, int width,
+                                               int kernel_size)
+{
+    KpnDims d{};
+    if (fill(d, batch, channels_event, channels_frame, height, width, kernel_size, 0.f) != EBFI_OK) return 0;
+    return ws_weights(d) + ebfi::round_up(ws_input(d), (size_t)256) + ws_gbox(d) + ws_bias_part(d) + 256;
+}
+
+int ebfi_kpn_fused_backward(void *stream, const float *event_feat, const float *frame_feat, const float *conv_weight,
+                            const float *conv_bias, float negative_slope, const float *grad_output, float *grad_pre,
+                            float *grad_event_fac, float *grad_bias, int batch, int channels_event, int channels_frame,
+                            int height, int width, int kernel_size, void *workspace, size_t workspace_bytes)
+{
+    KpnDims d{};
+    if (int rc = fill(d, batch, channels_event, channels_frame, height, width, kernel_size, negative_slope)) return rc;
+    EBFI_REQUIRE(event_feat && (frame_feat || channels_frame == 0) && conv_weight && conv_bias && grad_output &&
+                 grad_pre && grad_event_fac && grad_bias, "kpn_fused_backward: null pointer");
+    const size_t off_gbox = ws_weights(d) + ebfi::round_up(ws_input(d), (size_t)256);
+    const size_t off_part = off_gbox + ws_gbox(d);
+    const size_t need = off_part + ws_bias_part(d);
+    if (!workspace || workspace_bytes < need)
+        return ebfi::fail(EBFI_ERR_WORKSPACE, "kpn_fused_backward: workspace %zu < %zu bytes", workspace_bytes, need);
+    EBFI_REQUIRE(ebfi::aligned16(workspace), "kpn_fused_backward: workspace must be 16-byte aligned");
+    cudaStream_t st = ebfi::as_stream(stream);
+    CUtensorMap tmap;
+    if (int rc = prep_operands(d, st, event_feat, frame_feat, conv_weight, workspace, tmap)) return rc;
+    KpnBwdArgs bw;
+    bw.gout = grad_output;
+    bw.gpre = grad_pre;
+    bw.gbox = reinterpret_cast<float *>(static_cast<char *>(workspace) + off_gbox);
+    bw.bias_part = reinterpret_cast<float *>(static_cast<char *>(workspace) + off_part);
+    const int total = d.nslice * d.ntile;
+    const int grid = std::min(std::min(total, ebfi::sm_count()), BWD_MAX_GRID);
     const int per = ceil_div(total, grid);
-#define EBFI_KPN(KS, ST)                                                                                      \
-    do {                                                                                                      \
-        EBFI_CUDA_OK(cudaFuncSetAttribute(kpn_fused_kernel<KS, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-        kpn_fused_kernel<KS, ST><<<ceil_div(total, per), NTHR, smem, st>>>(tmap, wimg, conv_bias, event_feat, output, d, per); \
-    } while (0)
-#define EBFI_KPN_K(KS)                                                                                        \
-    switch (d.Cin / 32) {                                                                                     \
-    case 1: EBFI_KPN(KS, 1); break;                                                                           \
-    case 2: EBFI_KPN(KS, 2); break;                                                                           \
-    case 3: EBFI_KPN(KS, 3); break;                                                                           \
-    default: EBFI_KPN(KS, 4); break;                                                                          \
-    }
-    switch (d.K) {
-    case 1: EBFI_KPN_K(1); break;
-    case 3: EBFI_KPN_K(3); break;
-    default: EBFI_KPN_K(5); break;
-    }
-#undef EBFI_KPN_K
-#undef EBFI_KPN
-    EBFI_LAUNCH_OK("kpn_fused_kernel");
+    if (int rc = launch_fused<true>(d, st, tmap, workspace, conv_bias, event_feat, nullptr, bw, per)) return rc;
+    kpn_gev_collect<<<ebfi::sm_count() * 8, 256, 0, st>>>(bw.gbox, grad_event_fac, d);
+    EBFI_LAUNCH_OK("kpn_gev_collect");
+    kpn_bias_collect<<<ceil_div(d.Ce * d.KK, 128), 128, 0, st>>>(bw.bias_part, grad_bias, d, per);
+    EBFI_LAUNCH_OK("kpn_bias_collect");
     return EBFI_OK;
 }
 

@@ -190,13 +190,32 @@ int ebfi_fac_backward_bf16(void *stream, const void *input, const void *kernel, 
  *   output (B, Ce, H, W), every element written.
  * Precision: the convolution's operands are rounded to bf16 for the tcgen05 tensor cores, accumulation and the
  * FAC contraction are fp32 (the reference's conv runs in TF32 under torch's defaults). Shapes: (Ce+Cf) % 32 == 0,
- * Ce+Cf <= 128, odd K <= 5; otherwise EBFI_ERR_UNSUPPORTED. Inference path: there is no fused backward. */
+ * Ce+Cf <= 128, odd K <= 5; otherwise EBFI_ERR_UNSUPPORTED. The matching backward is ebfi_kpn_fused_backward. */
 size_t ebfi_kpn_fused_workspace_bytes(int batch, int channels_event, int channels_frame, int height, int width,
                                       int kernel_size);
 int ebfi_kpn_fused_forward(void *stream, const float *event_feat, const float *frame_feat,
                            const float *conv_weight, const float *conv_bias, float negative_slope,
                            float *output, int batch, int channels_event, int channels_frame,
                            int height, int width, int kernel_size, void *workspace, size_t workspace_bytes);
+
+/* Fused backward of the same block, given grad_output = dL/doutput (B, Ce, H, W). It recomputes the conv's
+ * pre-activation P = conv3x3(cat(event_feat, frame_feat)) + conv_bias on the tensor cores exactly as the forward does
+ * (same bf16 operands, same accumulation order, so the same LeakyReLU branches) and writes, fp32 NCHW contiguous:
+ *   grad_pre       (B, Ce*K*K, H, W)  dL/dP = G * Epad * (P > 0 ? 1 : negative_slope), every element written
+ *   grad_event_fac (B, Ce, H, W)      the FAC + ReplicationPad2d part of dL/devent_feat, every element written
+ *   grad_bias      (Ce*K*K)           dL/dconv_bias (sum of grad_pre over batch and pixels)
+ * Neither the kernel tensor LeakyReLU(P) nor P ever exists in HBM. The caller still computes the conv's weight and
+ * input gradients from grad_pre (an ordinary 3x3 pad-1 convolution backward of cat(event_feat, frame_feat)) and adds
+ * the event channels of the input gradient to grad_event_fac. Deterministic: no float atomics; results are
+ * bit-identical run to run on a device. Shapes, precision and error codes as ebfi_kpn_fused_forward; null pointers
+ * return EBFI_ERR_INVALID before any CUDA call. The workspace size does not depend on the device (0 = unsupported). */
+size_t ebfi_kpn_fused_backward_workspace_bytes(int batch, int channels_event, int channels_frame,
+                                               int height, int width, int kernel_size);
+int ebfi_kpn_fused_backward(void *stream, const float *event_feat, const float *frame_feat,
+                            const float *conv_weight, const float *conv_bias, float negative_slope,
+                            const float *grad_output, float *grad_pre, float *grad_event_fac, float *grad_bias,
+                            int batch, int channels_event, int channels_frame, int height, int width,
+                            int kernel_size, void *workspace, size_t workspace_bytes);
 
 /* ---- event encoders --------------------------------------------------------- */
 
