@@ -61,6 +61,8 @@ SIGNATURES = {
     "ebfi_kpn_fused_forward": (c_int, [c_void] * 5 + [ctypes.c_float, c_void] + [c_int] * 6 + [c_void, c_size]),
     "ebfi_kpn_fused_backward_workspace_bytes": (c_size, [c_int] * 6),
     "ebfi_kpn_fused_backward": (c_int, [c_void] * 5 + [ctypes.c_float] + [c_void] * 4 + [c_int] * 6 + [c_void, c_size]),
+    "ebfi_kpn_fused_forward_bf16": (c_int, [c_void] * 5 + [ctypes.c_float, c_void] + [c_int] * 6 + [c_void, c_size]),
+    "ebfi_kpn_fused_backward_bf16": (c_int, [c_void] * 5 + [ctypes.c_float] + [c_void] * 4 + [c_int] * 6 + [c_void, c_size]),
     "ebfi_events_to_image": (c_int, [c_void] * 4 + [c_int, c_i64, c_int, c_int, c_void, c_int]),
     "ebfi_events_to_mask": (c_int, [c_void] * 4 + [c_int, c_i64, c_int, c_int, c_void, c_void, c_int]),
     "ebfi_events_to_voxel": (c_int, [c_void] * 5 + [c_int, c_i64, c_int, c_int, c_int, c_void, c_int]),

@@ -35,11 +35,15 @@
 // Precision: tensors are fp32 at the boundary (like the reference); the conv operands are rounded to bf16
 // for the tensor cores, accumulation and the whole FAC part are fp32. Stated tolerance 1e-2 of max|out|
 // against the fp32/fp64 op sequence; 1e-5 against the same sequence with bf16-rounded conv operands.
+// Activation I/O (event / frame / output, and grad_output / grad_pre in the backward) may instead be bf16 (template
+// parameter T, the *_bf16 entries): only the loads convert (exactly) and the stores round once (RN) from the same
+// fp32 values, so on bf16-valued inputs a bf16 instantiation computes bit-identically to the fp32 one. Weights, bias,
+// grad_event_fac and grad_bias stay fp32.
 //
 // Backward (ebfi_kpn_fused_backward): the same kernel with BWD = true recomputes the pre-activation P in TMEM
 // through the identical main loop (same operands, same MMA chain -> bit-identical P, so forward and backward take
 // the same LeakyReLU branch everywhere) and replaces the FAC epilogue by its gradient. Thread = (pixel, channel):
-//   gP[c*KK+t, p]  = G[c,p] * Epad[c,p+t] * (P > 0 ? 1 : slope)      written fp32 NCHW = cuDNN's dgrad/wgrad input
+//   gP[c*KK+t, p]  = G[c,p] * Epad[c,p+t] * (P > 0 ? 1 : slope)      written NCHW (type T) = cuDNN's dgrad/wgrad input
 //   gEpad[c, q]   += LeakyReLU(P)[c*KK+t, q-t] * G[c, q-t]            per-warp box in unclamped Epad coordinates
 //   grad_bias      = per-lane running column sums of gP over the CTA's items of a slice
 // gEpad: a warp holds 4 x 8 pixels, i.e. an (4+K-1) x (8+K-1) box of Epad cells, <= 3 per lane. For a fixed tap every
@@ -79,16 +83,25 @@ struct KpnDims {
     float slope;
 };
 
+// Activation element type T (float | __nv_bfloat16): loads widen to fp32 exactly, stores round once (RN).
+__device__ __forceinline__ float ld_act(const float *p) { return __ldg(p); }
+__device__ __forceinline__ float ld_act(const __nv_bfloat16 *p) { return __bfloat162float(__ldg(p)); }
+template <typename T> __device__ __forceinline__ T st_act(float v);
+template <> __device__ __forceinline__ float st_act<float>(float v) { return v; }
+template <> __device__ __forceinline__ __nv_bfloat16 st_act<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+
 // Backward-only operands of the fused kernel (unused by the forward instantiation).
+template <typename T>
 struct KpnBwdArgs {
-    const float *gout;      // (B, Ce, H, W) dL/dout
-    float *gpre;            // (B, Ce*KK, H, W) dL/dP
+    const T *gout;          // (B, Ce, H, W) dL/dout
+    T *gpre;                // (B, Ce*KK, H, W) dL/dP
     float *gbox;            // [B][Ce][tiles_y*TH/WR][tiles_x][WR+K-1][TW+K-1] per-warp dL/dEpad boxes
     float *bias_part;       // [CTA + slice][NEPI/32 warps][KK] column sums of dL/dP
 };
 
-// (ev | fr) NCHW fp32 -> [b][chunk of 8 channels][y][x][8] bf16: one thread per (b, chunk, y, x)
-__global__ void kpn_prep_input(const float *__restrict__ ev, const float *__restrict__ fr, __nv_bfloat16 *__restrict__ dst,
+// (ev | fr) NCHW T -> [b][chunk of 8 channels][y][x][8] bf16: one thread per (b, chunk, y, x)
+template <typename T>
+__global__ void kpn_prep_input(const T *__restrict__ ev, const T *__restrict__ fr, __nv_bfloat16 *__restrict__ dst,
                                KpnDims d)
 {
     const size_t plane = (size_t)d.H * d.W, n = (size_t)d.B * d.kchunks * plane;
@@ -100,8 +113,8 @@ __global__ void kpn_prep_input(const float *__restrict__ ev, const float *__rest
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
             const int ch = kc * 8 + e;
-            const float x = ch < d.Ce ? __ldg(ev + ((size_t)b * d.Ce + ch) * plane + px)
-                                      : __ldg(fr + ((size_t)b * Cf + (ch - d.Ce)) * plane + px);
+            const float x = ch < d.Ce ? ld_act(ev + ((size_t)b * d.Ce + ch) * plane + px)
+                                      : ld_act(fr + ((size_t)b * Cf + (ch - d.Ce)) * plane + px);
             v[e] = __bfloat16_as_ushort(__float2bfloat16_rn(x));
         }
         *reinterpret_cast<uint4 *>(dst + i * 8) = make_uint4(v[0] | ((uint32_t)v[1] << 16), v[2] | ((uint32_t)v[3] << 16),
@@ -130,10 +143,10 @@ __global__ void kpn_prep_weights(const float *__restrict__ w, __nv_bfloat16 *__r
 }
 
 // Epilogue of warpgroup G: FAC channel c0 + G of every item's slice.
-template <int K, int G>
+template <int K, int G, typename T>
 __device__ __forceinline__ void kpn_epilogue(uint32_t tmem, uint64_t *acc_full, uint64_t *acc_free,
-                                             const float *__restrict__ bias, const float *__restrict__ ev,
-                                             float *__restrict__ out, const KpnDims &d, int item0, int item1)
+                                             const float *__restrict__ bias, const T *__restrict__ ev,
+                                             T *__restrict__ out, const KpnDims &d, int item0, int item1)
 {
     constexpr int KK = K * K, R = (K - 1) / 2;
     constexpr int COL0 = (G * KK / 8) * 8, OFF = G * KK - COL0, NLD = (OFF + KK + 7) / 8;   // 8-column TMEM loads covering the channel
@@ -154,15 +167,15 @@ __device__ __forceinline__ void kpn_epilogue(uint32_t tmem, uint64_t *acc_full, 
         // Event window of this pixel: independent of the accumulator -> in flight while waiting for it
         float e[KK];
         if (valid) {
-            const float *evc = ev + ((size_t)b * d.Ce + c) * plane;
+            const T *evc = ev + ((size_t)b * d.Ce + c) * plane;
             int xo[K];
 #pragma unroll
             for (int kx = 0; kx < K; ++kx) xo[kx] = min(max(x + kx - R, 0), d.W - 1);   // ReplicationPad2d (KernelConv2D.py:82-86)
 #pragma unroll
             for (int ky = 0; ky < K; ++ky) {
-                const float *row = evc + (size_t)min(max(y + ky - R, 0), d.H - 1) * d.W;
+                const T *row = evc + (size_t)min(max(y + ky - R, 0), d.H - 1) * d.W;
 #pragma unroll
-                for (int kx = 0; kx < K; ++kx) e[ky * K + kx] = __ldg(row + xo[kx]);
+                for (int kx = 0; kx < K; ++kx) e[ky * K + kx] = ld_act(row + xo[kx]);
             }
         }
         if (active && s != bias_slice) {
@@ -193,16 +206,16 @@ __device__ __forceinline__ void kpn_epilogue(uint32_t tmem, uint64_t *acc_full, 
                 a = a > 0.f ? a : a * d.slope;               // nn.LeakyReLU
                 res += e[q] * a;
             }
-            out[((size_t)b * d.Ce + c) * plane + (size_t)y * d.W + x] = res;
+            out[((size_t)b * d.Ce + c) * plane + (size_t)y * d.W + x] = st_act<T>(res);
         }
     }
 }
 
 // Backward epilogue of warpgroup G (see the header comment): gP, the warp's dL/dEpad box, bias column sums.
-template <int K, int G>
+template <int K, int G, typename T>
 __device__ __forceinline__ void kpn_bwd_epilogue(uint32_t tmem, uint64_t *acc_full, uint64_t *acc_free,
-                                                 const float *__restrict__ bias, const float *__restrict__ ev,
-                                                 const KpnBwdArgs &a, const KpnDims &d, int item0, int item1)
+                                                 const float *__restrict__ bias, const T *__restrict__ ev,
+                                                 const KpnBwdArgs<T> &a, const KpnDims &d, int item0, int item1)
 {
     constexpr int KK = K * K, R = (K - 1) / 2;
     constexpr int COL0 = (G * KK / 8) * 8, OFF = G * KK - COL0, NLD = (OFF + KK + 7) / 8;
@@ -265,17 +278,17 @@ __device__ __forceinline__ void kpn_bwd_epilogue(uint32_t tmem, uint64_t *acc_fu
         }
         float e[KK], g = 0.f;
         if (valid) {
-            const float *evc = ev + ((size_t)b * d.Ce + c) * plane;
+            const T *evc = ev + ((size_t)b * d.Ce + c) * plane;
             int xo[K];
 #pragma unroll
             for (int kx = 0; kx < K; ++kx) xo[kx] = min(max(x + kx - R, 0), d.W - 1);
 #pragma unroll
             for (int ky = 0; ky < K; ++ky) {
-                const float *row = evc + (size_t)min(max(y + ky - R, 0), d.H - 1) * d.W;
+                const T *row = evc + (size_t)min(max(y + ky - R, 0), d.H - 1) * d.W;
 #pragma unroll
-                for (int kx = 0; kx < K; ++kx) e[ky * K + kx] = __ldg(row + xo[kx]);
+                for (int kx = 0; kx < K; ++kx) e[ky * K + kx] = ld_act(row + xo[kx]);
             }
-            g = __ldg(a.gout + ((size_t)b * d.Ce + c) * plane + (size_t)y * d.W + x);
+            g = ld_act(a.gout + ((size_t)b * d.Ce + c) * plane + (size_t)y * d.W + x);
         }
         const int buf = n & 1;
         umma::mbar_wait_warp(&acc_full[buf], (uint32_t)((n >> 1) & 1));
@@ -296,7 +309,7 @@ __device__ __forceinline__ void kpn_bwd_epilogue(uint32_t tmem, uint64_t *acc_fu
             float box[NCELL];
 #pragma unroll
             for (int j = 0; j < NCELL; ++j) box[j] = 0.f;
-            float *gp = a.gpre + ((size_t)b * d.Ce * KK + (size_t)c * KK) * plane + (size_t)y * d.W + x;
+            T *gp = a.gpre + ((size_t)b * d.Ce * KK + (size_t)c * KK) * plane + (size_t)y * d.W + x;
 #pragma unroll
             for (int q = 0; q < KK; ++q) {
                 const float pre = v[OFF + q] + bias_s[wq][q];   // bit-identical to the forward's accumulator + bias
@@ -305,7 +318,7 @@ __device__ __forceinline__ void kpn_bwd_epilogue(uint32_t tmem, uint64_t *acc_fu
                 if (valid) {
                     const float ge = g * e[q];               // dL/dKernel (KernelConv2D backward)
                     const float gpq = pos ? ge : ge * d.slope;   // leaky_relu_backward: P == 0 takes the slope
-                    __stcs(gp + (size_t)q * plane, gpq);
+                    __stcs(gp + (size_t)q * plane, st_act<T>(gpq));   // bias sums use the unrounded gpq
                     bsum[q] += gpq;
                     kg = (pos ? pre : pre * d.slope) * g;
                 }
@@ -324,12 +337,13 @@ __device__ __forceinline__ void kpn_bwd_epilogue(uint32_t tmem, uint64_t *acc_fu
     if (cur_slice >= 0 && cur_slice * CPS + G < d.Ce) flush(cur_slice);
 }
 
-// K: FAC kernel size; NPART: halo parts = Cin / 32; BWD: backward epilogue (bw) instead of the FAC one (out)
-template <int K, int NPART, bool BWD>
+// K: FAC kernel size; NPART: halo parts = Cin / 32; BWD: backward epilogue (bw) instead of the FAC one (out);
+// T: activation element type of ev / out / bw.gout / bw.gpre
+template <int K, int NPART, bool BWD, typename T>
 __global__ void __launch_bounds__(NTHR, 1)
 kpn_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat16 *__restrict__ wimg,
-                 const float *__restrict__ bias, const float *__restrict__ ev, float *__restrict__ out,
-                 KpnBwdArgs bw, KpnDims d, int items_per_cta)
+                 const float *__restrict__ bias, const T *__restrict__ ev, T *__restrict__ out,
+                 KpnBwdArgs<T> bw, KpnDims d, int items_per_cta)
 {
     constexpr int KK = K * K, R = (K - 1) / 2;
     extern __shared__ __align__(128) unsigned char smem[];
@@ -431,13 +445,13 @@ kpn_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat16 *
         // ===================== epilogue warpgroups: thread = (pixel = TMEM lane, FAC channel G of the slice) ==========
         const int g = warp >> 2;
         if constexpr (BWD) {
-            if (g == 0) kpn_bwd_epilogue<K, 0>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
-            else if (g == 1) kpn_bwd_epilogue<K, 1>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
-            else kpn_bwd_epilogue<K, 2>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
+            if (g == 0) kpn_bwd_epilogue<K, 0, T>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
+            else if (g == 1) kpn_bwd_epilogue<K, 1, T>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
+            else kpn_bwd_epilogue<K, 2, T>(tmem, acc_full, acc_free, bias, ev, bw, d, item0, item1);
         } else {
-            if (g == 0) kpn_epilogue<K, 0>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
-            else if (g == 1) kpn_epilogue<K, 1>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
-            else kpn_epilogue<K, 2>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
+            if (g == 0) kpn_epilogue<K, 0, T>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
+            else if (g == 1) kpn_epilogue<K, 1, T>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
+            else kpn_epilogue<K, 2, T>(tmem, acc_full, acc_free, bias, ev, out, d, item0, item1);
         }
     }
     umma::fence_before_sync();
@@ -523,7 +537,8 @@ size_t ws_gbox(const KpnDims &d)
 size_t ws_bias_part(const KpnDims &d) { return (size_t)(BWD_MAX_GRID + d.nslice) * (NEPI / 32) * d.KK * 4; }
 
 // bf16 operand images for the main loop (weights per slice, channel-chunked input) and the input's tensor map
-int prep_operands(const KpnDims &d, cudaStream_t st, const float *ev, const float *fr, const float *w, void *workspace,
+template <typename T>
+int prep_operands(const KpnDims &d, cudaStream_t st, const T *ev, const T *fr, const float *w, void *workspace,
                   CUtensorMap &tmap)
 {
     __nv_bfloat16 *wimg = static_cast<__nv_bfloat16 *>(workspace);
@@ -535,17 +550,17 @@ int prep_operands(const KpnDims &d, cudaStream_t st, const float *ev, const floa
     return make_tmap(tmap, d, featb);
 }
 
-template <bool BWD>
+template <bool BWD, typename T>
 int launch_fused(const KpnDims &d, cudaStream_t st, const CUtensorMap &tmap, const void *workspace, const float *bias,
-                 const float *ev, float *out, const KpnBwdArgs &bw, int per)
+                 const T *ev, T *out, const KpnBwdArgs<T> &bw, int per)
 {
     const __nv_bfloat16 *wimg = static_cast<const __nv_bfloat16 *>(workspace);
     const int smem = d.w_bytes + d.npart * PART_BYTES;
     const int total = d.nslice * d.ntile;
 #define EBFI_KPN(KS, ST)                                                                                      \
     do {                                                                                                      \
-        EBFI_CUDA_OK(cudaFuncSetAttribute(kpn_fused_kernel<KS, ST, BWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-        kpn_fused_kernel<KS, ST, BWD><<<ceil_div(total, per), NTHR, smem, st>>>(tmap, wimg, bias, ev, out, bw, d, per); \
+        EBFI_CUDA_OK(cudaFuncSetAttribute(kpn_fused_kernel<KS, ST, BWD, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+        kpn_fused_kernel<KS, ST, BWD, T><<<ceil_div(total, per), NTHR, smem, st>>>(tmap, wimg, bias, ev, out, bw, d, per); \
     } while (0)
 #define EBFI_KPN_K(KS)                                                                                        \
     switch (d.Cin / 32) {                                                                                     \
@@ -562,6 +577,63 @@ int launch_fused(const KpnDims &d, cudaStream_t st, const CUtensorMap &tmap, con
 #undef EBFI_KPN_K
 #undef EBFI_KPN
     EBFI_LAUNCH_OK("kpn_fused_kernel");
+    return EBFI_OK;
+}
+
+template <typename T>
+int kpn_forward(void *stream, const T *event_feat, const T *frame_feat, const float *conv_weight, const float *conv_bias,
+                float negative_slope, T *output, int batch, int channels_event, int channels_frame, int height,
+                int width, int kernel_size, void *workspace, size_t workspace_bytes)
+{
+    KpnDims d{};
+    if (int rc = fill(d, batch, channels_event, channels_frame, height, width, kernel_size, negative_slope)) return rc;
+    EBFI_REQUIRE(event_feat && (frame_feat || channels_frame == 0) && conv_weight && conv_bias && output,
+                 "kpn_fused: null pointer");
+    const size_t need = ws_weights(d) + ws_input(d);
+    if (!workspace || workspace_bytes < need)
+        return ebfi::fail(EBFI_ERR_WORKSPACE, "kpn_fused: workspace %zu < %zu bytes", workspace_bytes, need);
+    EBFI_REQUIRE(ebfi::aligned16(workspace), "kpn_fused: workspace must be 16-byte aligned");
+    cudaStream_t st = ebfi::as_stream(stream);
+    CUtensorMap tmap;
+    if (int rc = prep_operands(d, st, event_feat, frame_feat, conv_weight, workspace, tmap)) return rc;
+    const int total = d.nslice * d.ntile;
+    const int grid = std::min(total, ebfi::sm_count());
+    return launch_fused<false>(d, st, tmap, workspace, conv_bias, event_feat, output, KpnBwdArgs<T>{}, ceil_div(total, grid));
+}
+
+template <typename T>
+int kpn_backward(void *stream, const T *event_feat, const T *frame_feat, const float *conv_weight,
+                 const float *conv_bias, float negative_slope, const T *grad_output, T *grad_pre,
+                 float *grad_event_fac, float *grad_bias, int batch, int channels_event, int channels_frame,
+                 int height, int width, int kernel_size, void *workspace, size_t workspace_bytes)
+{
+    KpnDims d{};
+    if (int rc = fill(d, batch, channels_event, channels_frame, height, width, kernel_size, negative_slope)) return rc;
+    EBFI_REQUIRE(event_feat && (frame_feat || channels_frame == 0) && conv_weight && conv_bias && grad_output &&
+                 grad_pre && grad_event_fac && grad_bias, "kpn_fused_backward: null pointer");
+    const size_t off_gbox = ws_weights(d) + ebfi::round_up(ws_input(d), (size_t)256);
+    const size_t off_part = off_gbox + ws_gbox(d);
+    const size_t need = off_part + ws_bias_part(d);
+    if (!workspace || workspace_bytes < need)
+        return ebfi::fail(EBFI_ERR_WORKSPACE, "kpn_fused_backward: workspace %zu < %zu bytes", workspace_bytes, need);
+    EBFI_REQUIRE(ebfi::aligned16(workspace), "kpn_fused_backward: workspace must be 16-byte aligned");
+    cudaStream_t st = ebfi::as_stream(stream);
+    CUtensorMap tmap;
+    if (int rc = prep_operands(d, st, event_feat, frame_feat, conv_weight, workspace, tmap)) return rc;
+    KpnBwdArgs<T> bw;
+    bw.gout = grad_output;
+    bw.gpre = grad_pre;
+    bw.gbox = reinterpret_cast<float *>(static_cast<char *>(workspace) + off_gbox);
+    bw.bias_part = reinterpret_cast<float *>(static_cast<char *>(workspace) + off_part);
+    const int total = d.nslice * d.ntile;
+    const int grid = std::min(std::min(total, ebfi::sm_count()), BWD_MAX_GRID);
+    const int per = ceil_div(total, grid);
+    if (int rc = launch_fused<true>(d, st, tmap, workspace, conv_bias, event_feat, static_cast<T *>(nullptr), bw, per))
+        return rc;
+    kpn_gev_collect<<<ebfi::sm_count() * 8, 256, 0, st>>>(bw.gbox, grad_event_fac, d);
+    EBFI_LAUNCH_OK("kpn_gev_collect");
+    kpn_bias_collect<<<ceil_div(d.Ce * d.KK, 128), 128, 0, st>>>(bw.bias_part, grad_bias, d, per);
+    EBFI_LAUNCH_OK("kpn_bias_collect");
     return EBFI_OK;
 }
 
@@ -582,20 +654,19 @@ int ebfi_kpn_fused_forward(void *stream, const float *event_feat, const float *f
                            int channels_event, int channels_frame, int height, int width, int kernel_size,
                            void *workspace, size_t workspace_bytes)
 {
-    KpnDims d{};
-    if (int rc = fill(d, batch, channels_event, channels_frame, height, width, kernel_size, negative_slope)) return rc;
-    EBFI_REQUIRE(event_feat && (frame_feat || channels_frame == 0) && conv_weight && conv_bias && output,
-                 "kpn_fused: null pointer");
-    const size_t need = ws_weights(d) + ws_input(d);
-    if (!workspace || workspace_bytes < need)
-        return ebfi::fail(EBFI_ERR_WORKSPACE, "kpn_fused: workspace %zu < %zu bytes", workspace_bytes, need);
-    EBFI_REQUIRE(ebfi::aligned16(workspace), "kpn_fused: workspace must be 16-byte aligned");
-    cudaStream_t st = ebfi::as_stream(stream);
-    CUtensorMap tmap;
-    if (int rc = prep_operands(d, st, event_feat, frame_feat, conv_weight, workspace, tmap)) return rc;
-    const int total = d.nslice * d.ntile;
-    const int grid = std::min(total, ebfi::sm_count());
-    return launch_fused<false>(d, st, tmap, workspace, conv_bias, event_feat, output, KpnBwdArgs{}, ceil_div(total, grid));
+    return kpn_forward(stream, event_feat, frame_feat, conv_weight, conv_bias, negative_slope, output, batch,
+                       channels_event, channels_frame, height, width, kernel_size, workspace, workspace_bytes);
+}
+
+int ebfi_kpn_fused_forward_bf16(void *stream, const void *event_feat, const void *frame_feat, const float *conv_weight,
+                                const float *conv_bias, float negative_slope, void *output, int batch,
+                                int channels_event, int channels_frame, int height, int width, int kernel_size,
+                                void *workspace, size_t workspace_bytes)
+{
+    return kpn_forward(stream, static_cast<const __nv_bfloat16 *>(event_feat),
+                       static_cast<const __nv_bfloat16 *>(frame_feat), conv_weight, conv_bias, negative_slope,
+                       static_cast<__nv_bfloat16 *>(output), batch, channels_event, channels_frame, height, width,
+                       kernel_size, workspace, workspace_bytes);
 }
 
 size_t ebfi_kpn_fused_backward_workspace_bytes(int batch, int channels_event, int channels_frame, int height, int width,
@@ -611,33 +682,22 @@ int ebfi_kpn_fused_backward(void *stream, const float *event_feat, const float *
                             float *grad_event_fac, float *grad_bias, int batch, int channels_event, int channels_frame,
                             int height, int width, int kernel_size, void *workspace, size_t workspace_bytes)
 {
-    KpnDims d{};
-    if (int rc = fill(d, batch, channels_event, channels_frame, height, width, kernel_size, negative_slope)) return rc;
-    EBFI_REQUIRE(event_feat && (frame_feat || channels_frame == 0) && conv_weight && conv_bias && grad_output &&
-                 grad_pre && grad_event_fac && grad_bias, "kpn_fused_backward: null pointer");
-    const size_t off_gbox = ws_weights(d) + ebfi::round_up(ws_input(d), (size_t)256);
-    const size_t off_part = off_gbox + ws_gbox(d);
-    const size_t need = off_part + ws_bias_part(d);
-    if (!workspace || workspace_bytes < need)
-        return ebfi::fail(EBFI_ERR_WORKSPACE, "kpn_fused_backward: workspace %zu < %zu bytes", workspace_bytes, need);
-    EBFI_REQUIRE(ebfi::aligned16(workspace), "kpn_fused_backward: workspace must be 16-byte aligned");
-    cudaStream_t st = ebfi::as_stream(stream);
-    CUtensorMap tmap;
-    if (int rc = prep_operands(d, st, event_feat, frame_feat, conv_weight, workspace, tmap)) return rc;
-    KpnBwdArgs bw;
-    bw.gout = grad_output;
-    bw.gpre = grad_pre;
-    bw.gbox = reinterpret_cast<float *>(static_cast<char *>(workspace) + off_gbox);
-    bw.bias_part = reinterpret_cast<float *>(static_cast<char *>(workspace) + off_part);
-    const int total = d.nslice * d.ntile;
-    const int grid = std::min(std::min(total, ebfi::sm_count()), BWD_MAX_GRID);
-    const int per = ceil_div(total, grid);
-    if (int rc = launch_fused<true>(d, st, tmap, workspace, conv_bias, event_feat, nullptr, bw, per)) return rc;
-    kpn_gev_collect<<<ebfi::sm_count() * 8, 256, 0, st>>>(bw.gbox, grad_event_fac, d);
-    EBFI_LAUNCH_OK("kpn_gev_collect");
-    kpn_bias_collect<<<ceil_div(d.Ce * d.KK, 128), 128, 0, st>>>(bw.bias_part, grad_bias, d, per);
-    EBFI_LAUNCH_OK("kpn_bias_collect");
-    return EBFI_OK;
+    return kpn_backward(stream, event_feat, frame_feat, conv_weight, conv_bias, negative_slope, grad_output, grad_pre,
+                        grad_event_fac, grad_bias, batch, channels_event, channels_frame, height, width, kernel_size,
+                        workspace, workspace_bytes);
+}
+
+int ebfi_kpn_fused_backward_bf16(void *stream, const void *event_feat, const void *frame_feat, const float *conv_weight,
+                                 const float *conv_bias, float negative_slope, const void *grad_output, void *grad_pre,
+                                 float *grad_event_fac, float *grad_bias, int batch, int channels_event,
+                                 int channels_frame, int height, int width, int kernel_size, void *workspace,
+                                 size_t workspace_bytes)
+{
+    return kpn_backward(stream, static_cast<const __nv_bfloat16 *>(event_feat),
+                        static_cast<const __nv_bfloat16 *>(frame_feat), conv_weight, conv_bias, negative_slope,
+                        static_cast<const __nv_bfloat16 *>(grad_output), static_cast<__nv_bfloat16 *>(grad_pre),
+                        grad_event_fac, grad_bias, batch, channels_event, channels_frame, height, width, kernel_size,
+                        workspace, workspace_bytes);
 }
 
 }  // extern "C"

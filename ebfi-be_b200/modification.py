@@ -8,7 +8,10 @@ is the same forward with a fused backward (ebfi_kpn_fused_backward): the kernel 
 on the tensor cores and writes dL/dP, the FAC/ReplicationPad part of dL/dEvent and dL/dbias; the conv's own weight
 and input gradients then run on torch's convolution backward, as the reference's nn.Conv2d does. Neither the
 pre-activation nor the kernel tensor is kept for the backward. `KernelPrediction.fused_backward = True` trains
-through it; by default the module trains on the reference's op sequence.
+through it; by default the module trains on the reference's op sequence. `KernelConvFACBF16Function` is the same
+fused forward and backward for bf16 activations (torch.autocast's mixed precision): the kernel reads and writes bf16
+activations and keeps P and the kernel tensor in fp32 registers, and the conv's gradients run as the bf16 convolution
+backward autocast's nn.Conv2d would run.
 """
 import torch
 from torch import nn
@@ -18,22 +21,19 @@ from .kernelconv2d import KernelConv2D
 
 
 def kernelconv_fac_fused(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope=0.01):
-    """out = KernelConv2D(K)(event_feat, LeakyReLU(conv3x3(cat([event_feat, frame_feat], 1)))) — fp32 CUDA tensors;
-    conv operands are rounded to bf16 for the tensor cores (fp32 accumulate, fp32 FAC)."""
+    """out = KernelConv2D(K)(event_feat, LeakyReLU(conv3x3(cat([event_feat, frame_feat], 1)))) — CUDA tensors, all fp32
+    or all bf16; conv operands are rounded to bf16 for the tensor cores (fp32 accumulate, fp32 FAC)."""
     L.require_cuda(event_feat, frame_feat, conv_weight, conv_bias)
     dts = {t.dtype for t in (event_feat, frame_feat, conv_weight, conv_bias)}
-    if dts == {torch.bfloat16}:
-        # bfloat16 model (the 720p inference config): the kernel's conv operands are bf16 anyway, so the values are used
-        # exactly; the fp32 staging copies and the final rounding of the output to bf16 happen at this boundary
-        return kernelconv_fac_fused(event_feat.float(), frame_feat.float(), conv_weight.float(), conv_bias.float(),
-                                    kernel_size, negative_slope).bfloat16()
-    if dts != {torch.float32}:
+    if dts != {torch.float32} and dts != {torch.bfloat16}:
         raise RuntimeError("kernelconv_fac_fused: all tensors must be float32 or all bfloat16, got "
                            f"{sorted(str(d) for d in dts)}")
     if torch.is_grad_enabled() and any(t.requires_grad for t in (event_feat, frame_feat, conv_weight, conv_bias)):
         raise RuntimeError("kernelconv_fac_fused is forward-only; run it under torch.no_grad() "
                            "(training goes through KernelConv2DFunction)")
-    return _fused_forward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope)
+    # bfloat16 model (the 720p inference config): the kernel reads the bf16 activations and rounds its output once;
+    # the weights' fp32 copies are exact (and small)
+    return _fused_forward(event_feat, frame_feat, conv_weight.float(), conv_bias.float(), kernel_size, negative_slope)
 
 
 def _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, what):
@@ -48,7 +48,9 @@ def _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, wha
 
 
 def _fused_forward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope):
-    """ebfi_kpn_fused_forward on fp32 CUDA tensors: the one forward of kernelconv_fac_fused and KernelConvFACFunction."""
+    """ebfi_kpn_fused_forward (fp32 activations) or ebfi_kpn_fused_forward_bf16 (bf16 activations) on CUDA tensors
+    with fp32 weight and bias: the one forward of kernelconv_fac_fused, KernelConvFACFunction and
+    KernelConvFACBF16Function. The output has the activations' dtype."""
     B, Ce, Cf, H, W, K = _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, "kernelconv_fac_fused")
     event_feat, frame_feat, conv_weight, conv_bias = (t.contiguous() for t in (event_feat, frame_feat, conv_weight, conv_bias))
     lib = L.load()
@@ -56,9 +58,10 @@ def _fused_forward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, 
         out = torch.empty_like(event_feat)
         nbytes = lib.ebfi_kpn_fused_workspace_bytes(B, Ce, Cf, H, W, K)
         ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=event_feat.device)
-        L.check(lib.ebfi_kpn_fused_forward(L.stream_ptr(event_feat.device), L.ptr(event_feat), L.ptr(frame_feat),
-                                           L.ptr(conv_weight), L.ptr(conv_bias), float(negative_slope), L.ptr(out),
-                                           B, Ce, Cf, H, W, K, L.ptr(ws), nbytes), "kernelconv_fac_fused")
+        fwd = lib.ebfi_kpn_fused_forward_bf16 if event_feat.dtype == torch.bfloat16 else lib.ebfi_kpn_fused_forward
+        L.check(fwd(L.stream_ptr(event_feat.device), L.ptr(event_feat), L.ptr(frame_feat),
+                    L.ptr(conv_weight), L.ptr(conv_bias), float(negative_slope), L.ptr(out),
+                    B, Ce, Cf, H, W, K, L.ptr(ws), nbytes), "kernelconv_fac_fused")
     return out
 
 
@@ -70,24 +73,54 @@ def kernelconv_fac_fused_backward(event_feat, frame_feat, conv_weight, conv_bias
     L.require_cuda(event_feat, frame_feat, conv_weight, conv_bias, grad_output)
     L.require_f32(event_feat=event_feat, frame_feat=frame_feat, conv_weight=conv_weight, conv_bias=conv_bias,
                   grad_output=grad_output)
-    B, Ce, Cf, H, W, K = _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size,
-                                     "kernelconv_fac_fused_backward")
+    return _fused_backward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope, grad_output,
+                           "kernelconv_fac_fused_backward")
+
+
+def kernelconv_fac_fused_backward_bf16(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope,
+                                       grad_output):
+    """ebfi_kpn_fused_backward_bf16: kernelconv_fac_fused_backward for bf16 event_feat, frame_feat and grad_output
+    (weight and bias fp32 or bf16; they are used as fp32) -> (grad_pre bf16, grad_event_fac fp32, grad_bias fp32).
+    grad_pre is the fp32 kernel's grad_pre rounded once to bf16; grad_event_fac and grad_bias are the fp32 kernel's."""
+    L.require_cuda(event_feat, frame_feat, conv_weight, conv_bias, grad_output)
+    _require_bf16_io("kernelconv_fac_fused_backward_bf16", dict(event_feat=event_feat, frame_feat=frame_feat,
+                                                                grad_output=grad_output),
+                     dict(conv_weight=conv_weight, conv_bias=conv_bias))
+    return _fused_backward(event_feat, frame_feat, conv_weight.float(), conv_bias.float(), kernel_size,
+                           negative_slope, grad_output, "kernelconv_fac_fused_backward_bf16")
+
+
+def _require_bf16_io(what, activations, parameters):
+    """bf16 activations; parameters fp32 (autocast) or bf16 (a .bfloat16() model)."""
+    for k, t in activations.items():
+        if t.dtype != torch.bfloat16:
+            raise RuntimeError(f"{what}: {k} must be bfloat16, got {t.dtype} "
+                               "(fp32 activations go through the fp32 entries)")
+    for k, t in parameters.items():
+        if t.dtype not in (torch.float32, torch.bfloat16):
+            raise RuntimeError(f"{what}: {k} must be float32 or bfloat16, got {t.dtype}")
+
+
+def _fused_backward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope, grad_output, what):
+    """ebfi_kpn_fused_backward or its _bf16 variant, chosen by the activations' dtype; fp32 weight and bias."""
+    B, Ce, Cf, H, W, K = _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, what)
     if tuple(grad_output.shape) != tuple(event_feat.shape):
-        raise RuntimeError("kernelconv_fac_fused_backward: grad_output must have the event features' shape")
+        raise RuntimeError(f"{what}: grad_output must have the event features' shape")
     event_feat, frame_feat, conv_weight, conv_bias, grad_output = (
         t.contiguous() for t in (event_feat, frame_feat, conv_weight, conv_bias, grad_output))
     lib = L.load()
     dev = event_feat.device
     with torch.cuda.device(dev):
-        grad_pre = torch.empty(B, Ce * K * K, H, W, device=dev)
-        grad_event_fac = torch.empty_like(event_feat)
+        grad_pre = torch.empty(B, Ce * K * K, H, W, device=dev, dtype=event_feat.dtype)
+        grad_event_fac = torch.empty(B, Ce, H, W, device=dev)
         grad_bias = torch.empty(Ce * K * K, device=dev)
         nbytes = lib.ebfi_kpn_fused_backward_workspace_bytes(B, Ce, Cf, H, W, K)
         ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
-        L.check(lib.ebfi_kpn_fused_backward(L.stream_ptr(dev), L.ptr(event_feat), L.ptr(frame_feat), L.ptr(conv_weight),
-                                            L.ptr(conv_bias), float(negative_slope), L.ptr(grad_output),
-                                            L.ptr(grad_pre), L.ptr(grad_event_fac), L.ptr(grad_bias),
-                                            B, Ce, Cf, H, W, K, L.ptr(ws), nbytes), "kernelconv_fac_fused_backward")
+        bwd = lib.ebfi_kpn_fused_backward_bf16 if event_feat.dtype == torch.bfloat16 else lib.ebfi_kpn_fused_backward
+        L.check(bwd(L.stream_ptr(dev), L.ptr(event_feat), L.ptr(frame_feat), L.ptr(conv_weight),
+                    L.ptr(conv_bias), float(negative_slope), L.ptr(grad_output),
+                    L.ptr(grad_pre), L.ptr(grad_event_fac), L.ptr(grad_bias),
+                    B, Ce, Cf, H, W, K, L.ptr(ws), nbytes), what)
     return grad_pre, grad_event_fac, grad_bias
 
 
@@ -127,6 +160,49 @@ class KernelConvFACFunction(torch.autograd.Function):
                 None, None)
 
 
+class KernelConvFACBF16Function(torch.autograd.Function):
+    """KernelConvFACFunction for bf16 activations, as torch.autocast(dtype=torch.bfloat16) feeds the block:
+    event_feat and frame_feat bf16; conv_weight and conv_bias fp32 (autocast parameters) or bf16 (a .bfloat16()
+    model); all CUDA. Returns bf16.
+
+    Saves only the four inputs. The forward and the fused backward kernel read the bf16 activations and use the
+    weights as fp32 (exact for bf16 ones); P and LeakyReLU(P) stay fp32 in registers, the output and dL/dP are
+    rounded once to bf16. The conv's weight and input gradients are the bf16 convolution backward of dL/dP that
+    autocast's nn.Conv2d runs (bf16 cat(event, frame), bf16 weight). grad_event = (FAC part + conv part) summed in
+    fp32 and rounded once; weight and bias gradients come back in the parameters' dtype. The backward does not
+    depend on the autocast state it runs under."""
+
+    @staticmethod
+    def forward(ctx, event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope=0.01):
+        L.require_cuda(event_feat, frame_feat, conv_weight, conv_bias)
+        _require_bf16_io("KernelConvFACBF16Function", dict(event_feat=event_feat, frame_feat=frame_feat),
+                         dict(conv_weight=conv_weight, conv_bias=conv_bias))
+        ctx.kernel_size, ctx.negative_slope = int(kernel_size), float(negative_slope)
+        ctx.save_for_backward(event_feat, frame_feat, conv_weight, conv_bias)
+        return _fused_forward(event_feat, frame_feat, conv_weight.float(), conv_bias.float(), kernel_size,
+                              negative_slope)
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        ev, fr, w, b = ctx.saved_tensors
+        need_ev, need_fr, need_w, need_b = ctx.needs_input_grad[:4]
+        with torch.autocast("cuda", enabled=False):
+            grad_pre, grad_ev, grad_b = kernelconv_fac_fused_backward_bf16(
+                ev, fr, w, b, ctx.kernel_size, ctx.negative_slope, grad_output.bfloat16())
+            need_x = need_ev or need_fr
+            grad_x = grad_w = grad_fr = None
+            if need_x or need_w:
+                x = torch.cat([ev, fr], 1) if fr.shape[1] else ev
+                grad_x, grad_w, _ = torch.ops.aten.convolution_backward(
+                    grad_pre, x, w.bfloat16(), None, [1, 1], [1, 1], [1, 1], False, [0, 0], 1, [need_x, need_w, False])
+            if need_x:
+                Ce = ev.shape[1]
+                grad_ev = (grad_ev + grad_x[:, :Ce].float()).bfloat16()
+                grad_fr = grad_x[:, Ce:] if need_fr else None
+        return (grad_ev if need_ev else None, grad_fr, grad_w.to(w.dtype) if need_w else None,
+                grad_b.to(b.dtype) if need_b else None, None, None)
+
+
 def kernelconv_fac_fused_supported(channels_event, channels_frame, kernel_size):
     """Shapes `ebfi_kpn_fused_forward` accepts (csrc/kpn.cu `fill`): odd K <= 5, (Ce + Cf) a multiple of 32 and <= 128."""
     K, cin = int(kernel_size), int(channels_event) + int(channels_frame)
@@ -160,7 +236,11 @@ class KernelPrediction(nn.Module):
     a supported shape train through `KernelConvFACFunction` (fused forward and backward; nothing but the inputs is
     kept for the backward). Opt-in because it changes training precision: the pre-activation comes from bf16 conv
     operands, so the gradients differ more from the fp64 op sequence than the TF32 reference sequence's do (measured
-    ratio in DESIGN §3). Every other case does exactly what it does with `fused_backward = False`."""
+    ratio in DESIGN §3). With bf16 event and frame tensors (torch.autocast(dtype=torch.bfloat16) mixed precision, or
+    a .bfloat16() model) and fp32 or bf16 parameters, the same opt-in trains through `KernelConvFACBF16Function`
+    instead: bf16 activation I/O, P and the kernel tensor in fp32 registers, the conv's gradients as autocast's bf16
+    convolution backward (precision and measured numbers in DESIGN §3). Every other case does exactly what it does with
+    `fused_backward = False`."""
 
     fused = True
     fused_backward = False
@@ -185,5 +265,11 @@ class KernelPrediction(nn.Module):
                 and kernelconv_fac_fused_supported(EventTensor.shape[1], FrameTensor.shape[1], self.kernel_size):
             return KernelConvFACFunction.apply(EventTensor, FrameTensor, conv.weight, conv.bias, self.kernel_size,
                                                self.KernelConv.activation.negative_slope)
+        if self.fused_backward and needs_grad and EventTensor.is_cuda and EventTensor.dtype == torch.bfloat16 \
+                and FrameTensor.dtype == torch.bfloat16 and conv.weight.dtype in (torch.float32, torch.bfloat16) \
+                and conv.bias.dtype == conv.weight.dtype \
+                and kernelconv_fac_fused_supported(EventTensor.shape[1], FrameTensor.shape[1], self.kernel_size):
+            return KernelConvFACBF16Function.apply(EventTensor, FrameTensor, conv.weight, conv.bias, self.kernel_size,
+                                                   self.KernelConv.activation.negative_slope)
         Kernel = self.KernelConv(torch.cat([EventTensor, FrameTensor], dim=1))
         return self.KPN(EventTensor, Kernel)

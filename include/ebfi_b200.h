@@ -217,6 +217,22 @@ int ebfi_kpn_fused_backward(void *stream, const float *event_feat, const float *
                             int batch, int channels_event, int channels_frame, int height, int width,
                             int kernel_size, void *workspace, size_t workspace_bytes);
 
+/* bf16 activation variants of the two entries above (mixed precision: bf16 activations, fp32 parameters), same
+ * argument order. event_feat, frame_feat, output, grad_output and grad_pre are `__nv_bfloat16*`; conv_weight,
+ * conv_bias, grad_event_fac and grad_bias stay fp32. Only the activation loads and stores change: loads widen
+ * exactly, output and grad_pre are rounded once (RN) from the fp32 values the fp32 entries store, so on bf16-valued
+ * inputs the results equal the fp32 entries' results rounded to bf16 (grad_event_fac, grad_bias: equal). Workspace
+ * sizes are those of ebfi_kpn_fused_workspace_bytes / ebfi_kpn_fused_backward_workspace_bytes. */
+int ebfi_kpn_fused_forward_bf16(void *stream, const void *event_feat, const void *frame_feat,
+                                const float *conv_weight, const float *conv_bias, float negative_slope,
+                                void *output, int batch, int channels_event, int channels_frame,
+                                int height, int width, int kernel_size, void *workspace, size_t workspace_bytes);
+int ebfi_kpn_fused_backward_bf16(void *stream, const void *event_feat, const void *frame_feat,
+                                 const float *conv_weight, const float *conv_bias, float negative_slope,
+                                 const void *grad_output, void *grad_pre, float *grad_event_fac, float *grad_bias,
+                                 int batch, int channels_event, int channels_frame, int height, int width,
+                                 int kernel_size, void *workspace, size_t workspace_bytes);
+
 /* ---- event encoders --------------------------------------------------------- */
 
 /* Coordinate / timestamp arrays may be fp32 or fp64, like the tensors the

@@ -8,9 +8,15 @@ channels, 256x256, K=5) and the cfg5 block shape (B=8, 128x128). Prints one JSON
   *_peak_mb         torch.cuda.max_memory_allocated over forward + backward, above what was allocated before
 and the device name and power limit read in the same run.
 
-    python tools/time_kpn_train.py [--reps 15]
+--bf16 times the same two workloads in mixed precision: bf16 event / frame tensors and fp32 parameters under
+torch.autocast(dtype=torch.bfloat16), the autocast op sequence (bf16 cuDNN conv, bf16 LeakyReLU and FAC) against
+fused_backward=True (KernelConvFACBF16Function: bf16 fused kernels + bf16 cuDNN dgrad/wgrad of the bf16 grad_pre);
+the reference_* keys then hold the autocast sequence.
+
+    python tools/time_kpn_train.py [--reps 15] [--bf16]
 """
 import argparse
+import contextlib
 import json
 import os
 import re
@@ -32,6 +38,7 @@ def device_info():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=15)
+    ap.add_argument("--bf16", action="store_true", help="bf16 activations under torch.autocast (mixed precision)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("time_kpn_train.py needs a CUDA device")
@@ -52,20 +59,24 @@ def main():
         return ts[len(ts) // 2]
 
     info = device_info()
+    act = torch.bfloat16 if args.bf16 else torch.float32
+    amp = (lambda: torch.autocast("cuda", dtype=torch.bfloat16)) if args.bf16 else contextlib.nullcontext
     for (B, H, W) in [(4, 256, 256), (8, 128, 128)]:
         C, K = 64, 5
         torch.manual_seed(0)
         m = modification.KernelPrediction(C, K).to(dev)
         conv = m.KernelConv.conv2d
-        ev = torch.randn(B, C, H, W, device=dev, requires_grad=True)
-        fr = torch.randn(B, C, H, W, device=dev, requires_grad=True)
-        G = torch.randn(B, C, H, W, device=dev)
+        ev = torch.randn(B, C, H, W, device=dev).to(act).requires_grad_()
+        fr = torch.randn(B, C, H, W, device=dev).to(act).requires_grad_()
+        G = torch.randn(B, C, H, W, device=dev).to(act)
 
         def step(fused):
             m.fused_backward = fused
             ev.grad = fr.grad = None
             m.zero_grad(set_to_none=True)
-            m(ev, fr).backward(G)
+            with amp():
+                out = m(ev, fr)
+            out.backward(G)
 
         for fused in (False, True, False, True):          # warm-up: cuDNN algorithm choice, module loads
             step(fused)
@@ -86,15 +97,19 @@ def main():
             peak[fused] = (torch.cuda.max_memory_allocated() - base) / 2 ** 20
 
         # backward pieces of the fused path, each alone
+        # (bf16: the calls KernelConvFACBF16Function makes — bf16 activations, fp32 weights for the fused kernels,
+        # bf16 weights for cuDNN's convolution backward)
         evd, frd, w, b = ev.detach(), fr.detach(), conv.weight.detach(), conv.bias.detach()
-        x = torch.cat([evd, frd], 1)
-        gpre = modification.kernelconv_fac_fused_backward(evd, frd, w, b, K, 0.01, G)[0]
+        x, wc = torch.cat([evd, frd], 1), w.to(act)
+        fused_bwd = modification.kernelconv_fac_fused_backward_bf16 if args.bf16 else \
+            modification.kernelconv_fac_fused_backward
+        gpre = fused_bwd(evd, frd, w, b, K, 0.01, G)[0]
         pieces = {
-            "fused_forward": lambda: modification.kernelconv_fac_fused(evd, frd, w, b, K, 0.01),
-            "kpn_fused_backward": lambda: modification.kernelconv_fac_fused_backward(evd, frd, w, b, K, 0.01, G),
-            "cudnn_dgrad": lambda: torch.ops.aten.convolution_backward(gpre, x, w, None, [1, 1], [1, 1], [1, 1], False,
+            "fused_forward": lambda: modification._fused_forward(evd, frd, w, b, K, 0.01),
+            "kpn_fused_backward": lambda: fused_bwd(evd, frd, w, b, K, 0.01, G),
+            "cudnn_dgrad": lambda: torch.ops.aten.convolution_backward(gpre, x, wc, None, [1, 1], [1, 1], [1, 1], False,
                                                                        [0, 0], 1, [True, False, False]),
-            "cudnn_wgrad": lambda: torch.ops.aten.convolution_backward(gpre, x, w, None, [1, 1], [1, 1], [1, 1], False,
+            "cudnn_wgrad": lambda: torch.ops.aten.convolution_backward(gpre, x, wc, None, [1, 1], [1, 1], [1, 1], False,
                                                                        [0, 0], 1, [False, True, False]),
         }
         with torch.no_grad():
@@ -113,6 +128,7 @@ def main():
         del gpre, x
 
         res = {"workload": f"B={B} Ce=Cf={C} K={K} {H}x{W}",
+               "precision": "bf16 activations, fp32 parameters, autocast" if args.bf16 else "fp32",
                "reference_fwd_bwd_ms": round(median(ts[False]), 4), "fused_fwd_bwd_ms": round(median(ts[True]), 4),
                "bwd_breakdown_ms": breakdown, "kpn_kernels_ms": kernels,
                "reference_peak_mb": round(peak[False], 1), "fused_peak_mb": round(peak[True], 1),
