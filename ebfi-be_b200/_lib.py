@@ -26,6 +26,7 @@ class DcnGeom(ctypes.Structure):
 
 EBFI_DCN_DETERMINISTIC = 1
 EBFI_DCN_INPUT_BLOCKED = 2
+EBFI_ERR_UNSUPPORTED = -4
 
 
 class DpComm(ctypes.Structure):
@@ -52,6 +53,11 @@ SIGNATURES = {
     "ebfi_dp_complete": (c_int, [c_void, ctypes.POINTER(DpComm), c_void, c_size, c_void, c_size]),
     "ebfi_dcnv2_forward_packed": (c_int, [c_void, _GEOM_P] + [c_void] * 6 + [c_void, c_size]),
     "ebfi_dcnv2_backward_packed": (c_int, [c_void, _GEOM_P] + [c_void] * 9 + [c_void, c_size]),
+    "ebfi_dcnv2_forward_bf16": (c_int, [c_void, _GEOM_P] + [c_void] * 6 + [c_void, c_size]),
+    "ebfi_dcnv2_backward_bf16": (c_int, [c_void, _GEOM_P] + [c_void] * 11 + [c_void, c_size]),
+    "ebfi_dcnv2_backward_dp_bf16": (c_int, [c_void, _GEOM_P] + [c_void] * 11 + [c_void, c_size, ctypes.POINTER(DpComm), c_int]),
+    "ebfi_dcnv2_forward_packed_bf16": (c_int, [c_void, _GEOM_P] + [c_void] * 6 + [c_void, c_size]),
+    "ebfi_dcnv2_backward_packed_bf16": (c_int, [c_void, _GEOM_P] + [c_void] * 9 + [c_void, c_size]),
     "ebfi_fac_forward": (c_int, [c_void] * 4 + [c_int] * 5),
     "ebfi_fac_backward_workspace_bytes": (c_size, [c_int] * 5),
     "ebfi_fac_backward": (c_int, [c_void] * 6 + [c_int] * 5 + [c_void, c_size]),

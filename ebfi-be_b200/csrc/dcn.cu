@@ -25,18 +25,22 @@
 #include "dp_comm.cuh"
 
 #include <algorithm>
+#include <type_traits>
 
 namespace ebfi_dcn {
-// tensor-core forward (dcn_tc.cu); returns EBFI_ERR_UNSUPPORTED when the shape is not eligible
-int forward_tc(cudaStream_t st, const DcnDims &d, const float *input, const float *weight, const float *bias,
-               const float *offset, const float *mask, float *output, void *workspace, size_t workspace_bytes);
+// tensor-core forward (dcn_fwd_box.cu); returns EBFI_ERR_UNSUPPORTED when the shape is not eligible.
+// T = float | __nv_bfloat16: the type of input, offset, mask and output.
+template <typename T>
+int forward_tc(cudaStream_t st, const DcnDims &d, const T *input, const float *weight, const float *bias,
+               const T *offset, const T *mask, T *output, void *workspace, size_t workspace_bytes);
 size_t forward_tc_workspace(const DcnDims &d);
 size_t forward_tc_blocked_offset(const DcnDims &d);
 // tensor-core backward (dcn_bwd_tc.cu); splits == 0 when the shape is not eligible
 int backward_box_splits(const DcnDims &d);
 size_t backward_box_scratch_bytes(const DcnDims &d);
-int backward_box(cudaStream_t st, const DcnDims &d, const float *input, const float *weight, const float *offset,
-                 const float *mask, const float *gout, float *gin, float *goff, float *gmask, float *gw, float *gb,
+template <typename T>
+int backward_box(cudaStream_t st, const DcnDims &d, const T *input, const float *weight, const T *offset,
+                 const T *mask, const T *gout, T *gin, T *goff, T *gmask, float *gw, float *gb,
                  float *gw_part, float *gb_part, void *scratch, const ebfi_dp::View *dp, bool dp_defer);
 int backward_tc_splits(const DcnDims &d);
 size_t backward_tc_scratch_bytes(const DcnDims &d);
@@ -487,31 +491,47 @@ size_t ebfi_dcnv2_forward_workspace_bytes(const ebfi_dcn_geom *q)
     return forward_tc_workspace(d) + 256;
 }
 
-static int run_forward(void *stream, const DcnDims &d, const float *input, const float *weight,
-                       const float *bias, const float *offset, const float *mask, float *output,
+}  // extern "C"
+
+// T = float: every shape. T = __nv_bfloat16 (the *_bf16 entries): only where the tensor-core kernels run; anything else
+// returns EBFI_ERR_UNSUPPORTED before the first launch, and the caller runs the float entry on widened copies.
+template <typename T>
+static int run_forward(void *stream, const DcnDims &d, const T *input, const float *weight,
+                       const float *bias, const T *offset, const T *mask, T *output,
                        void *workspace, size_t workspace_bytes)
 {
     EBFI_REQUIRE(input && weight && bias && offset && mask && output, "dcn_forward: null pointer");
     cudaStream_t st = ebfi::as_stream(stream);
-    if (d.abs_sum) EBFI_CUDA_OK(cudaMemsetAsync(d.abs_sum, 0, sizeof(float), st));
     // Tensor-core path (dcn_tc.cu) for the shapes it covers; EBFI_DCN_IMPL=simt forces the
     // CUDA-core kernel below, which handles every shape.
     const char *impl = getenv("EBFI_DCN_IMPL");
-    if (!(impl && impl[0] == 's')) {
-        const int rc = forward_tc(st, d, input, weight, bias, offset, mask, output, workspace, workspace_bytes);
+    const bool simt = impl && impl[0] == 's';
+    if constexpr (!std::is_same_v<T, float>) {
+        const size_t need = forward_tc_workspace(d);
+        if (simt || need == 0 || !workspace || workspace_bytes < need || (reinterpret_cast<uintptr_t>(workspace) & 31u))
+            return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_forward_bf16: no tensor-core forward for this call");
+    }
+    if (d.abs_sum) EBFI_CUDA_OK(cudaMemsetAsync(d.abs_sum, 0, sizeof(float), st));
+    if (!simt) {
+        const int rc = forward_tc<T>(st, d, input, weight, bias, offset, mask, output, workspace, workspace_bytes);
         if (rc != EBFI_ERR_UNSUPPORTED) return rc;
     }
-    EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
-    dim3 grid(d.ntile, ceil_div(d.Co, COT), d.B);
-    dcn_fwd_kernel<<<grid, NT, kFwdSmem, st>>>(input, weight, bias, offset, mask, output, d);
-    EBFI_LAUNCH_OK("dcn_fwd_kernel");
-    return EBFI_OK;
+    if constexpr (std::is_same_v<T, float>) {
+        EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
+        dim3 grid(d.ntile, ceil_div(d.Co, COT), d.B);
+        dcn_fwd_kernel<<<grid, NT, kFwdSmem, st>>>(input, weight, bias, offset, mask, output, d);
+        EBFI_LAUNCH_OK("dcn_fwd_kernel");
+        return EBFI_OK;
+    } else {
+        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_forward_bf16: no tensor-core forward for this call");
+    }
 }
 
-static int run_backward(void *stream, const DcnDims &d_in, const float *input, const float *weight,
-                        const float *offset, const float *mask,
-                        const float *grad_output, float *grad_input, float *grad_offset,
-                        float *grad_mask, float *grad_weight, float *grad_bias,
+template <typename T>
+static int run_backward(void *stream, const DcnDims &d_in, const T *input, const float *weight,
+                        const T *offset, const T *mask,
+                        const T *grad_output, T *grad_input, T *grad_offset,
+                        T *grad_mask, float *grad_weight, float *grad_bias,
                         void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm = nullptr, bool dp_defer = false)
 {
     EBFI_REQUIRE(input && weight && offset && mask && grad_output && grad_input && grad_offset &&
@@ -523,10 +543,13 @@ static int run_backward(void *stream, const DcnDims &d_in, const float *input, c
     cudaStream_t st = ebfi::as_stream(stream);
     DcnDims d = d_in;
     const char *impl = getenv("EBFI_DCN_IMPL");
-    // the tensor-core backward stages grad_output with 128-bit loads: it needs a 16-byte aligned base
+    // the tensor-core backward stages grad_output with 128-bit loads (8 pixels: two for fp32, one for bf16, when a row is a
+    // whole number of 16-byte words): it needs a 16-byte aligned base for either element size
     const bool tc_ok = !(impl && impl[0] == 's') && ebfi::aligned16(grad_output);
     // box kernel (dcn_bwd_box.cu) first; the group-specialised kernel (dcn_bwd_tc.cu) serves the deterministic flag
     const int S_box = tc_ok ? backward_box_splits(d) : 0;
+    if (!std::is_same_v<T, float> && S_box == 0)
+        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_backward_bf16: no box backward for this call (shape, flags or alignment)");
     const int S_tc = S_box > 0 ? S_box : (tc_ok ? backward_tc_splits(d) : 0);
     const int S = S_tc > 0 ? S_tc : bwd_splits(d);
     if (d.in_blocked) {
@@ -549,53 +572,60 @@ static int run_backward(void *stream, const DcnDims &d_in, const float *input, c
     float *gw_part = static_cast<float *>(workspace);
     float *gb_part = gw_part + (size_t)S * n_w;
     char *scratch = static_cast<char *>(workspace) + part_bytes;
-    if (d.det) {
-        float *bound = reinterpret_cast<float *>(scratch + scratch_bytes);
-        EBFI_CUDA_OK(cudaMemsetAsync(bound, 0, 3 * sizeof(float), st));
-        dcn_det_bound<<<ebfi::sm_count() * 4, 256, 0, st>>>(grad_output, weight, mask, bound, d);
-        EBFI_LAUNCH_OK("dcn_det_bound");
-        d.det_bound = bound;
-    }
     if (S_box > 0) {
         // writes all five gradients, including its own fixed-order reduction of the weight-gradient partials
-        return backward_box(st, d, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
-                            grad_weight, grad_bias, gw_part, gb_part, scratch, dp, dp_defer);
-    } else if (S_tc > 0) {
-        // tensor-core path (dcn_bwd_tc.cu): cpg == 8, Cout == 64
-        if (int rc = backward_tc(st, d, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
-                                 gw_part, gb_part, S, scratch))
-            return rc;
-    } else {
-        // deterministic mode accumulates into an int64 NCHW copy in the scratch and converts at the end
-        float *gin_acc = d.det ? reinterpret_cast<float *>(scratch) : grad_input;
-        EBFI_CUDA_OK(cudaMemsetAsync(gin_acc, 0, n_in * (d.det ? sizeof(long long) : sizeof(float)), st));
-        EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmem));
-        EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmem));
-        const int n_cot = ceil_div(d.Co, COT);
-        // Chunks of one group accumulate into the same grad_offset / grad_mask elements; separate,
-        // stream-ordered launches keep that read-modify-write race-free. nchunk is 1 unless
-        // channels-per-group * taps exceeds the KC_MAX-row slab.
-        for (int ch = 0; ch < d.nchunk; ++ch) {
-            dim3 grid(S, d.dg, n_cot);
-            if (d.det)
-                dcn_bwd_kernel<true><<<grid, NT, kBwdSmem, st>>>(input, weight, offset, mask, grad_output, gin_acc,
-                                                                 grad_offset, grad_mask, gw_part, gb_part, d, ch);
-            else
-                dcn_bwd_kernel<false><<<grid, NT, kBwdSmem, st>>>(input, weight, offset, mask, grad_output, gin_acc,
-                                                                  grad_offset, grad_mask, gw_part, gb_part, d, ch);
-            EBFI_LAUNCH_OK("dcn_bwd_kernel");
-        }
-        if (d.det) {
-            dcn_i64_to_f32<<<ebfi::sm_count() * 8, 256, 0, st>>>(reinterpret_cast<const long long *>(gin_acc), grad_input, n_in, d);
-            EBFI_LAUNCH_OK("dcn_i64_to_f32");
-        }
+        return backward_box<T>(st, d, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
+                               grad_weight, grad_bias, gw_part, gb_part, scratch, dp, dp_defer);
     }
-    const int n = (int)(n_w + n_b);
-    dcn_reduce_partials<<<ceil_div(n, 256), 256, 0, st>>>(gw_part, gb_part, grad_weight, grad_bias, S, (int)n_w, (int)n_b);
-    EBFI_LAUNCH_OK("dcn_reduce_partials");
-    if (dp) return ebfi_dp::allreduce_sum(st, *dp, grad_weight, n_w, grad_bias, n_b, dp_defer ? 1 : 0);
-    return EBFI_OK;
+    if constexpr (!std::is_same_v<T, float>) {
+        return EBFI_ERR_UNSUPPORTED;      // not reached: a bf16 call without the box path returned above
+    } else {
+        if (d.det) {
+            float *bound = reinterpret_cast<float *>(scratch + scratch_bytes);
+            EBFI_CUDA_OK(cudaMemsetAsync(bound, 0, 3 * sizeof(float), st));
+            dcn_det_bound<<<ebfi::sm_count() * 4, 256, 0, st>>>(grad_output, weight, mask, bound, d);
+            EBFI_LAUNCH_OK("dcn_det_bound");
+            d.det_bound = bound;
+        }
+        if (S_tc > 0) {
+            // tensor-core path (dcn_bwd_tc.cu): cpg == 8, Cout == 64
+            if (int rc = backward_tc(st, d, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
+                                     gw_part, gb_part, S, scratch))
+                return rc;
+        } else {
+            // deterministic mode accumulates into an int64 NCHW copy in the scratch and converts at the end
+            float *gin_acc = d.det ? reinterpret_cast<float *>(scratch) : grad_input;
+            EBFI_CUDA_OK(cudaMemsetAsync(gin_acc, 0, n_in * (d.det ? sizeof(long long) : sizeof(float)), st));
+            EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmem));
+            EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBwdSmem));
+            const int n_cot = ceil_div(d.Co, COT);
+            // Chunks of one group accumulate into the same grad_offset / grad_mask elements; separate,
+            // stream-ordered launches keep that read-modify-write race-free. nchunk is 1 unless
+            // channels-per-group * taps exceeds the KC_MAX-row slab.
+            for (int ch = 0; ch < d.nchunk; ++ch) {
+                dim3 grid(S, d.dg, n_cot);
+                if (d.det)
+                    dcn_bwd_kernel<true><<<grid, NT, kBwdSmem, st>>>(input, weight, offset, mask, grad_output, gin_acc,
+                                                                     grad_offset, grad_mask, gw_part, gb_part, d, ch);
+                else
+                    dcn_bwd_kernel<false><<<grid, NT, kBwdSmem, st>>>(input, weight, offset, mask, grad_output, gin_acc,
+                                                                      grad_offset, grad_mask, gw_part, gb_part, d, ch);
+                EBFI_LAUNCH_OK("dcn_bwd_kernel");
+            }
+            if (d.det) {
+                dcn_i64_to_f32<<<ebfi::sm_count() * 8, 256, 0, st>>>(reinterpret_cast<const long long *>(gin_acc), grad_input, n_in, d);
+                EBFI_LAUNCH_OK("dcn_i64_to_f32");
+            }
+        }
+        const int n = (int)(n_w + n_b);
+        dcn_reduce_partials<<<ceil_div(n, 256), 256, 0, st>>>(gw_part, gb_part, grad_weight, grad_bias, S, (int)n_w, (int)n_b);
+        EBFI_LAUNCH_OK("dcn_reduce_partials");
+        if (dp) return ebfi_dp::allreduce_sum(st, *dp, grad_weight, n_w, grad_bias, n_b, dp_defer ? 1 : 0);
+        return EBFI_OK;
+    }
 }
+
+extern "C" {
 
 int ebfi_dcnv2_forward(void *stream, const ebfi_dcn_geom *q, const float *input, const float *weight,
                        const float *bias, const float *offset, const float *mask, float *output,
@@ -659,6 +689,76 @@ int ebfi_dcnv2_backward_packed(void *stream, const ebfi_dcn_geom *q, const float
     set_packed(d);
     return run_backward(stream, d, input, weight, offset_mask, offset_mask + m0, grad_output, grad_input,
                         grad_offset_mask, grad_offset_mask + m0, grad_weight, grad_bias, workspace, workspace_bytes);
+}
+
+// ---- bf16 activations (ebfi_b200.h): same geometry handling as the float entries above ----
+using bf16 = __nv_bfloat16;
+static const bf16 *cb(const void *p) { return static_cast<const bf16 *>(p); }
+static bf16 *mb(void *p) { return static_cast<bf16 *>(p); }
+
+int ebfi_dcnv2_forward_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                            const float *bias, const void *offset, const void *mask, void *output,
+                            void *workspace, size_t workspace_bytes)
+{
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    return run_forward(stream, d, cb(input), weight, bias, cb(offset), cb(mask), mb(output), workspace, workspace_bytes);
+}
+
+int ebfi_dcnv2_backward_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                             const float *bias, const void *offset, const void *mask,
+                             const void *grad_output, void *grad_input, void *grad_offset,
+                             void *grad_mask, float *grad_weight, float *grad_bias,
+                             void *workspace, size_t workspace_bytes)
+{
+    (void)bias;
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    return run_backward(stream, d, cb(input), weight, cb(offset), cb(mask), cb(grad_output), mb(grad_input),
+                        mb(grad_offset), mb(grad_mask), grad_weight, grad_bias, workspace, workspace_bytes);
+}
+
+int ebfi_dcnv2_backward_dp_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                                const float *bias, const void *offset, const void *mask,
+                                const void *grad_output, void *grad_input, void *grad_offset,
+                                void *grad_mask, float *grad_weight, float *grad_bias,
+                                void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm, int defer)
+{
+    (void)bias;
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    EBFI_REQUIRE(comm != nullptr, "dcn_backward_dp: null communicator");
+    return run_backward(stream, d, cb(input), weight, cb(offset), cb(mask), cb(grad_output), mb(grad_input),
+                        mb(grad_offset), mb(grad_mask), grad_weight, grad_bias, workspace, workspace_bytes, comm, defer != 0);
+}
+
+int ebfi_dcnv2_forward_packed_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                                   const float *bias, const void *offset_mask, void *output,
+                                   float *abs_offset_sum, void *workspace, size_t workspace_bytes)
+{
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    EBFI_REQUIRE(offset_mask != nullptr, "dcn_forward_packed: null pointer");
+    const bf16 *mask_logits = cb(offset_mask) + 2 * d.mask_bs;
+    set_packed(d);
+    d.abs_sum = abs_offset_sum;
+    return run_forward(stream, d, cb(input), weight, bias, cb(offset_mask), mask_logits, mb(output), workspace, workspace_bytes);
+}
+
+int ebfi_dcnv2_backward_packed_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                                    const float *bias, const void *offset_mask, const void *grad_output,
+                                    void *grad_input, void *grad_offset_mask, float *grad_weight, float *grad_bias,
+                                    void *workspace, size_t workspace_bytes)
+{
+    (void)bias;
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    EBFI_REQUIRE(offset_mask && grad_offset_mask, "dcn_backward_packed: null pointer");
+    const long long m0 = 2 * d.mask_bs;
+    set_packed(d);
+    return run_backward(stream, d, cb(input), weight, cb(offset_mask), cb(offset_mask) + m0, cb(grad_output),
+                        mb(grad_input), mb(grad_offset_mask), mb(grad_offset_mask) + m0, grad_weight, grad_bias,
+                        workspace, workspace_bytes);
 }
 
 }  // extern "C"

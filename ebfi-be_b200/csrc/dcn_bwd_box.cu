@@ -32,6 +32,11 @@
 //     the reference's atomicAdd, im2col_cuda.cu:249).
 // Non-finite gradients: a NaN/Inf anywhere in the (tile, group) makes the scale undefined; the box is then written as NaN
 // so that overflow checks on grad_input (AMP GradScaler) still fire.
+// Activation type T (float | __nv_bfloat16, the *_bf16 entries): offsets, masks and grad_output are read as T and widened
+// (a bf16 grad_output splits into hi = the value, lo = 0: the bits the float path stages for the widened tensor);
+// grad_offset / grad_mask and grad_input are rounded once from the fp32 values the float instantiation stores. With
+// several units per group the running fp32 sums of the owner threads then stay in shared memory until the group's
+// last unit. Boxes, partials, weights and grad_weight / grad_bias are fp32 in both.
 #include "dcn_box.cuh"
 #include "dcn_common.cuh"
 #include "dp_comm.cuh"
@@ -67,7 +72,7 @@ struct BoxBwdPlan {
     int wt_bytes;        // one group's W^T image, hi | lo
     int col_part;        // one bf16 image of the column operand
     int om_bytes, use_om_tma;
-    int off_q, off_col, off_box, off_acc, off_cnt, off_om, smem;
+    int off_q, off_col, off_box, off_acc, off_cnt, off_om, off_gsum, smem;
     int units, ncs, ncs_shift;      // 8-channel units (C / 8) = iterations per tile over all CTA rows; units per deformable group (2^shift)
 };
 
@@ -281,12 +286,12 @@ __device__ __forceinline__ void sample_bwd(const DcnDims &d, const SampleCtx &sc
 }
 
 // MULTI: more than one 8-channel unit per deformable group (the group's offset / mask gradients accumulate over its units)
-template <bool PACKED, bool MULTI>
+template <bool PACKED, bool MULTI, typename T>
 __global__ void __launch_bounds__(NTHR, 1)
 dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__restrict__ wimg,
-                   const float *__restrict__ offset, const float *__restrict__ mask,
-                   const float *__restrict__ gout, float *__restrict__ gin_blk, float *__restrict__ pbox,
-                   float *__restrict__ goff, float *__restrict__ gmask,
+                   const T *__restrict__ offset, const T *__restrict__ mask,
+                   const T *__restrict__ gout, float *__restrict__ gin_blk, float *__restrict__ pbox,
+                   T *__restrict__ goff, T *__restrict__ gmask,
                    float *__restrict__ gw_part, float *__restrict__ gb_part, DcnDims d, BoxBwdPlan pl,
                    const __grid_constant__ CUtensorMap tm_box, const __grid_constant__ CUtensorMap tm_off,
                    const __grid_constant__ CUtensorMap tm_mask)
@@ -298,7 +303,9 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
     unsigned char *boxes = smem + pl.off_box;                        // [2][BH][BW][8] fp32 input boxes
     int4 *acc4 = reinterpret_cast<int4 *>(smem + pl.off_acc);        // [BH][BW][8] fixed-point grad_input box
     int *cnt = reinterpret_cast<int *>(smem + pl.off_cnt);           // [2][BH][BW] samples per cell (first corner), by iteration parity
-    const float *oms = reinterpret_cast<const float *>(smem + pl.off_om);   // [2][3*KK planes][128 px]
+    const T *oms = reinterpret_cast<const T *>(smem + pl.off_om);           // [2][3*KK planes][128 px]
+    constexpr bool RUN_SUMS = MULTI && sizeof(T) != 4;
+    float *gsum = reinterpret_cast<float *>(smem + pl.off_gsum);             // RUN_SUMS: [3*KK][128 px] fp32 running sums
     // bar_w / bar_in: bulk copies landed; bar_d1: GEMM1 complete; bar_g3: GEMM3 complete (Q, col free);
     // q_full / col_full: the sampler warps have written Q / the column operand (one arrival per warp)
     __shared__ __align__(8) uint64_t bar_w[2], bar_in[2], bar_d1[2], bar_g3, q_full, col_full;
@@ -382,7 +389,7 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
         if (use_tma) {
             unsigned char *dst = smem + pl.off_om + bb * pl.om_bytes;
             tma::load_3d(dst, &tm_off, it.tx0, it.ty0, it.b * d.off_bp + (MULTI ? it.g >> pl.ncs_shift : it.g) * 2 * d.KK, &bar_in[bb]);
-            tma::load_3d(dst + 2 * d.KK * TM * 4, &tm_mask, it.tx0, it.ty0, it.b * d.mask_bp + (MULTI ? it.g >> pl.ncs_shift : it.g) * d.KK, &bar_in[bb]);
+            tma::load_3d(dst + 2 * d.KK * TM * (int)sizeof(T), &tm_mask, it.tx0, it.ty0, it.b * d.mask_bp + (MULTI ? it.g >> pl.ncs_shift : it.g) * d.KK, &bar_in[bb]);
         }
     };
     auto issue_w = [&](int n) {                     // W^T image of iteration n's group
@@ -429,9 +436,9 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
     // All loads of a thread are issued before the wait for the previous tile's last GEMM3 (which still reads Q and col).
     constexpr int QI = (CO * (TM / 8) + NSAMP - 1) / NSAMP;
     auto tile_start = [&](const Iter &it, bool wait_g3) {
-        const float *go_b = gout + (size_t)it.b * d.Co * plane;
+        const T *go_b = gout + (size_t)it.b * d.Co * plane;
         float4 va[QI], vb[QI];
-        const bool vec = (d.Wo & 3) == 0;
+        const bool vec = d.Wo % (16 / (int)sizeof(T)) == 0;    // 8 pixels = whole 16-byte words
 #pragma unroll
         for (int q = 0; q < QI; ++q) {
             const int item = tid + q * NSAMP;
@@ -439,14 +446,22 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
             if (item < CO * (TM / 8)) {
                 const int j = item & 7, pc = (item >> 3) & (TM / 8 - 1), co = (item >> 7) * 8 + j;
                 const int hh = it.ty0 + (pc * 8) / TW, ww = it.tx0 + (pc * 8) % TW;
-                const float *src = go_b + (size_t)co * plane + (size_t)hh * d.Wo + ww;
+                const T *src = go_b + (size_t)co * plane + (size_t)hh * d.Wo + ww;
                 if (vec && hh < d.Ho && ww + 7 < d.Wo) {
-                    va[q] = __ldg(reinterpret_cast<const float4 *>(src));
-                    vb[q] = __ldg(reinterpret_cast<const float4 *>(src) + 1);
+                    if constexpr (sizeof(T) == 4) {
+                        va[q] = __ldg(reinterpret_cast<const float4 *>(src));
+                        vb[q] = __ldg(reinterpret_cast<const float4 *>(src) + 1);
+                    } else {
+                        const uint4 u = __ldg(reinterpret_cast<const uint4 *>(src));     // bf16 -> fp32: the bits move up
+                        va[q] = make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xFFFF0000u),
+                                            __uint_as_float(u.y << 16), __uint_as_float(u.y & 0xFFFF0000u));
+                        vb[q] = make_float4(__uint_as_float(u.z << 16), __uint_as_float(u.z & 0xFFFF0000u),
+                                            __uint_as_float(u.w << 16), __uint_as_float(u.w & 0xFFFF0000u));
+                    }
                 } else if (hh < d.Ho) {
                     float v[8];
 #pragma unroll
-                    for (int i = 0; i < 8; ++i) v[i] = (ww + i < d.Wo) ? __ldg(src + i) : 0.f;
+                    for (int i = 0; i < 8; ++i) v[i] = (ww + i < d.Wo) ? ld_act(src + i) : 0.f;
                     va[q] = make_float4(v[0], v[1], v[2], v[3]); vb[q] = make_float4(v[4], v[5], v[6], v[7]);
                 }
             }
@@ -477,7 +492,7 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
     };
     // ================= pass 1 of an iteration: M = max |colgrad * mask| (unsigned order of the float bits: NaN > Inf > finite,
     // so a non-finite value anywhere is seen) and the per-cell sums of the scatter's bilinear weights (rounded up, 16.16) ======
-    struct P1 { const float *om, *off_g, *mask_g; uint32_t d1, cnt_s; int by0, bxq0; };
+    struct P1 { const T *om, *off_g, *mask_g; uint32_t d1, cnt_s; int by0, bxq0; };
     auto pass1_begin = [&](const Iter &it) {
         const int bb = it.n & 1;
         const uint32_t par = (uint32_t)((it.n >> 1) & 1);
@@ -485,7 +500,7 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
         umma::fence_after_sync();
         umma::mbar_wait(&bar_in[bb], par);           // box + offsets / masks have landed
         P1 q;
-        q.om = oms + bb * (pl.om_bytes / 4);
+        q.om = oms + bb * (pl.om_bytes / (int)sizeof(T));
         q.off_g = offset + (size_t)it.b * d.off_bs + (size_t)(MULTI ? it.g >> pl.ncs_shift : it.g) * 2 * d.KK * plane;
         q.mask_g = mask + (size_t)it.b * d.mask_bs + (size_t)(MULTI ? it.g >> pl.ncs_shift : it.g) * d.KK * plane;
         q.d1 = tmem + (uint32_t)(bb * pl.N1);
@@ -500,9 +515,9 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
         if (it.valid) {
             float dy, dx, m;
             if (use_tma) {
-                dy = q.om[(2 * t) * TM + p];
-                dx = q.om[(2 * t + 1) * TM + p];
-                m = q.om[(2 * d.KK + t) * TM + p];
+                dy = act_f(q.om[(2 * t) * TM + p]);
+                dx = act_f(q.om[(2 * t + 1) * TM + p]);
+                m = act_f(q.om[(2 * d.KK + t) * TM + p]);
             } else {
                 tap_read(q.off_g, q.mask_g, uplane, (unsigned)t, (unsigned)it.pix, dy, dx, m);
             }
@@ -610,11 +625,11 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
             sc.ib = in_blk + ((size_t)cur.b * pl.units + cur.g) * in_plane * CS;
             sc.gb = gin_blk + ((size_t)cur.b * pl.units + cur.g) * in_plane * CS;
             sc.scale = ldexpf(1.f, k2);
-            const float *om = oms + bb * (pl.om_bytes / 4);
-            const float *off_g = offset + (size_t)cur.b * d.off_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * 2 * d.KK * plane;
-            const float *mask_g = mask + (size_t)cur.b * d.mask_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * d.KK * plane;
-            float *goff_g = goff + (size_t)cur.b * d.off_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * 2 * d.KK * plane;
-            float *gmask_g = gmask + (size_t)cur.b * d.mask_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * d.KK * plane;
+            const T *om = oms + bb * (pl.om_bytes / (int)sizeof(T));
+            const T *off_g = offset + (size_t)cur.b * d.off_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * 2 * d.KK * plane;
+            const T *mask_g = mask + (size_t)cur.b * d.mask_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * d.KK * plane;
+            T *goff_g = goff + (size_t)cur.b * d.off_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * 2 * d.KK * plane;
+            T *gmask_g = gmask + (size_t)cur.b * d.mask_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * d.KK * plane;
             const uint32_t d1 = tmem + (uint32_t)(bb * pl.N1);
             // pass 1 of the next group of the same tile is interleaved tap by tap (its colgrad was issued two iterations
             // ago): two independent instruction streams per warp; a new tile needs its Q first
@@ -635,9 +650,9 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
                 if (cur.valid) {
                     float dy, dx, m;
                     if (use_tma) {
-                        dy = om[(2 * t) * TM + p];
-                        dx = om[(2 * t + 1) * TM + p];
-                        m = om[(2 * d.KK + t) * TM + p];
+                        dy = act_f(om[(2 * t) * TM + p]);
+                        dx = act_f(om[(2 * t + 1) * TM + p]);
+                        m = act_f(om[(2 * d.KK + t) * TM + p]);
                     } else {
                         tap_read(off_g, mask_g, uplane, (unsigned)t, (unsigned)cur.pix, dy, dx, m);
                     }
@@ -645,12 +660,24 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
                     sample_bwd<PACKED>(d, sc, gc, dy, dx, m, ti, tj, lane, wrot, colv, g_y, g_x, g_m);
                     // more than 8 channels per deformable group: the group's units follow each other in this CTA and the
                     // same thread owns the element in each of them -> plain read-modify-write, fixed order
-                    float *gy = goff_g + (2u * (unsigned)t * uplane + (unsigned)cur.pix);
-                    if (MULTI && (cur.g & (pl.ncs - 1))) {
-                        g_y += gy[0]; g_x += gy[uplane]; g_m += gmask_g[(unsigned)t * uplane + (unsigned)cur.pix];
+                    T *gy = goff_g + (2u * (unsigned)t * uplane + (unsigned)cur.pix);
+                    if constexpr (RUN_SUMS) {
+                        // bf16 outputs: the running sums stay fp32 (same additions as below), one rounding at the last unit
+                        float *gs = gsum + 3 * t * TM + p;
+                        if (cur.g & (pl.ncs - 1)) { g_y += gs[0]; g_x += gs[TM]; g_m += gs[2 * TM]; }
+                        if ((cur.g & (pl.ncs - 1)) != pl.ncs - 1) {
+                            gs[0] = g_y; gs[TM] = g_x; gs[2 * TM] = g_m;
+                        } else {
+                            gy[0] = st_act<T>(g_y); gy[uplane] = st_act<T>(g_x);
+                            gmask_g[(unsigned)t * uplane + (unsigned)cur.pix] = st_act<T>(g_m);
+                        }
+                    } else {
+                        if (MULTI && (cur.g & (pl.ncs - 1))) {
+                            g_y += act_f(gy[0]); g_x += act_f(gy[uplane]); g_m += act_f(gmask_g[(unsigned)t * uplane + (unsigned)cur.pix]);
+                        }
+                        gy[0] = st_act<T>(g_y); gy[uplane] = st_act<T>(g_x);
+                        gmask_g[(unsigned)t * uplane + (unsigned)cur.pix] = st_act<T>(g_m);
                     }
-                    gy[0] = g_y; gy[uplane] = g_x;
-                    gmask_g[(unsigned)t * uplane + (unsigned)cur.pix] = g_m;
                 }
                 // column operand: the 8 channels of (tap t, pixel p) are one 16-byte chunk. col is read by GEMM3 of the
                 // previous iteration until bar_g3 completes: waited for here, behind the first sample's gather and scatter
@@ -788,7 +815,8 @@ __global__ void dcn_bwd_prep_weights(const float *__restrict__ weight, unsigned 
 
 // grad_input[b][g*8 + c][y][x] = sum, in a fixed order, over the boxes that cover (y, x) + the far-sample buffer.
 // One thread per (b, g, y, x): 32 contiguous bytes per box, coalesced along x; NCHW plane stores.
-__global__ void dcn_gin_collect(const float *__restrict__ pbox, const float *__restrict__ gin_blk, float *__restrict__ gin,
+template <typename T>
+__global__ void dcn_gin_collect(const float *__restrict__ pbox, const float *__restrict__ gin_blk, T *__restrict__ gin,
                                 DcnDims d, BoxBwdPlan pl)
 {
     const int HW = d.H * d.W;
@@ -827,13 +855,15 @@ __global__ void dcn_gin_collect(const float *__restrict__ pbox, const float *__r
             a0.x += u0[q].x; a0.y += u0[q].y; a0.z += u0[q].z; a0.w += u0[q].w;
             a1.x += u1[q].x; a1.y += u1[q].y; a1.z += u1[q].z; a1.w += u1[q].w;
         }
-        float *dp = gin + bg * CS * HW + px;
-        dp[0] = a0.x; dp[(size_t)HW] = a0.y; dp[(size_t)2 * HW] = a0.z; dp[(size_t)3 * HW] = a0.w;
-        dp[(size_t)4 * HW] = a1.x; dp[(size_t)5 * HW] = a1.y; dp[(size_t)6 * HW] = a1.z; dp[(size_t)7 * HW] = a1.w;
+        T *dp = gin + bg * CS * HW + px;
+        dp[0] = st_act<T>(a0.x); dp[(size_t)HW] = st_act<T>(a0.y); dp[(size_t)2 * HW] = st_act<T>(a0.z); dp[(size_t)3 * HW] = st_act<T>(a0.w);
+        dp[(size_t)4 * HW] = st_act<T>(a1.x); dp[(size_t)5 * HW] = st_act<T>(a1.y); dp[(size_t)6 * HW] = st_act<T>(a1.z); dp[(size_t)7 * HW] = st_act<T>(a1.w);
     }
 }
 
-bool make_plan(const DcnDims &d, BoxBwdPlan &pl)
+// act_bytes: size of one activation element (4 or 2). It sets the offset / mask planes in shared memory and the TMA
+// row alignment; with 2 (bf16 outputs) and several units per group the owners' fp32 running sums take the bytes saved.
+bool make_plan(const DcnDims &d, BoxBwdPlan &pl, int act_bytes = 4)
 {
     if (d.cpg % CS != 0 || d.Co != CO || d.det) return false;
     pl.units = d.C / CS;
@@ -863,15 +893,16 @@ bool make_plan(const DcnDims &d, BoxBwdPlan &pl)
     pl.mx = (box::BW - 1 - fw + 1) / 2;
     pl.wt_bytes = 2 * pl.N1 * CO * 2;
     pl.col_part = (pl.N3 / 8) * TM * 16;
-    pl.om_bytes = 3 * d.KK * TM * 4;
-    pl.use_om_tma = d.Wo % 4 == 0 && getenv("EBFI_DCN_NO_TMA") == nullptr;
+    pl.om_bytes = 3 * d.KK * TM * act_bytes;
+    pl.use_om_tma = d.Wo % (16 / act_bytes) == 0 && getenv("EBFI_DCN_NO_TMA") == nullptr;
     pl.off_q = 2 * pl.wt_bytes;
     pl.off_col = pl.off_q + 2 * Q_PART;
     pl.off_box = pl.off_col + 2 * pl.col_part;
     pl.off_acc = pl.off_box + 2 * box::BYTES;
     pl.off_cnt = pl.off_acc + box::BYTES;
     pl.off_om = pl.off_cnt + 2 * CNT_PAD;
-    pl.smem = pl.off_om + 2 * pl.om_bytes;
+    pl.off_gsum = pl.off_om + 2 * pl.om_bytes;
+    pl.smem = pl.off_gsum + (act_bytes != 4 && pl.ncs > 1 ? 3 * d.KK * TM * 4 : 0);
     return pl.smem <= 226 * 1024;
 }
 
@@ -900,12 +931,13 @@ size_t backward_box_scratch_bytes(const DcnDims &d)
            (size_t)d.B * pl.ntiles * pl.units * box::BYTES;
 }
 
-int backward_box(cudaStream_t st, const DcnDims &d, const float *input, const float *weight, const float *offset,
-                 const float *mask, const float *gout, float *gin, float *goff, float *gmask, float *gw, float *gb,
+template <typename T>
+int backward_box(cudaStream_t st, const DcnDims &d, const T *input, const float *weight, const T *offset,
+                 const T *mask, const T *gout, T *gin, T *goff, T *gmask, float *gw, float *gb,
                  float *gw_part, float *gb_part, void *scratch, const ebfi_dp::View *dp, bool dp_defer)
 {
     BoxBwdPlan pl{};
-    if (!make_plan(d, pl)) return EBFI_ERR_UNSUPPORTED;
+    if (!make_plan(d, pl, (int)sizeof(T))) return EBFI_ERR_UNSUPPORTED;
     const size_t n = (size_t)d.B * d.C * d.H * d.W;
     float *in_blk = static_cast<float *>(scratch), *gin_blk = in_blk + n;
     unsigned char *wimg = reinterpret_cast<unsigned char *>(gin_blk + n);
@@ -913,7 +945,7 @@ int backward_box(cudaStream_t st, const DcnDims &d, const float *input, const fl
     const int BG = d.B * pl.units, HW = d.H * d.W;
     if (d.in_blocked) {
         // the caller kept the forward's blocked copy (EBFI_DCN_INPUT_BLOCKED): only the far-sample accumulator is cleared
-        in_blk = const_cast<float *>(input);
+        in_blk = const_cast<float *>(reinterpret_cast<const float *>(input));
         EBFI_CUDA_OK(cudaMemsetAsync(gin_blk, 0, n * sizeof(float), st));
     } else if (int rc = launch_nchw_to_blocked(st, input, in_blk, BG, HW, gin_blk, 2)) {
         return rc;       // blocked copy of the input + zero fill of the far-sample accumulator in one pass
@@ -930,26 +962,27 @@ int backward_box(cudaStream_t st, const DcnDims &d, const float *input, const fl
     }
     if (pl.use_om_tma && !(ebfi::aligned16(offset) && ebfi::aligned16(mask))) pl.use_om_tma = 0;
     if (pl.use_om_tma) {
-        const uint64_t str[2] = {(uint64_t)d.Wo * 4, (uint64_t)d.Ho * d.Wo * 4};
+        constexpr CUtensorMapDataType om_type = sizeof(T) == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        const uint64_t str[2] = {(uint64_t)d.Wo * sizeof(T), (uint64_t)d.Ho * d.Wo * sizeof(T)};
         const uint64_t dims_o[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.off_bp + 2 * d.dg * d.KK};
         const uint64_t dims_m[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.mask_bp + d.dg * d.KK};
         const uint32_t box_o[3] = {TW, TH, (uint32_t)(2 * d.KK)}, box_m[3] = {TW, TH, (uint32_t)d.KK};
-        if (int rc = tma::encode_3d(tm_off, offset, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dims_o, str, box_o)) return rc;
-        if (int rc = tma::encode_3d(tm_mask, mask, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dims_m, str, box_m)) return rc;
+        if (int rc = tma::encode_3d(tm_off, offset, om_type, dims_o, str, box_o)) return rc;
+        if (int rc = tma::encode_3d(tm_mask, mask, om_type, dims_m, str, box_m)) return rc;
     }
     dim3 grid(box_splits(d, pl), pl.NH);
 #define EBFI_BWD_BOX(P, M)                                                                                             \
     do {                                                                                                               \
-        EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_box_kernel<P, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
-        dcn_bwd_box_kernel<P, M><<<grid, NTHR, pl.smem, st>>>(in_blk, wimg, offset, mask, gout, gin_blk, pbox, goff, gmask, \
-                                                              gw_part, gb_part, d, pl, tm_box, tm_off, tm_mask);       \
+        EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_box_kernel<P, M, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
+        dcn_bwd_box_kernel<P, M, T><<<grid, NTHR, pl.smem, st>>>(in_blk, wimg, offset, mask, gout, gin_blk, pbox, goff, gmask, \
+                                                                 gw_part, gb_part, d, pl, tm_box, tm_off, tm_mask);    \
     } while (0)
     if (pl.ncs > 1) { if (d.packed) EBFI_BWD_BOX(true, true); else EBFI_BWD_BOX(false, true); }
     else            { if (d.packed) EBFI_BWD_BOX(true, false); else EBFI_BWD_BOX(false, false); }
 #undef EBFI_BWD_BOX
     EBFI_LAUNCH_OK("dcn_bwd_box_kernel");
     const unsigned cgrid = (unsigned)std::min<size_t>(ceil_div((size_t)BG * HW, (size_t)256), (size_t)ebfi::sm_count() * 16);
-    dcn_gin_collect<<<cgrid, 256, 0, st>>>(pbox, gin_blk, gin, d, pl);
+    dcn_gin_collect<T><<<cgrid, 256, 0, st>>>(pbox, gin_blk, gin, d, pl);
     EBFI_LAUNCH_OK("dcn_gin_collect");
     const int Kdim = d.C * d.KK;
     const int rblocks = ceil_div(Kdim * CO + CO, 64);
@@ -961,5 +994,12 @@ int backward_box(cudaStream_t st, const DcnDims &d, const float *input, const fl
     if (dp && !dp_defer) return ebfi_dp::allreduce_sum(st, *dp, gw, (size_t)Kdim * CO, gb, (size_t)CO, 2);
     return EBFI_OK;
 }
+template int backward_box<float>(cudaStream_t, const DcnDims &, const float *, const float *, const float *, const float *,
+                                 const float *, float *, float *, float *, float *, float *, float *, float *, void *,
+                                 const ebfi_dp::View *, bool);
+template int backward_box<__nv_bfloat16>(cudaStream_t, const DcnDims &, const __nv_bfloat16 *, const float *,
+                                         const __nv_bfloat16 *, const __nv_bfloat16 *, const __nv_bfloat16 *, __nv_bfloat16 *,
+                                         __nv_bfloat16 *, __nv_bfloat16 *, float *, float *, float *, float *, void *,
+                                         const ebfi_dp::View *, bool);
 
 }  // namespace ebfi_dcn

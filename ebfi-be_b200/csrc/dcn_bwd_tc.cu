@@ -354,16 +354,17 @@ dcn_bwd_tc_kernel(const float *__restrict__ in_blk, const float *__restrict__ we
 // `zero` (nullable): a second (BG, HW, 8)-shaped buffer of `zero_f4` float4 per item that is cleared in the same pass
 // (the backward's grad_input accumulator: 2 float4 per item, 4 for the int64 copy of the deterministic mode) — saves the
 // separate memset launch.
-__global__ void nchw_to_blocked(const float *__restrict__ src, float *__restrict__ dst, int BG, int HW,
+template <typename T>
+__global__ void nchw_to_blocked(const T *__restrict__ src, float *__restrict__ dst, int BG, int HW,
                                 float4 *__restrict__ zero, int zero_f4)
 {
     const size_t n = (size_t)BG * HW;
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         const size_t bg = i / HW, px = i - bg * HW;
-        const float *sp = src + bg * CS * HW + px;
+        const T *sp = src + bg * CS * HW + px;
         float v[CS];
 #pragma unroll
-        for (int c = 0; c < CS; ++c) v[c] = __ldg(sp + (size_t)c * HW);
+        for (int c = 0; c < CS; ++c) v[c] = ld_act(sp + (size_t)c * HW);
         float4 *dp = reinterpret_cast<float4 *>(dst + i * CS);
         dp[0] = make_float4(v[0], v[1], v[2], v[3]);
         dp[1] = make_float4(v[4], v[5], v[6], v[7]);
@@ -439,13 +440,16 @@ int backward_tc_splits(const DcnDims &d)
     return std::max(1, std::min(tiles, ceil_div(2 * ebfi::sm_count(), d.dg)));
 }
 
-int launch_nchw_to_blocked(cudaStream_t st, const float *src, float *dst, int BG, int HW, void *zero, int zero_f4)
+template <typename T>
+int launch_nchw_to_blocked(cudaStream_t st, const T *src, float *dst, int BG, int HW, void *zero, int zero_f4)
 {
     const unsigned tgrid = (unsigned)std::min<size_t>(ceil_div((size_t)BG * HW, (size_t)256), (size_t)ebfi::sm_count() * 16);
-    nchw_to_blocked<<<tgrid, 256, 0, st>>>(src, dst, BG, HW, static_cast<float4 *>(zero), zero_f4);
+    nchw_to_blocked<T><<<tgrid, 256, 0, st>>>(src, dst, BG, HW, static_cast<float4 *>(zero), zero_f4);
     EBFI_LAUNCH_OK("nchw_to_blocked");
     return EBFI_OK;
 }
+template int launch_nchw_to_blocked<float>(cudaStream_t, const float *, float *, int, int, void *, int);
+template int launch_nchw_to_blocked<__nv_bfloat16>(cudaStream_t, const __nv_bfloat16 *, float *, int, int, void *, int);
 
 // Extra scratch of the tensor-core backward: group-blocked copies of input and grad_input.
 size_t backward_tc_scratch_bytes(const DcnDims &d)

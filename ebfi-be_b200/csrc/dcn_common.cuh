@@ -3,6 +3,8 @@
 #pragma once
 #include "common.cuh"
 
+#include <cuda_bf16.h>
+
 namespace ebfi_dcn {
 
 constexpr int KC_MAX = 96;    // rows of the sampled slab in the SIMT kernels (channels-in-chunk * kh*kw)
@@ -52,11 +54,24 @@ __device__ __forceinline__ void det_add(long long *p, float v, float scale)
     atomicAdd(reinterpret_cast<unsigned long long *>(p), (unsigned long long)__float2ll_rn(v * scale));
 }
 
-__device__ __forceinline__ const float *off_ptr(const DcnDims &d, const float *offset, int b, int g, size_t plane)
+// Activation element type T (float | __nv_bfloat16) of the tensor-core kernels: input, offset, mask and grad_output are
+// read as T and widened exactly, output and the activation gradients are rounded once (RN) from the fp32 values the
+// float instantiation stores. Everything in between (blocked input copy, boxes, weights, partials) is fp32.
+__device__ __forceinline__ float act_f(float v) { return v; }
+__device__ __forceinline__ float act_f(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float ld_act(const float *p) { return __ldg(p); }
+__device__ __forceinline__ float ld_act(const __nv_bfloat16 *p) { return __bfloat162float(__ldg(p)); }
+template <typename T> __device__ __forceinline__ T st_act(float v);
+template <> __device__ __forceinline__ float st_act<float>(float v) { return v; }
+template <> __device__ __forceinline__ __nv_bfloat16 st_act<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+
+template <typename T>
+__device__ __forceinline__ const T *off_ptr(const DcnDims &d, const T *offset, int b, int g, size_t plane)
 {
     return offset + (size_t)b * d.off_bs + (size_t)g * 2 * d.KK * plane;
 }
-__device__ __forceinline__ const float *mask_ptr(const DcnDims &d, const float *mask, int b, int g, size_t plane)
+template <typename T>
+__device__ __forceinline__ const T *mask_ptr(const DcnDims &d, const T *mask, int b, int g, size_t plane)
 {
     return mask + (size_t)b * d.mask_bs + (size_t)g * d.KK * plane;
 }
@@ -128,13 +143,14 @@ __device__ __forceinline__ void warp_atomic_sum(float *dst, float v)
 
 // Division-free read of one tap's (dy, dx, raw mask value) for kernels that already know the pixel index:
 // offset channel 2t = dy, 2t+1 = dx inside the group (im2col_cuda.cu:170-171); plane = Ho * Wo.
-__device__ __forceinline__ void tap_read(const float *__restrict__ off_bg, const float *__restrict__ mask_bg,
+template <typename T>
+__device__ __forceinline__ void tap_read(const T *__restrict__ off_bg, const T *__restrict__ mask_bg,
                                          unsigned plane, unsigned t, unsigned pix, float &dy, float &dx, float &m)
 {
     const unsigned o = 2u * t * plane + pix;
-    dy = __ldg(off_bg + o);
-    dx = __ldg(off_bg + o + plane);
-    m = __ldg(mask_bg + t * plane + pix);
+    dy = ld_act(off_bg + o);
+    dx = ld_act(off_bg + o + plane);
+    m = ld_act(mask_bg + t * plane + pix);
 }
 
 // 256-bit read-only global load (sm_100+: LDG.E.256): the 8 channels of one bilinear corner in the
@@ -157,7 +173,8 @@ __device__ __forceinline__ f8 ldg_f8(const float *p32B_aligned, bool ok)
 // {max_px sum_co |gO|, max |weight|, max |mask|} -> bound[3] (dcn.cu)
 int launch_det_bound(cudaStream_t st, const DcnDims &d, const float *gout, const float *weight, const float *mask, float *bound);
 
-// NCHW (BG*8 planes of HW pixels) -> group-blocked (BG, HW, 8) copy (dcn_bwd_tc.cu)
-int launch_nchw_to_blocked(cudaStream_t st, const float *src, float *dst, int BG, int HW, void *zero = nullptr, int zero_f4 = 0);
+// NCHW (BG*8 planes of HW pixels, T = float | __nv_bfloat16) -> fp32 group-blocked (BG, HW, 8) copy (dcn_bwd_tc.cu)
+template <typename T>
+int launch_nchw_to_blocked(cudaStream_t st, const T *src, float *dst, int BG, int HW, void *zero = nullptr, int zero_f4 = 0);
 
 }  // namespace ebfi_dcn

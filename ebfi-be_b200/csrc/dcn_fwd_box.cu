@@ -26,6 +26,8 @@
 //
 // fp32 parity: products are 3xTF32 (umma.cuh); the hi*hi chain is spread over several TMEM accumulators because
 // the tensor core's fp32 accumulate rounds toward zero.
+// Activation type T (float | __nv_bfloat16, the *_bf16 entries): the input is widened into the same fp32 blocked copy,
+// offsets / masks arrive by TMA as T planes and are widened where the samplers read them, the epilogue rounds once.
 #include "dcn_box.cuh"
 #include "dcn_common.cuh"
 #include "tma.cuh"
@@ -126,11 +128,11 @@ __device__ __forceinline__ bool sample8(float y, float x, float m, int H, int W,
     return false;
 }
 
-template <int TPR, bool PACKED>
+template <int TPR, bool PACKED, typename T>
 __global__ void __launch_bounds__(NTHR, 1)
 dcn_fwd_box_kernel(const float *__restrict__ in_blk, const float *__restrict__ bias,
-                   const float *__restrict__ offset, const float *__restrict__ mask,
-                   float *__restrict__ output, const float *__restrict__ wimg, DcnDims d, BoxPlan pl,
+                   const T *__restrict__ offset, const T *__restrict__ mask,
+                   T *__restrict__ output, const float *__restrict__ wimg, DcnDims d, BoxPlan pl,
                    const __grid_constant__ CUtensorMap tm_box, const __grid_constant__ CUtensorMap tm_off,
                    const __grid_constant__ CUtensorMap tm_mask)
 {
@@ -138,7 +140,7 @@ dcn_fwd_box_kernel(const float *__restrict__ in_blk, const float *__restrict__ b
     unsigned char *aring = smem;                       // [NS][a_hi | a_lo]
     unsigned char *wring = smem + pl.off_w;            // [2 units][TPR stages][b_hi | b_lo], one unit ahead of the samplers
     unsigned char *boxes = smem + pl.off_box;          // [2][BH][BW][8] fp32
-    const float *oms = reinterpret_cast<const float *>(smem + pl.off_om);   // [2][3*KK planes][128 px]
+    const T *oms = reinterpret_cast<const T *>(smem + pl.off_om);           // [2][3*KK planes][128 px]
     __shared__ __align__(8) uint64_t slot_free[NS], a_full[NS], wu_full[2], wu_free[2];
     __shared__ __align__(8) uint64_t box_full[2], box_free[2], om_full[2], om_free[2], acc_full[2], acc_free[2];
     __shared__ uint32_t tmem_slot;
@@ -191,7 +193,7 @@ dcn_fwd_box_kernel(const float *__restrict__ in_blk, const float *__restrict__ b
             tile_origin(tile, b, ty0, tx0);
             const int ho = ty0 + p / TW, wo = tx0 + p % TW;
             const bool valid = ho < d.Ho && wo < d.Wo;
-            float *out_p = output + (size_t)b * d.Co * plane + (size_t)ho * d.Wo + wo;
+            T *out_p = output + (size_t)b * d.Co * plane + (size_t)ho * d.Wo + wo;
             umma::mbar_wait(&acc_full[ab], (uint32_t)((k >> 1) & 1));
             umma::fence_after_sync();
             const uint32_t tb = tmem + (uint32_t)(ab * ACC_COLS);
@@ -207,7 +209,7 @@ dcn_fwd_box_kernel(const float *__restrict__ in_blk, const float *__restrict__ b
                 }
                 if (valid) {
 #pragma unroll
-                    for (int i = 0; i < 8; ++i) out_p[(size_t)(cb + i) * plane] = v[i] + __ldg(bias + cb + i);
+                    for (int i = 0; i < 8; ++i) out_p[(size_t)(cb + i) * plane] = st_act<T>(v[i] + __ldg(bias + cb + i));
                 }
             }
             umma::fence_before_sync();
@@ -245,12 +247,12 @@ dcn_fwd_box_kernel(const float *__restrict__ in_blk, const float *__restrict__ b
                 if (pl.use_om_tma) {
                     const int ob = G & 1;
                     umma::mbar_wait(&om_full[ob], (uint32_t)((G >> 1) & 1));
-                    const float *om = oms + ob * (pl.om_bytes / 4);
+                    const T *om = oms + ob * (pl.om_bytes / (int)sizeof(T));
 #pragma unroll
                     for (int s = 0; s < TPR; ++s) {
                         const int t = r * TPR + s;
                         float dy = 0.f, dx = 0.f, m = 0.f;
-                        if (tv[s]) { dy = om[(2 * t) * TM + p]; dx = om[(2 * t + 1) * TM + p]; m = om[(2 * d.KK + t) * TM + p]; }
+                        if (tv[s]) { dy = act_f(om[(2 * t) * TM + p]); dx = act_f(om[(2 * t + 1) * TM + p]); m = act_f(om[(2 * d.KK + t) * TM + p]); }
                         sy[s] = tv[s] ? by[s] + dy : -2.f;
                         sx[s] = tv[s] ? bx[s] + dx : -2.f;
                         sm[s] = mask_act_t<PACKED>(m);
@@ -259,8 +261,8 @@ dcn_fwd_box_kernel(const float *__restrict__ in_blk, const float *__restrict__ b
                     __syncwarp();
                     if (lane == 0) umma::mbar_arrive(&om_free[ob]);
                 } else {
-                    const float *off_bg = off_ptr(d, offset, b, g, plane);
-                    const float *mask_bg = mask_ptr(d, mask, b, g, plane);
+                    const T *off_bg = off_ptr(d, offset, b, g, plane);
+                    const T *mask_bg = mask_ptr(d, mask, b, g, plane);
 #pragma unroll
                     for (int s = 0; s < TPR; ++s) {
                         float dy = 0.f, dx = 0.f, m = 0.f;
@@ -371,7 +373,7 @@ dcn_fwd_box_kernel(const float *__restrict__ in_blk, const float *__restrict__ b
                         unsigned char *dst = smem + pl.off_om + ob * pl.om_bytes;
                         umma::mbar_expect_tx(&om_full[ob], (uint32_t)pl.om_bytes);
                         tma::load_3d(dst, &tm_off, tx0, ty0, b * d.off_bp + g * 2 * d.KK, &om_full[ob]);
-                        tma::load_3d(dst + 2 * d.KK * TM * 4, &tm_mask, tx0, ty0, b * d.mask_bp + g * d.KK, &om_full[ob]);
+                        tma::load_3d(dst + 2 * d.KK * TM * (int)sizeof(T), &tm_mask, tx0, ty0, b * d.mask_bp + g * d.KK, &om_full[ob]);
                     }
                     for (int ci = 0; ci < pl.ncs; ++ci, ++U) {
                         const int bb = U & 1;
@@ -424,7 +426,8 @@ __global__ void dcn_prep_weights(const float *__restrict__ weight, float *__rest
     }
 }
 
-bool make_plan(const DcnDims &d, BoxPlan &pl)
+// act_bytes: size of one offset / mask element (4 or 2); it sets the shared-memory planes and the TMA row alignment
+bool make_plan(const DcnDims &d, BoxPlan &pl, int act_bytes = 4)
 {
     if (d.Co % 16 != 0 || d.Co > 128 || d.cpg % 8 != 0) return false;   // blocked layout: 8-channel chunks
     if ((long)2 * d.KK * d.Ho * d.Wo >= (1L << 31)) return false;        // 32-bit offsets inside one group
@@ -446,8 +449,8 @@ bool make_plan(const DcnDims &d, BoxPlan &pl)
     const int fh = (TH - 1) * d.sh + (d.kh - 1) * d.dh + 1, fw = (TW - 1) * d.sw + (d.kw - 1) * d.dw + 1;
     pl.my = std::max(0, (BH - 1 - fh + 1) / 2);
     pl.mx = std::max(0, (BW - 1 - fw + 1) / 2);
-    pl.om_bytes = 3 * d.KK * TM * 4;
-    pl.use_om_tma = d.Wo % 4 == 0 && getenv("EBFI_DCN_NO_TMA") == nullptr;
+    pl.om_bytes = 3 * d.KK * TM * act_bytes;
+    pl.use_om_tma = d.Wo % (16 / act_bytes) == 0 && getenv("EBFI_DCN_NO_TMA") == nullptr;
     pl.unit_bytes = pl.TPR * 2 * pl.b_bytes;
     pl.off_w = NS * 2 * pl.a_bytes;
     pl.off_box = pl.off_w + 2 * pl.unit_bytes;
@@ -474,11 +477,12 @@ size_t forward_tc_workspace(const DcnDims &d)
            (size_t)d.B * d.C * d.H * d.W * sizeof(float);
 }
 
-int forward_tc(cudaStream_t st, const DcnDims &d, const float *input, const float *weight, const float *bias,
-               const float *offset, const float *mask, float *output, void *workspace, size_t workspace_bytes)
+template <typename T>
+int forward_tc(cudaStream_t st, const DcnDims &d, const T *input, const float *weight, const float *bias,
+               const T *offset, const T *mask, T *output, void *workspace, size_t workspace_bytes)
 {
     BoxPlan pl{};
-    if (!make_plan(d, pl)) return EBFI_ERR_UNSUPPORTED;
+    if (!make_plan(d, pl, (int)sizeof(T))) return EBFI_ERR_UNSUPPORTED;
     const size_t wbytes = (size_t)d.dg * pl.ncs * pl.TPR * 2 * pl.b_bytes;
     const size_t need = ebfi::round_up(wbytes, (size_t)256) + (size_t)d.B * d.C * d.H * d.W * sizeof(float);
     // the blocked input copy inside the workspace is read by TMA (16-byte) and by 256-bit loads (32-byte alignment)
@@ -498,22 +502,23 @@ int forward_tc(cudaStream_t st, const DcnDims &d, const float *input, const floa
     }
     if (pl.use_om_tma && !(ebfi::aligned16(offset) && ebfi::aligned16(mask))) pl.use_om_tma = 0;
     if (pl.use_om_tma) {
-        const uint64_t str[2] = {(uint64_t)d.Wo * 4, (uint64_t)d.Ho * d.Wo * 4};
+        constexpr CUtensorMapDataType om_type = sizeof(T) == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        const uint64_t str[2] = {(uint64_t)d.Wo * sizeof(T), (uint64_t)d.Ho * d.Wo * sizeof(T)};
         const uint64_t dims_o[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.off_bp + 2 * d.dg * d.KK};
         const uint64_t dims_m[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.mask_bp + d.dg * d.KK};
         const uint32_t box_o[3] = {TW, TH, (uint32_t)(2 * d.KK)}, box_m[3] = {TW, TH, (uint32_t)d.KK};
-        if (int rc = tma::encode_3d(tm_off, offset, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dims_o, str, box_o)) return rc;
-        if (int rc = tma::encode_3d(tm_mask, mask, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dims_m, str, box_m)) return rc;
+        if (int rc = tma::encode_3d(tm_off, offset, om_type, dims_o, str, box_o)) return rc;
+        if (int rc = tma::encode_3d(tm_mask, mask, om_type, dims_m, str, box_m)) return rc;
     }
     const unsigned grid = (unsigned)std::min(ebfi::sm_count(), d.B * pl.ntiles);
-#define EBFI_FWD_BOX(T)                                                                                       \
+#define EBFI_FWD_BOX(R)                                                                                       \
     do {                                                                                                      \
         if (d.packed) {                                                                                       \
-            EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_fwd_box_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
-            dcn_fwd_box_kernel<T, true><<<grid, NTHR, pl.smem, st>>>(in_blk, bias, offset, mask, output, wimg, d, pl, tm_box, tm_off, tm_mask); \
+            EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_fwd_box_kernel<R, true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
+            dcn_fwd_box_kernel<R, true, T><<<grid, NTHR, pl.smem, st>>>(in_blk, bias, offset, mask, output, wimg, d, pl, tm_box, tm_off, tm_mask); \
         } else {                                                                                              \
-            EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_fwd_box_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
-            dcn_fwd_box_kernel<T, false><<<grid, NTHR, pl.smem, st>>>(in_blk, bias, offset, mask, output, wimg, d, pl, tm_box, tm_off, tm_mask); \
+            EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_fwd_box_kernel<R, false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
+            dcn_fwd_box_kernel<R, false, T><<<grid, NTHR, pl.smem, st>>>(in_blk, bias, offset, mask, output, wimg, d, pl, tm_box, tm_off, tm_mask); \
         }                                                                                                     \
     } while (0)
     switch (pl.TPR) {
@@ -526,5 +531,9 @@ int forward_tc(cudaStream_t st, const DcnDims &d, const float *input, const floa
     EBFI_LAUNCH_OK("dcn_fwd_box_kernel");
     return EBFI_OK;
 }
+template int forward_tc<float>(cudaStream_t, const DcnDims &, const float *, const float *, const float *, const float *,
+                               const float *, float *, void *, size_t);
+template int forward_tc<__nv_bfloat16>(cudaStream_t, const DcnDims &, const __nv_bfloat16 *, const float *, const float *,
+                                       const __nv_bfloat16 *, const __nv_bfloat16 *, __nv_bfloat16 *, void *, size_t);
 
 }  // namespace ebfi_dcn

@@ -22,8 +22,15 @@ from .shims import _ext as _backend
 logger = logging.getLogger("base")
 
 
+def _as_dtypes(grads, tensors):
+    """Gradients in the dtype of the tensor each one belongs to (bf16 calls return bf16 activation gradients; under
+    autocast an input can be fp32)."""
+    return tuple(gr.to(t.dtype) for gr, t in zip(grads, tensors))
+
+
 class _DCNv2(Function):
-    """Modulated deformable convolution; arguments as dcn_v2.py:18-21."""
+    """Modulated deformable convolution; arguments as dcn_v2.py:18-21. bf16 and mixed bf16 / fp32 tensors (autocast)
+    follow shims/_ext.py: the output is bf16, each gradient has its input's dtype."""
 
     @staticmethod
     def forward(ctx, input, offset, mask, weight, bias, stride, padding, dilation, deformable_groups):
@@ -42,7 +49,8 @@ class _DCNv2(Function):
         g_in, g_off, g_mask, g_w, g_b = _backend.dcn_v2_backward(
             input, weight, bias, offset, mask, grad_output, *ctx.kernel_size, *ctx.stride,
             *ctx.padding, *ctx.dilation, ctx.deformable_groups)
-        return g_in, g_off, g_mask, g_w, g_b, None, None, None, None
+        return (*_as_dtypes((g_in, g_off, g_mask, g_w, g_b), (input, offset, mask, weight, bias)),
+                None, None, None, None)
 
 
 dcn_v2_conv = _DCNv2.apply
@@ -71,7 +79,8 @@ class _DCNv2Packed(Function):
         g_in, g_om, g_w, g_b = _backend.dcn_v2_backward_packed(
             input, weight, bias, offset_mask, grad_output, *ctx.kernel_size, *ctx.stride,
             *ctx.padding, *ctx.dilation, ctx.deformable_groups)
-        return g_in, g_om, g_w, g_b, None, None, None, None, None
+        return (*_as_dtypes((g_in, g_om, g_w, g_b), (input, offset_mask, weight, bias)),
+                None, None, None, None, None)
 
 
 def dcn_v2_conv_packed(input, offset_mask, weight, bias, stride, padding, dilation, deformable_groups, stat=None):

@@ -145,6 +145,40 @@ int ebfi_dcnv2_backward_packed(void *stream, const ebfi_dcn_geom *g,
                                float *grad_weight, float *grad_bias,
                                void *workspace, size_t workspace_bytes);
 
+/* bf16 activation variants of the five DCNv2 entries above (mixed precision: bf16 activations, fp32 parameters), same
+ * argument order and the same workspace queries. input, offset, mask / offset_mask, grad_output, output, grad_input,
+ * grad_offset, grad_mask and grad_offset_mask are `__nv_bfloat16*` NCHW; weight, bias, grad_weight, grad_bias and
+ * abs_offset_sum stay fp32. With EBFI_DCN_INPUT_BLOCKED, `input` is the fp32 group-blocked copy, as for the fp32 entry.
+ * Only the activation loads and stores change: loads widen exactly, results are rounded once (RN) from the fp32 values
+ * the fp32 entries store, so on bf16-valued inputs every activation result equals the fp32 entry's result rounded to
+ * bf16, and grad_weight / grad_bias are equal.
+ * They run only where the tensor-core kernels run: the forward for Cout a multiple of 16 up to 128, channels per group
+ * a multiple of 8 and up to 12 taps, with a workspace of ebfi_dcnv2_forward_workspace_bytes; the backward for
+ * Cout == 64, 8 / 16 / 32 channels per group, no EBFI_DCN_DETERMINISTIC and a 16-byte aligned grad_output; neither
+ * under EBFI_DCN_IMPL=simt. Anything else returns EBFI_ERR_UNSUPPORTED before any work is enqueued: take the fp32 entry
+ * on widened copies. ebfi_dcnv2_backward_dp_bf16 is declared with the data-parallel entries below. */
+int ebfi_dcnv2_forward_bf16(void *stream, const ebfi_dcn_geom *g,
+                            const void *input, const float *weight, const float *bias,
+                            const void *offset, const void *mask,
+                            void *output, void *workspace, size_t workspace_bytes);
+int ebfi_dcnv2_backward_bf16(void *stream, const ebfi_dcn_geom *g,
+                             const void *input, const float *weight, const float *bias,
+                             const void *offset, const void *mask,
+                             const void *grad_output,
+                             void *grad_input, void *grad_offset, void *grad_mask,
+                             float *grad_weight, float *grad_bias,
+                             void *workspace, size_t workspace_bytes);
+int ebfi_dcnv2_forward_packed_bf16(void *stream, const ebfi_dcn_geom *g,
+                                   const void *input, const float *weight, const float *bias,
+                                   const void *offset_mask, void *output, float *abs_offset_sum,
+                                   void *workspace, size_t workspace_bytes);
+int ebfi_dcnv2_backward_packed_bf16(void *stream, const ebfi_dcn_geom *g,
+                                    const void *input, const float *weight, const float *bias,
+                                    const void *offset_mask, const void *grad_output,
+                                    void *grad_input, void *grad_offset_mask,
+                                    float *grad_weight, float *grad_bias,
+                                    void *workspace, size_t workspace_bytes);
+
 /* ---- FAC KernelConv2D ------------------------------------------------------- */
 
 /* input  : (B, C, H+K-1, W+K-1)   already padded by the caller (KernelConv2D.py:82-86)
@@ -359,6 +393,14 @@ int ebfi_dcnv2_backward_dp(void *stream, const ebfi_dcn_geom *g,
                            float *grad_input, float *grad_offset, float *grad_mask,
                            float *grad_weight, float *grad_bias,
                            void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm, int defer);
+/* The same with bf16 activations, as ebfi_dcnv2_backward_bf16 (EBFI_ERR_UNSUPPORTED: take ebfi_dcnv2_backward_dp on
+ * widened copies). grad_weight / grad_bias are fp32, exchanged exactly as above. */
+int ebfi_dcnv2_backward_dp_bf16(void *stream, const ebfi_dcn_geom *g,
+                                const void *input, const float *weight, const float *bias,
+                                const void *offset, const void *mask, const void *grad_output,
+                                void *grad_input, void *grad_offset, void *grad_mask,
+                                float *grad_weight, float *grad_bias,
+                                void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm, int defer);
 
 #ifdef __cplusplus
 }
