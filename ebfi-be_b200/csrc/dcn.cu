@@ -29,7 +29,7 @@
 
 namespace ebfi_dcn {
 // tensor-core forward (dcn_fwd_box.cu); returns EBFI_ERR_UNSUPPORTED when the shape is not eligible.
-// T = float | __nv_bfloat16: the type of input, offset, mask and output.
+// T = float | __nv_bfloat16 | __half: the type of input, offset, mask and output.
 template <typename T>
 int forward_tc(cudaStream_t st, const DcnDims &d, const T *input, const float *weight, const float *bias,
                const T *offset, const T *mask, T *output, void *workspace, size_t workspace_bytes);
@@ -493,8 +493,11 @@ size_t ebfi_dcnv2_forward_workspace_bytes(const ebfi_dcn_geom *q)
 
 }  // extern "C"
 
-// T = float: every shape. T = __nv_bfloat16 (the *_bf16 entries): only where the tensor-core kernels run; anything else
-// returns EBFI_ERR_UNSUPPORTED before the first launch, and the caller runs the float entry on widened copies.
+// T = float: every shape. T = __nv_bfloat16 | __half (the *_bf16 / *_fp16 entries): only where the tensor-core kernels
+// run; anything else returns EBFI_ERR_UNSUPPORTED before the first launch, and the caller runs the float entry on
+// widened copies.
+template <typename T> static constexpr const char *act_name() { return std::is_same_v<T, __half> ? "fp16" : "bf16"; }
+
 template <typename T>
 static int run_forward(void *stream, const DcnDims &d, const T *input, const float *weight,
                        const float *bias, const T *offset, const T *mask, T *output,
@@ -509,7 +512,7 @@ static int run_forward(void *stream, const DcnDims &d, const T *input, const flo
     if constexpr (!std::is_same_v<T, float>) {
         const size_t need = forward_tc_workspace(d);
         if (simt || need == 0 || !workspace || workspace_bytes < need || (reinterpret_cast<uintptr_t>(workspace) & 31u))
-            return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_forward_bf16: no tensor-core forward for this call");
+            return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_forward_%s: no tensor-core forward for this call", act_name<T>());
     }
     if (d.abs_sum) EBFI_CUDA_OK(cudaMemsetAsync(d.abs_sum, 0, sizeof(float), st));
     if (!simt) {
@@ -523,7 +526,7 @@ static int run_forward(void *stream, const DcnDims &d, const T *input, const flo
         EBFI_LAUNCH_OK("dcn_fwd_kernel");
         return EBFI_OK;
     } else {
-        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_forward_bf16: no tensor-core forward for this call");
+        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_forward_%s: no tensor-core forward for this call", act_name<T>());
     }
 }
 
@@ -543,13 +546,14 @@ static int run_backward(void *stream, const DcnDims &d_in, const T *input, const
     cudaStream_t st = ebfi::as_stream(stream);
     DcnDims d = d_in;
     const char *impl = getenv("EBFI_DCN_IMPL");
-    // the tensor-core backward stages grad_output with 128-bit loads (8 pixels: two for fp32, one for bf16, when a row is a
-    // whole number of 16-byte words): it needs a 16-byte aligned base for either element size
+    // the tensor-core backward stages grad_output with 128-bit loads (8 pixels: two for fp32, one for bf16 / fp16, when a
+    // row is a whole number of 16-byte words): it needs a 16-byte aligned base for either element size
     const bool tc_ok = !(impl && impl[0] == 's') && ebfi::aligned16(grad_output);
     // box kernel (dcn_bwd_box.cu) first; the group-specialised kernel (dcn_bwd_tc.cu) serves the deterministic flag
     const int S_box = tc_ok ? backward_box_splits(d) : 0;
     if (!std::is_same_v<T, float> && S_box == 0)
-        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_backward_bf16: no box backward for this call (shape, flags or alignment)");
+        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_backward_%s: no box backward for this call (shape, flags or alignment)",
+                          act_name<T>());
     const int S_tc = S_box > 0 ? S_box : (tc_ok ? backward_tc_splits(d) : 0);
     const int S = S_tc > 0 ? S_tc : bwd_splits(d);
     if (d.in_blocked) {
@@ -578,7 +582,7 @@ static int run_backward(void *stream, const DcnDims &d_in, const T *input, const
                                grad_weight, grad_bias, gw_part, gb_part, scratch, dp, dp_defer);
     }
     if constexpr (!std::is_same_v<T, float>) {
-        return EBFI_ERR_UNSUPPORTED;      // not reached: a bf16 call without the box path returned above
+        return EBFI_ERR_UNSUPPORTED;      // not reached: a 16-bit call without the box path returned above
     } else {
         if (d.det) {
             float *bound = reinterpret_cast<float *>(scratch + scratch_bytes);
@@ -691,18 +695,73 @@ int ebfi_dcnv2_backward_packed(void *stream, const ebfi_dcn_geom *q, const float
                         grad_offset_mask, grad_offset_mask + m0, grad_weight, grad_bias, workspace, workspace_bytes);
 }
 
-// ---- bf16 activations (ebfi_b200.h): same geometry handling as the float entries above ----
-using bf16 = __nv_bfloat16;
-static const bf16 *cb(const void *p) { return static_cast<const bf16 *>(p); }
-static bf16 *mb(void *p) { return static_cast<bf16 *>(p); }
+}  // extern "C"
+
+// ---- 16-bit activations (ebfi_b200.h, T = __nv_bfloat16 | __half): same geometry handling as the float entries above ----
+template <typename T>
+static int forward16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight, const float *bias,
+                     const void *offset, const void *mask, void *output, void *workspace, size_t workspace_bytes)
+{
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    return run_forward(stream, d, static_cast<const T *>(input), weight, bias, static_cast<const T *>(offset),
+                       static_cast<const T *>(mask), static_cast<T *>(output), workspace, workspace_bytes);
+}
+
+template <typename T>
+static int backward16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                      const void *offset, const void *mask, const void *grad_output, void *grad_input,
+                      void *grad_offset, void *grad_mask, float *grad_weight, float *grad_bias,
+                      void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm = nullptr, int defer = 0)
+{
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    return run_backward(stream, d, static_cast<const T *>(input), weight, static_cast<const T *>(offset),
+                        static_cast<const T *>(mask), static_cast<const T *>(grad_output), static_cast<T *>(grad_input),
+                        static_cast<T *>(grad_offset), static_cast<T *>(grad_mask), grad_weight, grad_bias,
+                        workspace, workspace_bytes, comm, defer != 0);
+}
+
+template <typename T>
+static int forward_packed16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                            const float *bias, const void *offset_mask, void *output, float *abs_offset_sum,
+                            void *workspace, size_t workspace_bytes)
+{
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    EBFI_REQUIRE(offset_mask != nullptr, "dcn_forward_packed: null pointer");
+    const T *om = static_cast<const T *>(offset_mask);
+    const T *mask_logits = om + 2 * d.mask_bs;
+    set_packed(d);
+    d.abs_sum = abs_offset_sum;
+    return run_forward(stream, d, static_cast<const T *>(input), weight, bias, om, mask_logits, static_cast<T *>(output),
+                       workspace, workspace_bytes);
+}
+
+template <typename T>
+static int backward_packed16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                             const void *offset_mask, const void *grad_output, void *grad_input,
+                             void *grad_offset_mask, float *grad_weight, float *grad_bias,
+                             void *workspace, size_t workspace_bytes)
+{
+    DcnDims d{};
+    if (int rc = fill_dims(q, d)) return rc;
+    EBFI_REQUIRE(offset_mask && grad_offset_mask, "dcn_backward_packed: null pointer");
+    const long long m0 = 2 * d.mask_bs;
+    set_packed(d);
+    const T *om = static_cast<const T *>(offset_mask);
+    T *gom = static_cast<T *>(grad_offset_mask);
+    return run_backward(stream, d, static_cast<const T *>(input), weight, om, om + m0, static_cast<const T *>(grad_output),
+                        static_cast<T *>(grad_input), gom, gom + m0, grad_weight, grad_bias, workspace, workspace_bytes);
+}
+
+extern "C" {
 
 int ebfi_dcnv2_forward_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
                             const float *bias, const void *offset, const void *mask, void *output,
                             void *workspace, size_t workspace_bytes)
 {
-    DcnDims d{};
-    if (int rc = fill_dims(q, d)) return rc;
-    return run_forward(stream, d, cb(input), weight, bias, cb(offset), cb(mask), mb(output), workspace, workspace_bytes);
+    return forward16<__nv_bfloat16>(stream, q, input, weight, bias, offset, mask, output, workspace, workspace_bytes);
 }
 
 int ebfi_dcnv2_backward_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
@@ -712,10 +771,8 @@ int ebfi_dcnv2_backward_bf16(void *stream, const ebfi_dcn_geom *q, const void *i
                              void *workspace, size_t workspace_bytes)
 {
     (void)bias;
-    DcnDims d{};
-    if (int rc = fill_dims(q, d)) return rc;
-    return run_backward(stream, d, cb(input), weight, cb(offset), cb(mask), cb(grad_output), mb(grad_input),
-                        mb(grad_offset), mb(grad_mask), grad_weight, grad_bias, workspace, workspace_bytes);
+    return backward16<__nv_bfloat16>(stream, q, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
+                           grad_weight, grad_bias, workspace, workspace_bytes);
 }
 
 int ebfi_dcnv2_backward_dp_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
@@ -725,24 +782,17 @@ int ebfi_dcnv2_backward_dp_bf16(void *stream, const ebfi_dcn_geom *q, const void
                                 void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm, int defer)
 {
     (void)bias;
-    DcnDims d{};
-    if (int rc = fill_dims(q, d)) return rc;
     EBFI_REQUIRE(comm != nullptr, "dcn_backward_dp: null communicator");
-    return run_backward(stream, d, cb(input), weight, cb(offset), cb(mask), cb(grad_output), mb(grad_input),
-                        mb(grad_offset), mb(grad_mask), grad_weight, grad_bias, workspace, workspace_bytes, comm, defer != 0);
+    return backward16<__nv_bfloat16>(stream, q, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
+                           grad_weight, grad_bias, workspace, workspace_bytes, comm, defer);
 }
 
 int ebfi_dcnv2_forward_packed_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
                                    const float *bias, const void *offset_mask, void *output,
                                    float *abs_offset_sum, void *workspace, size_t workspace_bytes)
 {
-    DcnDims d{};
-    if (int rc = fill_dims(q, d)) return rc;
-    EBFI_REQUIRE(offset_mask != nullptr, "dcn_forward_packed: null pointer");
-    const bf16 *mask_logits = cb(offset_mask) + 2 * d.mask_bs;
-    set_packed(d);
-    d.abs_sum = abs_offset_sum;
-    return run_forward(stream, d, cb(input), weight, bias, cb(offset_mask), mask_logits, mb(output), workspace, workspace_bytes);
+    return forward_packed16<__nv_bfloat16>(stream, q, input, weight, bias, offset_mask, output, abs_offset_sum, workspace,
+                                 workspace_bytes);
 }
 
 int ebfi_dcnv2_backward_packed_bf16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
@@ -751,14 +801,56 @@ int ebfi_dcnv2_backward_packed_bf16(void *stream, const ebfi_dcn_geom *q, const 
                                     void *workspace, size_t workspace_bytes)
 {
     (void)bias;
-    DcnDims d{};
-    if (int rc = fill_dims(q, d)) return rc;
-    EBFI_REQUIRE(offset_mask && grad_offset_mask, "dcn_backward_packed: null pointer");
-    const long long m0 = 2 * d.mask_bs;
-    set_packed(d);
-    return run_backward(stream, d, cb(input), weight, cb(offset_mask), cb(offset_mask) + m0, cb(grad_output),
-                        mb(grad_input), mb(grad_offset_mask), mb(grad_offset_mask) + m0, grad_weight, grad_bias,
-                        workspace, workspace_bytes);
+    return backward_packed16<__nv_bfloat16>(stream, q, input, weight, offset_mask, grad_output, grad_input, grad_offset_mask,
+                                  grad_weight, grad_bias, workspace, workspace_bytes);
+}
+
+int ebfi_dcnv2_forward_fp16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                            const float *bias, const void *offset, const void *mask, void *output,
+                            void *workspace, size_t workspace_bytes)
+{
+    return forward16<__half>(stream, q, input, weight, bias, offset, mask, output, workspace, workspace_bytes);
+}
+
+int ebfi_dcnv2_backward_fp16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                             const float *bias, const void *offset, const void *mask,
+                             const void *grad_output, void *grad_input, void *grad_offset,
+                             void *grad_mask, float *grad_weight, float *grad_bias,
+                             void *workspace, size_t workspace_bytes)
+{
+    (void)bias;
+    return backward16<__half>(stream, q, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
+                           grad_weight, grad_bias, workspace, workspace_bytes);
+}
+
+int ebfi_dcnv2_backward_dp_fp16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                                const float *bias, const void *offset, const void *mask,
+                                const void *grad_output, void *grad_input, void *grad_offset,
+                                void *grad_mask, float *grad_weight, float *grad_bias,
+                                void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm, int defer)
+{
+    (void)bias;
+    EBFI_REQUIRE(comm != nullptr, "dcn_backward_dp: null communicator");
+    return backward16<__half>(stream, q, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
+                           grad_weight, grad_bias, workspace, workspace_bytes, comm, defer);
+}
+
+int ebfi_dcnv2_forward_packed_fp16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                                   const float *bias, const void *offset_mask, void *output,
+                                   float *abs_offset_sum, void *workspace, size_t workspace_bytes)
+{
+    return forward_packed16<__half>(stream, q, input, weight, bias, offset_mask, output, abs_offset_sum, workspace,
+                                 workspace_bytes);
+}
+
+int ebfi_dcnv2_backward_packed_fp16(void *stream, const ebfi_dcn_geom *q, const void *input, const float *weight,
+                                    const float *bias, const void *offset_mask, const void *grad_output,
+                                    void *grad_input, void *grad_offset_mask, float *grad_weight, float *grad_bias,
+                                    void *workspace, size_t workspace_bytes)
+{
+    (void)bias;
+    return backward_packed16<__half>(stream, q, input, weight, offset_mask, grad_output, grad_input, grad_offset_mask,
+                                  grad_weight, grad_bias, workspace, workspace_bytes);
 }
 
 }  // extern "C"

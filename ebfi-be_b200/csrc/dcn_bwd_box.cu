@@ -32,11 +32,12 @@
 //     the reference's atomicAdd, im2col_cuda.cu:249).
 // Non-finite gradients: a NaN/Inf anywhere in the (tile, group) makes the scale undefined; the box is then written as NaN
 // so that overflow checks on grad_input (AMP GradScaler) still fire.
-// Activation type T (float | __nv_bfloat16, the *_bf16 entries): offsets, masks and grad_output are read as T and widened
-// (a bf16 grad_output splits into hi = the value, lo = 0: the bits the float path stages for the widened tensor);
-// grad_offset / grad_mask and grad_input are rounded once from the fp32 values the float instantiation stores. With
-// several units per group the running fp32 sums of the owner threads then stay in shared memory until the group's
-// last unit. Boxes, partials, weights and grad_weight / grad_bias are fp32 in both.
+// Activation type T (float | __nv_bfloat16 | __half, the *_bf16 / *_fp16 entries): offsets, masks and grad_output are
+// read as T and widened (a bf16 grad_output splits into hi = the value, lo = 0, an fp16 one exactly into bf16 hi + lo:
+// the bits the float path stages for the widened tensor); grad_offset / grad_mask and grad_input are rounded once from
+// the fp32 values the float instantiation stores. With several units per group the running fp32 sums of the owner
+// threads then stay in shared memory until the group's last unit. Boxes, partials, weights and grad_weight / grad_bias
+// are fp32 in all three.
 #include "dcn_box.cuh"
 #include "dcn_common.cuh"
 #include "dp_comm.cuh"
@@ -44,6 +45,7 @@
 #include "umma.cuh"
 
 #include <algorithm>
+#include <type_traits>
 
 namespace ebfi_dcn {
 
@@ -451,6 +453,13 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
                     if constexpr (sizeof(T) == 4) {
                         va[q] = __ldg(reinterpret_cast<const float4 *>(src));
                         vb[q] = __ldg(reinterpret_cast<const float4 *>(src) + 1);
+                    } else if constexpr (std::is_same_v<T, __half>) {
+                        const uint4 u = __ldg(reinterpret_cast<const uint4 *>(src));     // fp16 -> fp32: exact conversion
+                        const __half2 *h = reinterpret_cast<const __half2 *>(&u);
+                        const float2 a = __half22float2(h[0]), b = __half22float2(h[1]);
+                        const float2 c = __half22float2(h[2]), e = __half22float2(h[3]);
+                        va[q] = make_float4(a.x, a.y, b.x, b.y);
+                        vb[q] = make_float4(c.x, c.y, e.x, e.y);
                     } else {
                         const uint4 u = __ldg(reinterpret_cast<const uint4 *>(src));     // bf16 -> fp32: the bits move up
                         va[q] = make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xFFFF0000u),
@@ -662,7 +671,7 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
                     // same thread owns the element in each of them -> plain read-modify-write, fixed order
                     T *gy = goff_g + (2u * (unsigned)t * uplane + (unsigned)cur.pix);
                     if constexpr (RUN_SUMS) {
-                        // bf16 outputs: the running sums stay fp32 (same additions as below), one rounding at the last unit
+                        // 16-bit outputs: the running sums stay fp32 (same additions as below), one rounding at the last unit
                         float *gs = gsum + 3 * t * TM + p;
                         if (cur.g & (pl.ncs - 1)) { g_y += gs[0]; g_x += gs[TM]; g_m += gs[2 * TM]; }
                         if ((cur.g & (pl.ncs - 1)) != pl.ncs - 1) {
@@ -962,7 +971,7 @@ int backward_box(cudaStream_t st, const DcnDims &d, const T *input, const float 
     }
     if (pl.use_om_tma && !(ebfi::aligned16(offset) && ebfi::aligned16(mask))) pl.use_om_tma = 0;
     if (pl.use_om_tma) {
-        constexpr CUtensorMapDataType om_type = sizeof(T) == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        constexpr CUtensorMapDataType om_type = tma::elem_type<T>();
         const uint64_t str[2] = {(uint64_t)d.Wo * sizeof(T), (uint64_t)d.Ho * d.Wo * sizeof(T)};
         const uint64_t dims_o[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.off_bp + 2 * d.dg * d.KK};
         const uint64_t dims_m[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.mask_bp + d.dg * d.KK};
@@ -1001,5 +1010,8 @@ template int backward_box<__nv_bfloat16>(cudaStream_t, const DcnDims &, const __
                                          const __nv_bfloat16 *, const __nv_bfloat16 *, const __nv_bfloat16 *, __nv_bfloat16 *,
                                          __nv_bfloat16 *, __nv_bfloat16 *, float *, float *, float *, float *, void *,
                                          const ebfi_dp::View *, bool);
+template int backward_box<__half>(cudaStream_t, const DcnDims &, const __half *, const float *, const __half *,
+                                  const __half *, const __half *, __half *, __half *, __half *, float *, float *,
+                                  float *, float *, void *, const ebfi_dp::View *, bool);
 
 }  // namespace ebfi_dcn

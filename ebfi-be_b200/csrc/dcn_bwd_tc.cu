@@ -450,6 +450,7 @@ int launch_nchw_to_blocked(cudaStream_t st, const T *src, float *dst, int BG, in
 }
 template int launch_nchw_to_blocked<float>(cudaStream_t, const float *, float *, int, int, void *, int);
 template int launch_nchw_to_blocked<__nv_bfloat16>(cudaStream_t, const __nv_bfloat16 *, float *, int, int, void *, int);
+template int launch_nchw_to_blocked<__half>(cudaStream_t, const __half *, float *, int, int, void *, int);
 
 // Extra scratch of the tensor-core backward: group-blocked copies of input and grad_input.
 size_t backward_tc_scratch_bytes(const DcnDims &d)

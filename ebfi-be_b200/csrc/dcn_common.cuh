@@ -4,6 +4,7 @@
 #include "common.cuh"
 
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 namespace ebfi_dcn {
 
@@ -54,16 +55,20 @@ __device__ __forceinline__ void det_add(long long *p, float v, float scale)
     atomicAdd(reinterpret_cast<unsigned long long *>(p), (unsigned long long)__float2ll_rn(v * scale));
 }
 
-// Activation element type T (float | __nv_bfloat16) of the tensor-core kernels: input, offset, mask and grad_output are
-// read as T and widened exactly, output and the activation gradients are rounded once (RN) from the fp32 values the
-// float instantiation stores. Everything in between (blocked input copy, boxes, weights, partials) is fp32.
+// Activation element type T (float | __nv_bfloat16 | __half) of the tensor-core kernels: input, offset, mask and
+// grad_output are read as T and widened exactly, output and the activation gradients are rounded once (RN) from the fp32
+// values the float instantiation stores; an fp16 store overflows to +-inf, as tensor.half() does. Everything in between
+// (blocked input copy, boxes, weights, partials) is fp32.
 __device__ __forceinline__ float act_f(float v) { return v; }
 __device__ __forceinline__ float act_f(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float act_f(__half v) { return __half2float(v); }
 __device__ __forceinline__ float ld_act(const float *p) { return __ldg(p); }
 __device__ __forceinline__ float ld_act(const __nv_bfloat16 *p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ float ld_act(const __half *p) { return __half2float(__ldg(p)); }
 template <typename T> __device__ __forceinline__ T st_act(float v);
 template <> __device__ __forceinline__ float st_act<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 st_act<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half st_act<__half>(float v) { return __float2half_rn(v); }
 
 template <typename T>
 __device__ __forceinline__ const T *off_ptr(const DcnDims &d, const T *offset, int b, int g, size_t plane)
@@ -173,7 +178,7 @@ __device__ __forceinline__ f8 ldg_f8(const float *p32B_aligned, bool ok)
 // {max_px sum_co |gO|, max |weight|, max |mask|} -> bound[3] (dcn.cu)
 int launch_det_bound(cudaStream_t st, const DcnDims &d, const float *gout, const float *weight, const float *mask, float *bound);
 
-// NCHW (BG*8 planes of HW pixels, T = float | __nv_bfloat16) -> fp32 group-blocked (BG, HW, 8) copy (dcn_bwd_tc.cu)
+// NCHW (BG*8 planes of HW pixels, T = float | __nv_bfloat16 | __half) -> fp32 group-blocked (BG, HW, 8) copy (dcn_bwd_tc.cu)
 template <typename T>
 int launch_nchw_to_blocked(cudaStream_t st, const T *src, float *dst, int BG, int HW, void *zero = nullptr, int zero_f4 = 0);
 

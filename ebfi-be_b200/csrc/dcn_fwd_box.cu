@@ -26,8 +26,9 @@
 //
 // fp32 parity: products are 3xTF32 (umma.cuh); the hi*hi chain is spread over several TMEM accumulators because
 // the tensor core's fp32 accumulate rounds toward zero.
-// Activation type T (float | __nv_bfloat16, the *_bf16 entries): the input is widened into the same fp32 blocked copy,
-// offsets / masks arrive by TMA as T planes and are widened where the samplers read them, the epilogue rounds once.
+// Activation type T (float | __nv_bfloat16 | __half, the *_bf16 / *_fp16 entries): the input is widened into the same
+// fp32 blocked copy, offsets / masks arrive by TMA as T planes and are widened where the samplers read them, the
+// epilogue rounds once.
 #include "dcn_box.cuh"
 #include "dcn_common.cuh"
 #include "tma.cuh"
@@ -502,7 +503,7 @@ int forward_tc(cudaStream_t st, const DcnDims &d, const T *input, const float *w
     }
     if (pl.use_om_tma && !(ebfi::aligned16(offset) && ebfi::aligned16(mask))) pl.use_om_tma = 0;
     if (pl.use_om_tma) {
-        constexpr CUtensorMapDataType om_type = sizeof(T) == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        constexpr CUtensorMapDataType om_type = tma::elem_type<T>();
         const uint64_t str[2] = {(uint64_t)d.Wo * sizeof(T), (uint64_t)d.Ho * d.Wo * sizeof(T)};
         const uint64_t dims_o[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.off_bp + 2 * d.dg * d.KK};
         const uint64_t dims_m[3] = {(uint64_t)d.Wo, (uint64_t)d.Ho, (uint64_t)(d.B - 1) * d.mask_bp + d.dg * d.KK};
@@ -535,5 +536,7 @@ template int forward_tc<float>(cudaStream_t, const DcnDims &, const float *, con
                                const float *, float *, void *, size_t);
 template int forward_tc<__nv_bfloat16>(cudaStream_t, const DcnDims &, const __nv_bfloat16 *, const float *, const float *,
                                        const __nv_bfloat16 *, const __nv_bfloat16 *, __nv_bfloat16 *, void *, size_t);
+template int forward_tc<__half>(cudaStream_t, const DcnDims &, const __half *, const float *, const float *,
+                                const __half *, const __half *, __half *, void *, size_t);
 
 }  // namespace ebfi_dcn

@@ -27,19 +27,25 @@
 
 #include <algorithm>
 #include <cuda_bf16.h>      // mbarrier + 1-D bulk (TMA) copy helpers
+#include <cuda_fp16.h>
 
 namespace {
 
 using ebfi::ceil_div;
 
-// Element types: fp32 (the reference's) and bf16 (storage only; all arithmetic is fp32).
+// Element types: fp32 (the reference's), bf16 and fp16 (storage only; all arithmetic is fp32). Loads widen exactly,
+// stores round once (RN); an fp16 store overflows to +-inf, as tensor.half() does.
 using bf16 = __nv_bfloat16;
+using fp16 = __half;
 __device__ __forceinline__ float ld_elt(const float *p) { return __ldg(p); }
 __device__ __forceinline__ float ld_elt(const bf16 *p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ float ld_elt(const fp16 *p) { return __half2float(__ldg(p)); }
 __device__ __forceinline__ float ld_elt_cg(const float *p) { return __ldcg(p); }
 __device__ __forceinline__ float ld_elt_cg(const bf16 *p) { return __bfloat162float(__ldcg(p)); }
+__device__ __forceinline__ float ld_elt_cg(const fp16 *p) { return __half2float(__ldcg(p)); }
 __device__ __forceinline__ void st_elt(float *p, float v) { *p = v; }
 __device__ __forceinline__ void st_elt(bf16 *p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void st_elt(fp16 *p, float v) { *p = __float2half_rn(v); }
 
 // PX-wide vectors (held as fp32) with streaming (evict-first) global access and shared-memory reads.
 template <int PX> struct Vec;
@@ -56,6 +62,11 @@ template <> struct Vec<4> {
         return Vec{{__uint_as_float(t.x << 16), __uint_as_float(t.x & 0xFFFF0000u),
                     __uint_as_float(t.y << 16), __uint_as_float(t.y & 0xFFFF0000u)}};
     }
+    __device__ __forceinline__ static Vec load_stream(const fp16 *p)
+    {
+        const uint2 t = __ldcs(reinterpret_cast<const uint2 *>(p));
+        return from_half2(t);
+    }
     __device__ __forceinline__ static Vec load_smem(const float *p)
     {
         const float4 t = *reinterpret_cast<const float4 *>(p);
@@ -67,6 +78,13 @@ template <> struct Vec<4> {
         return Vec{{__uint_as_float(t.x << 16), __uint_as_float(t.x & 0xFFFF0000u),
                     __uint_as_float(t.y << 16), __uint_as_float(t.y & 0xFFFF0000u)}};
     }
+    __device__ __forceinline__ static Vec load_smem(const fp16 *p) { return from_half2(*reinterpret_cast<const uint2 *>(p)); }
+    __device__ __forceinline__ static Vec from_half2(uint2 t)
+    {
+        const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(&t.x));
+        const float2 b = __half22float2(*reinterpret_cast<const __half2 *>(&t.y));
+        return Vec{{a.x, a.y, b.x, b.y}};
+    }
     __device__ __forceinline__ void store_stream(float *p) const
     {
         __stcs(reinterpret_cast<float4 *>(p), make_float4(v[0], v[1], v[2], v[3]));
@@ -77,13 +95,21 @@ template <> struct Vec<4> {
         __stcs(reinterpret_cast<uint2 *>(p), make_uint2(*reinterpret_cast<const uint32_t *>(&a),
                                                          *reinterpret_cast<const uint32_t *>(&b)));
     }
+    __device__ __forceinline__ void store_stream(fp16 *p) const
+    {
+        const __half2 a = __floats2half2_rn(v[0], v[1]), b = __floats2half2_rn(v[2], v[3]);
+        __stcs(reinterpret_cast<uint2 *>(p), make_uint2(*reinterpret_cast<const uint32_t *>(&a),
+                                                         *reinterpret_cast<const uint32_t *>(&b)));
+    }
 };
 template <> struct Vec<1> {
     float v[1];
     __device__ __forceinline__ static Vec load_stream(const float *p) { return Vec{{__ldcs(p)}}; }
     __device__ __forceinline__ static Vec load_stream(const bf16 *p) { return Vec{{__bfloat162float(*p)}}; }
+    __device__ __forceinline__ static Vec load_stream(const fp16 *p) { return Vec{{__half2float(*p)}}; }
     __device__ __forceinline__ void store_stream(float *p) const { __stcs(p, v[0]); }
     __device__ __forceinline__ void store_stream(bf16 *p) const { *p = __float2bfloat16_rn(v[0]); }
+    __device__ __forceinline__ void store_stream(fp16 *p) const { *p = __float2half_rn(v[0]); }
 };
 
 struct FacDims {
@@ -654,6 +680,13 @@ int ebfi_fac_forward_bf16(void *stream, const void *input, const void *kernel, v
                                   static_cast<bf16 *>(output), batch, channels, height_out, width_out, kernel_size);
 }
 
+int ebfi_fac_forward_fp16(void *stream, const void *input, const void *kernel, void *output,
+                          int batch, int channels, int height_out, int width_out, int kernel_size)
+{
+    return fac_forward_impl<fp16>(stream, static_cast<const fp16 *>(input), static_cast<const fp16 *>(kernel),
+                                  static_cast<fp16 *>(output), batch, channels, height_out, width_out, kernel_size);
+}
+
 size_t ebfi_fac_backward_workspace_bytes(int batch, int channels, int height_out, int width_out,
                                          int kernel_size)
 {
@@ -681,6 +714,16 @@ int ebfi_fac_backward_bf16(void *stream, const void *input, const void *kernel, 
     return fac_backward_impl<bf16>(stream, static_cast<const bf16 *>(input), static_cast<const bf16 *>(kernel),
                                    static_cast<const bf16 *>(grad_output), static_cast<bf16 *>(grad_input),
                                    static_cast<bf16 *>(grad_kernel), batch, channels, height_out, width_out,
+                                   kernel_size, workspace, workspace_bytes);
+}
+
+int ebfi_fac_backward_fp16(void *stream, const void *input, const void *kernel, const void *grad_output,
+                           void *grad_input, void *grad_kernel, int batch, int channels, int height_out,
+                           int width_out, int kernel_size, void *workspace, size_t workspace_bytes)
+{
+    return fac_backward_impl<fp16>(stream, static_cast<const fp16 *>(input), static_cast<const fp16 *>(kernel),
+                                   static_cast<const fp16 *>(grad_output), static_cast<fp16 *>(grad_input),
+                                   static_cast<fp16 *>(grad_kernel), batch, channels, height_out, width_out,
                                    kernel_size, workspace, workspace_bytes);
 }
 

@@ -35,10 +35,10 @@
 // Precision: tensors are fp32 at the boundary (like the reference); the conv operands are rounded to bf16
 // for the tensor cores, accumulation and the whole FAC part are fp32. Stated tolerance 1e-2 of max|out|
 // against the fp32/fp64 op sequence; 1e-5 against the same sequence with bf16-rounded conv operands.
-// Activation I/O (event / frame / output, and grad_output / grad_pre in the backward) may instead be bf16 (template
-// parameter T, the *_bf16 entries): only the loads convert (exactly) and the stores round once (RN) from the same
-// fp32 values, so on bf16-valued inputs a bf16 instantiation computes bit-identically to the fp32 one. Weights, bias,
-// grad_event_fac and grad_bias stay fp32.
+// Activation I/O (event / frame / output, and grad_output / grad_pre in the backward) may instead be bf16 or fp16
+// (template parameter T, the *_bf16 / *_fp16 entries): only the loads convert (exactly) and the stores round once (RN)
+// from the same fp32 values, so on bf16- or fp16-valued inputs such an instantiation computes bit-identically to the
+// fp32 one. The conv operands are bf16 for every T. Weights, bias, grad_event_fac and grad_bias stay fp32.
 //
 // Backward (ebfi_kpn_fused_backward): the same kernel with BWD = true recomputes the pre-activation P in TMEM
 // through the identical main loop (same operands, same MMA chain -> bit-identical P, so forward and backward take
@@ -56,6 +56,7 @@
 #include "umma.cuh"
 
 #include <algorithm>
+#include <cuda_fp16.h>
 
 namespace {
 
@@ -83,12 +84,15 @@ struct KpnDims {
     float slope;
 };
 
-// Activation element type T (float | __nv_bfloat16): loads widen to fp32 exactly, stores round once (RN).
+// Activation element type T (float | __nv_bfloat16 | __half): loads widen to fp32 exactly, stores round once (RN; an
+// fp16 store overflows to +-inf, as tensor.half() does).
 __device__ __forceinline__ float ld_act(const float *p) { return __ldg(p); }
 __device__ __forceinline__ float ld_act(const __nv_bfloat16 *p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ float ld_act(const __half *p) { return __half2float(__ldg(p)); }
 template <typename T> __device__ __forceinline__ T st_act(float v);
 template <> __device__ __forceinline__ float st_act<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 st_act<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half st_act<__half>(float v) { return __float2half_rn(v); }
 
 // Backward-only operands of the fused kernel (unused by the forward instantiation).
 template <typename T>
@@ -669,6 +673,16 @@ int ebfi_kpn_fused_forward_bf16(void *stream, const void *event_feat, const void
                        kernel_size, workspace, workspace_bytes);
 }
 
+int ebfi_kpn_fused_forward_fp16(void *stream, const void *event_feat, const void *frame_feat, const float *conv_weight,
+                                const float *conv_bias, float negative_slope, void *output, int batch,
+                                int channels_event, int channels_frame, int height, int width, int kernel_size,
+                                void *workspace, size_t workspace_bytes)
+{
+    return kpn_forward(stream, static_cast<const __half *>(event_feat), static_cast<const __half *>(frame_feat),
+                       conv_weight, conv_bias, negative_slope, static_cast<__half *>(output), batch, channels_event,
+                       channels_frame, height, width, kernel_size, workspace, workspace_bytes);
+}
+
 size_t ebfi_kpn_fused_backward_workspace_bytes(int batch, int channels_event, int channels_frame, int height, int width,
                                                int kernel_size)
 {
@@ -698,6 +712,18 @@ int ebfi_kpn_fused_backward_bf16(void *stream, const void *event_feat, const voi
                         static_cast<const __nv_bfloat16 *>(grad_output), static_cast<__nv_bfloat16 *>(grad_pre),
                         grad_event_fac, grad_bias, batch, channels_event, channels_frame, height, width, kernel_size,
                         workspace, workspace_bytes);
+}
+
+int ebfi_kpn_fused_backward_fp16(void *stream, const void *event_feat, const void *frame_feat, const float *conv_weight,
+                                 const float *conv_bias, float negative_slope, const void *grad_output, void *grad_pre,
+                                 float *grad_event_fac, float *grad_bias, int batch, int channels_event,
+                                 int channels_frame, int height, int width, int kernel_size, void *workspace,
+                                 size_t workspace_bytes)
+{
+    return kpn_backward(stream, static_cast<const __half *>(event_feat), static_cast<const __half *>(frame_feat),
+                        conv_weight, conv_bias, negative_slope, static_cast<const __half *>(grad_output),
+                        static_cast<__half *>(grad_pre), grad_event_fac, grad_bias, batch, channels_event,
+                        channels_frame, height, width, kernel_size, workspace, workspace_bytes);
 }
 
 }  // extern "C"

@@ -5,7 +5,22 @@
 #include "common.cuh"
 #include "umma.cuh"
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+#include <type_traits>
+
 namespace tma {
+
+// tensor-map element type of an activation type T (float | __nv_bfloat16 | __half)
+template <typename T> constexpr CUtensorMapDataType elem_type()
+{
+    if constexpr (std::is_same_v<T, float>) return CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    else if constexpr (std::is_same_v<T, __half>) return CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    else {
+        static_assert(std::is_same_v<T, __nv_bfloat16>, "activation type");
+        return CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    }
+}
 
 // 3-D tensor of `elem_bytes`-sized elements, dims fastest -> slowest = {d0, d1, d2}, byte strides of d1 and d2
 // (multiples of 16); box = the tile one copy moves; out-of-range elements are read as zero. Returns an EBFI_* code.

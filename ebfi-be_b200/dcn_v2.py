@@ -23,14 +23,14 @@ logger = logging.getLogger("base")
 
 
 def _as_dtypes(grads, tensors):
-    """Gradients in the dtype of the tensor each one belongs to (bf16 calls return bf16 activation gradients; under
-    autocast an input can be fp32)."""
+    """Gradients in the dtype of the tensor each one belongs to (bf16 / fp16 calls return 16-bit activation gradients;
+    under autocast an input can be fp32)."""
     return tuple(gr.to(t.dtype) for gr, t in zip(grads, tensors))
 
 
 class _DCNv2(Function):
-    """Modulated deformable convolution; arguments as dcn_v2.py:18-21. bf16 and mixed bf16 / fp32 tensors (autocast)
-    follow shims/_ext.py: the output is bf16, each gradient has its input's dtype."""
+    """Modulated deformable convolution; arguments as dcn_v2.py:18-21. bf16 or fp16 tensors, also mixed with fp32 ones
+    (autocast), follow shims/_ext.py: the output is 16-bit, each gradient has its input's dtype."""
 
     @staticmethod
     def forward(ctx, input, offset, mask, weight, bias, stride, padding, dilation, deformable_groups):

@@ -9,9 +9,9 @@ on the tensor cores and writes dL/dP, the FAC/ReplicationPad part of dL/dEvent a
 and input gradients then run on torch's convolution backward, as the reference's nn.Conv2d does. Neither the
 pre-activation nor the kernel tensor is kept for the backward. `KernelPrediction.fused_backward = True` trains
 through it; by default the module trains on the reference's op sequence. `KernelConvFACBF16Function` is the same
-fused forward and backward for bf16 activations (torch.autocast's mixed precision): the kernel reads and writes bf16
-activations and keeps P and the kernel tensor in fp32 registers, and the conv's gradients run as the bf16 convolution
-backward autocast's nn.Conv2d would run.
+fused forward and backward for bf16 or fp16 activations (torch.autocast's mixed precision): the kernel reads and writes
+the 16-bit activations and keeps P and the kernel tensor in fp32 registers, and the conv's gradients run as the 16-bit
+convolution backward autocast's nn.Conv2d would run.
 """
 import torch
 from torch import nn
@@ -20,19 +20,23 @@ from . import _lib as L
 from .kernelconv2d import KernelConv2D
 
 
+# activation dtype -> suffix of the fused block's C entries
+_SUFFIX = {torch.float32: "", torch.bfloat16: "_bf16", torch.float16: "_fp16"}
+
+
 def kernelconv_fac_fused(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope=0.01):
-    """out = KernelConv2D(K)(event_feat, LeakyReLU(conv3x3(cat([event_feat, frame_feat], 1)))) — CUDA tensors, all fp32
-    or all bf16; conv operands are rounded to bf16 for the tensor cores (fp32 accumulate, fp32 FAC)."""
+    """out = KernelConv2D(K)(event_feat, LeakyReLU(conv3x3(cat([event_feat, frame_feat], 1)))) — CUDA tensors, all fp32,
+    all bf16 or all fp16; conv operands are rounded to bf16 for the tensor cores (fp32 accumulate, fp32 FAC)."""
     L.require_cuda(event_feat, frame_feat, conv_weight, conv_bias)
     dts = {t.dtype for t in (event_feat, frame_feat, conv_weight, conv_bias)}
-    if dts != {torch.float32} and dts != {torch.bfloat16}:
-        raise RuntimeError("kernelconv_fac_fused: all tensors must be float32 or all bfloat16, got "
+    if len(dts) != 1 or not dts <= set(_SUFFIX):
+        raise RuntimeError("kernelconv_fac_fused: all tensors must be float32, all bfloat16 or all float16, got "
                            f"{sorted(str(d) for d in dts)}")
     if torch.is_grad_enabled() and any(t.requires_grad for t in (event_feat, frame_feat, conv_weight, conv_bias)):
         raise RuntimeError("kernelconv_fac_fused is forward-only; run it under torch.no_grad() "
                            "(training goes through KernelConv2DFunction)")
-    # bfloat16 model (the 720p inference config): the kernel reads the bf16 activations and rounds its output once;
-    # the weights' fp32 copies are exact (and small)
+    # bfloat16 / float16 model (the 720p inference config runs bf16): the kernel reads the 16-bit activations and
+    # rounds its output once; the weights' fp32 copies are exact (and small)
     return _fused_forward(event_feat, frame_feat, conv_weight.float(), conv_bias.float(), kernel_size, negative_slope)
 
 
@@ -48,7 +52,7 @@ def _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, wha
 
 
 def _fused_forward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope):
-    """ebfi_kpn_fused_forward (fp32 activations) or ebfi_kpn_fused_forward_bf16 (bf16 activations) on CUDA tensors
+    """ebfi_kpn_fused_forward (fp32 activations) or its _bf16 / _fp16 variant (16-bit activations) on CUDA tensors
     with fp32 weight and bias: the one forward of kernelconv_fac_fused, KernelConvFACFunction and
     KernelConvFACBF16Function. The output has the activations' dtype."""
     B, Ce, Cf, H, W, K = _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, "kernelconv_fac_fused")
@@ -58,7 +62,7 @@ def _fused_forward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, 
         out = torch.empty_like(event_feat)
         nbytes = lib.ebfi_kpn_fused_workspace_bytes(B, Ce, Cf, H, W, K)
         ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=event_feat.device)
-        fwd = lib.ebfi_kpn_fused_forward_bf16 if event_feat.dtype == torch.bfloat16 else lib.ebfi_kpn_fused_forward
+        fwd = getattr(lib, "ebfi_kpn_fused_forward" + _SUFFIX[event_feat.dtype])
         L.check(fwd(L.stream_ptr(event_feat.device), L.ptr(event_feat), L.ptr(frame_feat),
                     L.ptr(conv_weight), L.ptr(conv_bias), float(negative_slope), L.ptr(out),
                     B, Ce, Cf, H, W, K, L.ptr(ws), nbytes), "kernelconv_fac_fused")
@@ -79,30 +83,34 @@ def kernelconv_fac_fused_backward(event_feat, frame_feat, conv_weight, conv_bias
 
 def kernelconv_fac_fused_backward_bf16(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope,
                                        grad_output):
-    """ebfi_kpn_fused_backward_bf16: kernelconv_fac_fused_backward for bf16 event_feat, frame_feat and grad_output
-    (weight and bias fp32 or bf16; they are used as fp32) -> (grad_pre bf16, grad_event_fac fp32, grad_bias fp32).
-    grad_pre is the fp32 kernel's grad_pre rounded once to bf16; grad_event_fac and grad_bias are the fp32 kernel's."""
+    """ebfi_kpn_fused_backward_bf16 / _fp16: kernelconv_fac_fused_backward for event_feat, frame_feat and grad_output
+    all bf16 or all fp16 (weight and bias fp32 or of that type; they are used as fp32) -> (grad_pre of that type,
+    grad_event_fac fp32, grad_bias fp32). grad_pre is the fp32 kernel's grad_pre rounded once to the 16-bit type;
+    grad_event_fac and grad_bias are the fp32 kernel's."""
     L.require_cuda(event_feat, frame_feat, conv_weight, conv_bias, grad_output)
-    _require_bf16_io("kernelconv_fac_fused_backward_bf16", dict(event_feat=event_feat, frame_feat=frame_feat,
+    _require_half_io("kernelconv_fac_fused_backward_bf16", dict(event_feat=event_feat, frame_feat=frame_feat,
                                                                 grad_output=grad_output),
                      dict(conv_weight=conv_weight, conv_bias=conv_bias))
     return _fused_backward(event_feat, frame_feat, conv_weight.float(), conv_bias.float(), kernel_size,
                            negative_slope, grad_output, "kernelconv_fac_fused_backward_bf16")
 
 
-def _require_bf16_io(what, activations, parameters):
-    """bf16 activations; parameters fp32 (autocast) or bf16 (a .bfloat16() model)."""
-    for k, t in activations.items():
-        if t.dtype != torch.bfloat16:
-            raise RuntimeError(f"{what}: {k} must be bfloat16, got {t.dtype} "
-                               "(fp32 activations go through the fp32 entries)")
+def _require_half_io(what, activations, parameters):
+    """Activations all bf16 or all fp16; parameters fp32 (autocast) or of the activations' type (a .bfloat16() or
+    .half() model)."""
+    dts = {t.dtype for t in activations.values()}
+    if len(dts) != 1 or not dts <= {torch.bfloat16, torch.float16}:
+        got = ", ".join(f"{k} {t.dtype}" for k, t in activations.items())
+        raise RuntimeError(f"{what}: the activations must be all bfloat16 or all float16, got {got} "
+                           "(fp32 activations go through the fp32 entries)")
+    half = dts.pop()
     for k, t in parameters.items():
-        if t.dtype not in (torch.float32, torch.bfloat16):
-            raise RuntimeError(f"{what}: {k} must be float32 or bfloat16, got {t.dtype}")
+        if t.dtype not in (torch.float32, half):
+            raise RuntimeError(f"{what}: {k} must be float32 or {half}, got {t.dtype}")
 
 
 def _fused_backward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope, grad_output, what):
-    """ebfi_kpn_fused_backward or its _bf16 variant, chosen by the activations' dtype; fp32 weight and bias."""
+    """ebfi_kpn_fused_backward or its _bf16 / _fp16 variant, chosen by the activations' dtype; fp32 weight and bias."""
     B, Ce, Cf, H, W, K = _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, what)
     if tuple(grad_output.shape) != tuple(event_feat.shape):
         raise RuntimeError(f"{what}: grad_output must have the event features' shape")
@@ -116,7 +124,7 @@ def _fused_backward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size,
         grad_bias = torch.empty(Ce * K * K, device=dev)
         nbytes = lib.ebfi_kpn_fused_backward_workspace_bytes(B, Ce, Cf, H, W, K)
         ws = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
-        bwd = lib.ebfi_kpn_fused_backward_bf16 if event_feat.dtype == torch.bfloat16 else lib.ebfi_kpn_fused_backward
+        bwd = getattr(lib, "ebfi_kpn_fused_backward" + _SUFFIX[event_feat.dtype])
         L.check(bwd(L.stream_ptr(dev), L.ptr(event_feat), L.ptr(frame_feat), L.ptr(conv_weight),
                     L.ptr(conv_bias), float(negative_slope), L.ptr(grad_output),
                     L.ptr(grad_pre), L.ptr(grad_event_fac), L.ptr(grad_bias),
@@ -161,21 +169,21 @@ class KernelConvFACFunction(torch.autograd.Function):
 
 
 class KernelConvFACBF16Function(torch.autograd.Function):
-    """KernelConvFACFunction for bf16 activations, as torch.autocast(dtype=torch.bfloat16) feeds the block:
-    event_feat and frame_feat bf16; conv_weight and conv_bias fp32 (autocast parameters) or bf16 (a .bfloat16()
-    model); all CUDA. Returns bf16.
+    """KernelConvFACFunction for 16-bit activations, as torch.autocast feeds the block (dtype=torch.bfloat16, or its
+    default torch.float16): event_feat and frame_feat both bf16 or both fp16; conv_weight and conv_bias fp32 (autocast
+    parameters) or of the activations' type (a .bfloat16() / .half() model); all CUDA. Returns the activations' type.
 
-    Saves only the four inputs. The forward and the fused backward kernel read the bf16 activations and use the
-    weights as fp32 (exact for bf16 ones); P and LeakyReLU(P) stay fp32 in registers, the output and dL/dP are
-    rounded once to bf16. The conv's weight and input gradients are the bf16 convolution backward of dL/dP that
-    autocast's nn.Conv2d runs (bf16 cat(event, frame), bf16 weight). grad_event = (FAC part + conv part) summed in
-    fp32 and rounded once; weight and bias gradients come back in the parameters' dtype. The backward does not
-    depend on the autocast state it runs under."""
+    Saves only the four inputs. The forward and the fused backward kernel read the 16-bit activations and use the
+    weights as fp32 (exact for 16-bit ones); P and LeakyReLU(P) stay fp32 in registers, the output and dL/dP are
+    rounded once to the 16-bit type. The conv's weight and input gradients are the 16-bit convolution backward of
+    dL/dP that autocast's nn.Conv2d runs (16-bit cat(event, frame) and weight). grad_event = (FAC part + conv part)
+    summed in fp32 and rounded once; weight and bias gradients come back in the parameters' dtype. The backward does
+    not depend on the autocast state it runs under."""
 
     @staticmethod
     def forward(ctx, event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope=0.01):
         L.require_cuda(event_feat, frame_feat, conv_weight, conv_bias)
-        _require_bf16_io("KernelConvFACBF16Function", dict(event_feat=event_feat, frame_feat=frame_feat),
+        _require_half_io("KernelConvFACBF16Function", dict(event_feat=event_feat, frame_feat=frame_feat),
                          dict(conv_weight=conv_weight, conv_bias=conv_bias))
         ctx.kernel_size, ctx.negative_slope = int(kernel_size), float(negative_slope)
         ctx.save_for_backward(event_feat, frame_feat, conv_weight, conv_bias)
@@ -186,18 +194,19 @@ class KernelConvFACBF16Function(torch.autograd.Function):
     def backward(ctx, grad_output):
         ev, fr, w, b = ctx.saved_tensors
         need_ev, need_fr, need_w, need_b = ctx.needs_input_grad[:4]
+        half = ev.dtype
         with torch.autocast("cuda", enabled=False):
             grad_pre, grad_ev, grad_b = kernelconv_fac_fused_backward_bf16(
-                ev, fr, w, b, ctx.kernel_size, ctx.negative_slope, grad_output.bfloat16())
+                ev, fr, w, b, ctx.kernel_size, ctx.negative_slope, grad_output.to(half))
             need_x = need_ev or need_fr
             grad_x = grad_w = grad_fr = None
             if need_x or need_w:
                 x = torch.cat([ev, fr], 1) if fr.shape[1] else ev
                 grad_x, grad_w, _ = torch.ops.aten.convolution_backward(
-                    grad_pre, x, w.bfloat16(), None, [1, 1], [1, 1], [1, 1], False, [0, 0], 1, [need_x, need_w, False])
+                    grad_pre, x, w.to(half), None, [1, 1], [1, 1], [1, 1], False, [0, 0], 1, [need_x, need_w, False])
             if need_x:
                 Ce = ev.shape[1]
-                grad_ev = (grad_ev + grad_x[:, :Ce].float()).bfloat16()
+                grad_ev = (grad_ev + grad_x[:, :Ce].float()).to(half)
                 grad_fr = grad_x[:, Ce:] if need_fr else None
         return (grad_ev if need_ev else None, grad_fr, grad_w.to(w.dtype) if need_w else None,
                 grad_b.to(b.dtype) if need_b else None, None, None)
@@ -236,11 +245,11 @@ class KernelPrediction(nn.Module):
     a supported shape train through `KernelConvFACFunction` (fused forward and backward; nothing but the inputs is
     kept for the backward). Opt-in because it changes training precision: the pre-activation comes from bf16 conv
     operands, so the gradients differ more from the fp64 op sequence than the TF32 reference sequence's do (measured
-    ratio in DESIGN §3). With bf16 event and frame tensors (torch.autocast(dtype=torch.bfloat16) mixed precision, or
-    a .bfloat16() model) and fp32 or bf16 parameters, the same opt-in trains through `KernelConvFACBF16Function`
-    instead: bf16 activation I/O, P and the kernel tensor in fp32 registers, the conv's gradients as autocast's bf16
-    convolution backward (precision and measured numbers in DESIGN §3). Every other case does exactly what it does with
-    `fused_backward = False`."""
+    ratio in DESIGN §3). With event and frame tensors both bf16 or both fp16 (torch.autocast mixed precision, or a
+    .bfloat16() / .half() model) and parameters fp32 or of that type, the same opt-in trains through
+    `KernelConvFACBF16Function` instead: 16-bit activation I/O, P and the kernel tensor in fp32 registers, the conv's
+    gradients as autocast's 16-bit convolution backward (precision and measured numbers in DESIGN §3). Every other case
+    does exactly what it does with `fused_backward = False`."""
 
     fused = True
     fused_backward = False
@@ -255,7 +264,7 @@ class KernelPrediction(nn.Module):
         conv = self.KernelConv.conv2d
         needs_grad = torch.is_grad_enabled() and (EventTensor.requires_grad or FrameTensor.requires_grad
                                                   or conv.weight.requires_grad)
-        if self.fused and not needs_grad and EventTensor.is_cuda and EventTensor.dtype in (torch.float32, torch.bfloat16) \
+        if self.fused and not needs_grad and EventTensor.is_cuda and EventTensor.dtype in _SUFFIX \
                 and FrameTensor.dtype == EventTensor.dtype and conv.weight.dtype == EventTensor.dtype \
                 and kernelconv_fac_fused_supported(EventTensor.shape[1], FrameTensor.shape[1], self.kernel_size):
             return kernelconv_fac_fused(EventTensor, FrameTensor, conv.weight, conv.bias, self.kernel_size,
@@ -265,8 +274,9 @@ class KernelPrediction(nn.Module):
                 and kernelconv_fac_fused_supported(EventTensor.shape[1], FrameTensor.shape[1], self.kernel_size):
             return KernelConvFACFunction.apply(EventTensor, FrameTensor, conv.weight, conv.bias, self.kernel_size,
                                                self.KernelConv.activation.negative_slope)
-        if self.fused_backward and needs_grad and EventTensor.is_cuda and EventTensor.dtype == torch.bfloat16 \
-                and FrameTensor.dtype == torch.bfloat16 and conv.weight.dtype in (torch.float32, torch.bfloat16) \
+        if self.fused_backward and needs_grad and EventTensor.is_cuda \
+                and EventTensor.dtype in (torch.bfloat16, torch.float16) and FrameTensor.dtype == EventTensor.dtype \
+                and conv.weight.dtype in (torch.float32, EventTensor.dtype) \
                 and conv.bias.dtype == conv.weight.dtype \
                 and kernelconv_fac_fused_supported(EventTensor.shape[1], FrameTensor.shape[1], self.kernel_size):
             return KernelConvFACBF16Function.apply(EventTensor, FrameTensor, conv.weight, conv.bias, self.kernel_size,

@@ -4,17 +4,19 @@
 Differences, all deliberate:
   * CUDA only. The reference dispatches CPU tensors to dcn_v2_cpu_* (dcn_v2.h:35-44), whose
     forward returns uninitialised memory (cpu/dcn_v2_cpu.cpp:65,127); here a CPU tensor raises.
-  * bf16 (new; the reference is fp32-only). Activations (input, offset, mask / offset_mask, grad_output) that are
-    bf16 — all of them, or some with the rest fp32, as under torch.autocast — run as all-bf16: fp32 activations are
-    rounded to bf16 once (autocast's own cast). weight / bias may then be fp32 or bf16 and are used as fp32. Outputs and
-    activation gradients are bf16, grad_weight / grad_bias have the parameter's dtype. The tensor-core kernels read and
-    write bf16 directly; every other call (other shapes, EBFI_DCN_DETERMINISTIC, EBFI_DCN_IMPL=simt, a misaligned
-    grad_output) converts at this boundary (_bf16_via_fp32) with the same result dtypes. Both give the bits of the
-    fp32 kernels on the widened values, rounded once. With fp32 activations everything must be fp32, as in the
-    reference.
+  * 16-bit floats, bf16 or fp16 (new; the reference is fp32-only). Activations (input, offset, mask / offset_mask,
+    grad_output) of one 16-bit type — all of them, or some with the rest fp32, as under torch.autocast — run in that
+    type: fp32 activations are rounded to it once (autocast's own cast). weight / bias may then be fp32 or of that type
+    and are used as fp32. Outputs and activation gradients have the 16-bit type, grad_weight / grad_bias the
+    parameter's dtype. The tensor-core kernels read and write the 16-bit activations directly; every other call (other
+    shapes, EBFI_DCN_DETERMINISTIC, EBFI_DCN_IMPL=simt, a misaligned grad_output) converts at this boundary
+    (_via_fp32) with the same result dtypes. Both give the bits of the fp32 kernels on the widened values, rounded
+    once; an fp16 result beyond the fp16 range is inf, as tensor.half() gives. bf16 mixed with fp16 raises. With fp32
+    activations everything must be fp32, as in the reference.
   * the deformable PS-ROI pooling pair (dcn_v2.h:94-190) is out of scope and raises
     NotImplementedError (it is never imported by EBFI-BE).
 """
+import functools
 import os
 
 import torch
@@ -93,9 +95,13 @@ def _geom(input, weight, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
 _PARAMS = ("weight", "bias")
 
 
+# 16-bit activation dtypes -> suffix of their C entries
+_HALF = {torch.bfloat16: "_bf16", torch.float16: "_fp16"}
+
+
 def _check_cuda(**named):
-    """float32: every tensor is fp32 (the reference). bfloat16: the activations are bf16, or bf16 and fp32 mixed, and
-    the parameters fp32 or bf16. Anything else raises."""
+    """float32: every tensor is fp32 (the reference). bfloat16 / float16: the activations are of that type, or of it
+    and fp32 mixed, and the parameters fp32 or of that type. Anything else (bf16 with fp16, fp64) raises."""
     for k, t in named.items():
         if not t.is_cuda:
             raise RuntimeError(f"{k} must be a CUDA tensor")   # AT_ASSERTM, dcn_v2_cuda.cu:38-42
@@ -103,26 +109,31 @@ def _check_cuda(**named):
     acts = {t.dtype for k, t in named.items() if k not in _PARAMS}
     if dts == {torch.float32}:
         return torch.float32
-    if torch.bfloat16 in acts and dts <= {torch.float32, torch.bfloat16}:
-        return torch.bfloat16
-    raise RuntimeError("dcn_v2: all tensors must be float32 (the reference's `using scalar_t = float`) or all "
-                       f"bfloat16, got {sorted(str(d) for d in dts)}")
+    for half in _HALF:
+        if half in acts and dts <= {torch.float32, half}:
+            return half
+    raise RuntimeError("dcn_v2: all tensors must be float32 (the reference's `using scalar_t = float`), or the "
+                       "activations one 16-bit type (bfloat16 or float16) with parameters of it or float32, got "
+                       f"{sorted(str(d) for d in dts)}")
 
 
-def _bf16_via_fp32(fn, tensors, ints, out_dtypes=None):
-    """bfloat16 at the boundary: the fp32 entry `fn` on exactly widened copies, results rounded once to bf16 (or
-    converted to `out_dtypes`, one per result). This is what a bf16 call runs where the kernels have no native bf16
-    I/O: the CUDA-core kernels (shapes outside the tensor-core ones, EBFI_DCN_IMPL=simt), the deterministic backward,
-    and a grad_output that is not 16-byte aligned. It costs extra elementwise passes, and the widened input is a new
-    tensor, so a backward through here re-blocks it."""
+def _via_fp32(dtype, fn, tensors, ints, out_dtypes=None):
+    """16-bit activations at the boundary: the fp32 entry `fn` on exactly widened copies, results rounded once to
+    `dtype` (or converted to `out_dtypes`, one per result). This is what a bf16 / fp16 call runs where the kernels have
+    no native 16-bit I/O: the CUDA-core kernels (shapes outside the tensor-core ones, EBFI_DCN_IMPL=simt), the
+    deterministic backward, and a grad_output that is not 16-byte aligned. It costs extra elementwise passes, and the
+    widened input is a new tensor, so a backward through here re-blocks it."""
     out = fn(*(t.float() for t in tensors), *ints)
     if torch.is_tensor(out):
-        return out.to(out_dtypes[0] if out_dtypes else torch.bfloat16)
-    return [o.to(dt) for o, dt in zip(out, out_dtypes or [torch.bfloat16] * len(out))]
+        return out.to(out_dtypes[0] if out_dtypes else dtype)
+    return [o.to(dt) for o, dt in zip(out, out_dtypes or [dtype] * len(out))]
 
 
-def _native_bf16(rc, what):
-    """True when a *_bf16 entry ran; False when it declined the call (EBFI_ERR_UNSUPPORTED, nothing was enqueued)."""
+_bf16_via_fp32 = functools.partial(_via_fp32, torch.bfloat16)
+
+
+def _ran_native(rc, what):
+    """True when a 16-bit entry ran; False when it declined the call (EBFI_ERR_UNSUPPORTED, nothing was enqueued)."""
     if rc == L.EBFI_ERR_UNSUPPORTED:
         return False
     L.check(rc, what)
@@ -141,10 +152,11 @@ def _check_offset_mask(g, ho, wo, offset, mask):
 def dcn_v2_forward(input, weight, bias, offset, mask, kernel_h, kernel_w, stride_h, stride_w,
                    pad_h, pad_w, dilation_h, dilation_w, deformable_group):
     """dcn_v2_cuda_forward (src/cuda/dcn_v2_cuda.cu:20-95). Returns a new (B, Cout, Ho, Wo) tensor."""
-    bf16 = _check_cuda(input=input, weight=weight, bias=bias, offset=offset, mask=mask) == torch.bfloat16
+    dt = _check_cuda(input=input, weight=weight, bias=bias, offset=offset, mask=mask)
+    half = _HALF.get(dt)
     ints = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group)
-    if bf16:
-        input, offset, mask = (t.bfloat16() for t in (input, offset, mask))
+    if half:
+        input, offset, mask = (t.to(dt) for t in (input, offset, mask))
         weight, bias = weight.float(), bias.float()
     g, ho, wo = _geom(input, weight, *ints)
     _check_offset_mask(g, ho, wo, offset, mask)
@@ -156,10 +168,10 @@ def dcn_v2_forward(input, weight, bias, offset, mask, kernel_h, kernel_w, stride
         ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
         args = (L.stream_ptr(input.device), g, L.ptr(input), L.ptr(weight), L.ptr(bias), L.ptr(offset), L.ptr(mask),
                 L.ptr(output), L.ptr(ws), nbytes)
-        if not bf16:
+        if not half:
             L.check(lib.ebfi_dcnv2_forward(*args), "dcn_v2_forward")
-        elif not _native_bf16(lib.ebfi_dcnv2_forward_bf16(*args), "dcn_v2_forward_bf16"):
-            return _bf16_via_fp32(dcn_v2_forward, (input, weight, bias, offset, mask), ints)
+        elif not _ran_native(getattr(lib, "ebfi_dcnv2_forward" + half)(*args), "dcn_v2_forward" + half):
+            return _via_fp32(dt, dcn_v2_forward, (input, weight, bias, offset, mask), ints)
         _remember_blocked(lib, g, input, ws)
     return output
 
@@ -176,11 +188,11 @@ def dcn_v2_backward(input, weight, bias, offset, mask, grad_output, kernel_h, ke
         raise RuntimeError("input tensor has to be contiguous")
     if not weight.is_contiguous():
         raise RuntimeError("weight tensor has to be contiguous")
-    bf16 = _check_cuda(input=input, weight=weight, bias=bias, offset=offset, mask=mask,
-                       grad_output=grad_output) == torch.bfloat16
+    dt = _check_cuda(input=input, weight=weight, bias=bias, offset=offset, mask=mask, grad_output=grad_output)
+    half = _HALF.get(dt)
     ints = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group)
-    if bf16:
-        input, offset, mask, grad_output = (t.bfloat16() for t in (input, offset, mask, grad_output))
+    if half:
+        input, offset, mask, grad_output = (t.to(dt) for t in (input, offset, mask, grad_output))
         param_dtypes = [weight.dtype, bias.dtype]
         weight, bias = weight.float(), bias.float()
     g, ho, wo = _geom(input, weight, *ints, _deterministic())
@@ -196,21 +208,21 @@ def dcn_v2_backward(input, weight, bias, offset, mask, grad_output, kernel_h, ke
         in_ptr = _blocked_input_ptr(g, input)
         args = (L.stream_ptr(input.device), g, in_ptr, L.ptr(weight), L.ptr(bias), L.ptr(offset), L.ptr(mask),
                 L.ptr(grad_output), *(L.ptr(t) for t in grads), L.ptr(ws), nbytes)
-        if not bf16:
+        if not half:
             if comm is None:
                 L.check(lib.ebfi_dcnv2_backward(*args), "dcn_v2_backward")
             else:
                 L.check(lib.ebfi_dcnv2_backward_dp(*args, comm.struct, 1 if defer else 0), "dcn_v2_backward_dp")
             return grads
         if comm is None:
-            ran = _native_bf16(lib.ebfi_dcnv2_backward_bf16(*args), "dcn_v2_backward_bf16")
+            ran = _ran_native(getattr(lib, "ebfi_dcnv2_backward" + half)(*args), "dcn_v2_backward" + half)
         else:
-            ran = _native_bf16(lib.ebfi_dcnv2_backward_dp_bf16(*args, comm.struct, 1 if defer else 0),
-                               "dcn_v2_backward_dp_bf16")
-    out_dtypes = [torch.bfloat16] * 3 + param_dtypes
+            ran = _ran_native(getattr(lib, "ebfi_dcnv2_backward_dp" + half)(*args, comm.struct, 1 if defer else 0),
+                              "dcn_v2_backward_dp" + half)
+    out_dtypes = [dt] * 3 + param_dtypes
     if not ran:
-        return _bf16_via_fp32(dcn_v2_backward, (input, weight, bias, offset, mask, grad_output), ints + (comm, defer),
-                              out_dtypes)
+        return _via_fp32(dt, dcn_v2_backward, (input, weight, bias, offset, mask, grad_output), ints + (comm, defer),
+                         out_dtypes)
     return [t.to(dt) for t, dt in zip(grads, out_dtypes)]
 
 
@@ -234,10 +246,11 @@ def dcn_v2_forward_packed(input, weight, bias, offset_mask, kernel_h, kernel_w, 
     output, i.e. chunk / cat / sigmoid of DCN.forward / DCN_sep.forward (dcn_v2.py:179-187, :217-227)
     folded into the kernel. `abs_offset_sum`: optional 1-element fp32 CUDA tensor that receives
     sum |offset| (for the `offset_mean > 100` warning, :221-223)."""
-    bf16 = _check_cuda(input=input, weight=weight, bias=bias, offset_mask=offset_mask) == torch.bfloat16
+    dt = _check_cuda(input=input, weight=weight, bias=bias, offset_mask=offset_mask)
+    half = _HALF.get(dt)
     ints = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group)
-    if bf16:
-        input, offset_mask = input.bfloat16(), offset_mask.bfloat16()
+    if half:
+        input, offset_mask = input.to(dt), offset_mask.to(dt)
         weight, bias = weight.float(), bias.float()
     g, ho, wo = _geom(input, weight, *ints)
     _check_packed(g, ho, wo, offset_mask)
@@ -252,10 +265,10 @@ def dcn_v2_forward_packed(input, weight, bias, offset_mask, kernel_h, kernel_w, 
         ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
         args = (L.stream_ptr(input.device), g, L.ptr(input), L.ptr(weight), L.ptr(bias), L.ptr(offset_mask),
                 L.ptr(output), L.ptr(abs_offset_sum) if abs_offset_sum is not None else None, L.ptr(ws), nbytes)
-        if not bf16:
+        if not half:
             L.check(lib.ebfi_dcnv2_forward_packed(*args), "dcn_v2_forward_packed")
-        elif not _native_bf16(lib.ebfi_dcnv2_forward_packed_bf16(*args), "dcn_v2_forward_packed_bf16"):
-            return _bf16_via_fp32(dcn_v2_forward_packed, (input, weight, bias, offset_mask), ints + (abs_offset_sum,))
+        elif not _ran_native(getattr(lib, "ebfi_dcnv2_forward_packed" + half)(*args), "dcn_v2_forward_packed" + half):
+            return _via_fp32(dt, dcn_v2_forward_packed, (input, weight, bias, offset_mask), ints + (abs_offset_sum,))
         _remember_blocked(lib, g, input, ws)
     return output
 
@@ -268,11 +281,11 @@ def dcn_v2_backward_packed(input, weight, bias, offset_mask, grad_output, kernel
         raise RuntimeError("input tensor has to be contiguous")
     if not weight.is_contiguous():
         raise RuntimeError("weight tensor has to be contiguous")
-    bf16 = _check_cuda(input=input, weight=weight, bias=bias, offset_mask=offset_mask,
-                       grad_output=grad_output) == torch.bfloat16
+    dt = _check_cuda(input=input, weight=weight, bias=bias, offset_mask=offset_mask, grad_output=grad_output)
+    half = _HALF.get(dt)
     ints = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group)
-    if bf16:
-        input, offset_mask, grad_output = (t.bfloat16() for t in (input, offset_mask, grad_output))
+    if half:
+        input, offset_mask, grad_output = (t.to(dt) for t in (input, offset_mask, grad_output))
         param_dtypes = [weight.dtype, bias.dtype]
         weight, bias = weight.float(), bias.float()
     g, ho, wo = _geom(input, weight, *ints, _deterministic())
@@ -288,13 +301,13 @@ def dcn_v2_backward_packed(input, weight, bias, offset_mask, grad_output, kernel
         in_ptr = _blocked_input_ptr(g, input)
         args = (L.stream_ptr(input.device), g, in_ptr, L.ptr(weight), L.ptr(bias), L.ptr(offset_mask),
                 L.ptr(grad_output), *(L.ptr(t) for t in grads), L.ptr(ws), nbytes)
-        if not bf16:
+        if not half:
             L.check(lib.ebfi_dcnv2_backward_packed(*args), "dcn_v2_backward_packed")
             return grads
-        ran = _native_bf16(lib.ebfi_dcnv2_backward_packed_bf16(*args), "dcn_v2_backward_packed_bf16")
-    out_dtypes = [torch.bfloat16] * 2 + param_dtypes
+        ran = _ran_native(getattr(lib, "ebfi_dcnv2_backward_packed" + half)(*args), "dcn_v2_backward_packed" + half)
+    out_dtypes = [dt] * 2 + param_dtypes
     if not ran:
-        return _bf16_via_fp32(dcn_v2_backward_packed, (input, weight, bias, offset_mask, grad_output), ints, out_dtypes)
+        return _via_fp32(dt, dcn_v2_backward_packed, (input, weight, bias, offset_mask, grad_output), ints, out_dtypes)
     return [t.to(dt) for t, dt in zip(grads, out_dtypes)]
 
 

@@ -17,11 +17,15 @@ except ImportError:  # shims directory used stand-alone on sys.path
     from ebfi_be_b200 import _lib as L
 
 
+# dtype -> suffix of the C entries (bf16 / fp16: storage only, fp32 arithmetic)
+_SUFFIX = {torch.float32: "", torch.bfloat16: "_bf16", torch.float16: "_fp16"}
+
+
 def _dims(input, kernel, kernel_size, what):
     L.require_cuda(input, kernel)
-    if input.dtype not in (torch.float32, torch.bfloat16) or kernel.dtype != input.dtype:
-        raise RuntimeError(f"{what}: input and kernel must both be float32 (the reference's dtype) or both "
-                           f"bfloat16, got {input.dtype} / {kernel.dtype}")
+    if input.dtype not in _SUFFIX or kernel.dtype != input.dtype:
+        raise RuntimeError(f"{what}: input and kernel must both be float32 (the reference's dtype), both "
+                           f"bfloat16 or both float16, got {input.dtype} / {kernel.dtype}")
     if input.dim() != 4 or kernel.dim() != 4:
         raise RuntimeError(f"{what}: input and kernel must be 4-D")
     B, C, Hi, Wi = input.shape
@@ -40,7 +44,7 @@ def forward(input, kernel, kernel_size, output):
     if tuple(output.shape) != (B, C, H, W) or not output.is_contiguous() or output.dtype != input.dtype:
         raise RuntimeError("kernelconv2d_cuda.forward: output must be a contiguous (B, C, H, W) tensor of the input dtype")
     lib = L.load()
-    fn = lib.ebfi_fac_forward if input.dtype == torch.float32 else lib.ebfi_fac_forward_bf16
+    fn = getattr(lib, "ebfi_fac_forward" + _SUFFIX[input.dtype])
     with torch.cuda.device(input.device):
         L.check(fn(L.stream_ptr(input.device), L.ptr(input), L.ptr(kernel), L.ptr(output), B, C, H, W, K), "CUDA call")
     return 1
@@ -60,7 +64,7 @@ def backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel):
     with torch.cuda.device(input.device):
         nbytes = lib.ebfi_fac_backward_workspace_bytes(B, C, H, W, K)
         ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
-        fn = lib.ebfi_fac_backward if input.dtype == torch.float32 else lib.ebfi_fac_backward_bf16
+        fn = getattr(lib, "ebfi_fac_backward" + _SUFFIX[input.dtype])
         L.check(fn(L.stream_ptr(input.device), L.ptr(input), L.ptr(kernel), L.ptr(grad_output), L.ptr(grad_input),
                    L.ptr(grad_kernel), B, C, H, W, K, L.ptr(ws), nbytes), "CUDA call")
     return 1

@@ -179,6 +179,33 @@ int ebfi_dcnv2_backward_packed_bf16(void *stream, const ebfi_dcn_geom *g,
                                     float *grad_weight, float *grad_bias,
                                     void *workspace, size_t workspace_bytes);
 
+/* fp16 activation variants (torch.autocast's default dtype): the *_bf16 entries above with `__half*` in place of
+ * `__nv_bfloat16*`, same arguments, workspaces, coverage and EBFI_ERR_UNSUPPORTED. On fp16-valued inputs every
+ * activation result equals the fp32 entry's result rounded once (RN) to fp16, and grad_weight / grad_bias are equal.
+ * An activation result beyond the fp16 range is +-inf, as a cast to fp16 gives; NaN stays NaN.
+ * ebfi_dcnv2_backward_dp_fp16 is declared with the data-parallel entries below. */
+int ebfi_dcnv2_forward_fp16(void *stream, const ebfi_dcn_geom *g,
+                            const void *input, const float *weight, const float *bias,
+                            const void *offset, const void *mask,
+                            void *output, void *workspace, size_t workspace_bytes);
+int ebfi_dcnv2_backward_fp16(void *stream, const ebfi_dcn_geom *g,
+                             const void *input, const float *weight, const float *bias,
+                             const void *offset, const void *mask,
+                             const void *grad_output,
+                             void *grad_input, void *grad_offset, void *grad_mask,
+                             float *grad_weight, float *grad_bias,
+                             void *workspace, size_t workspace_bytes);
+int ebfi_dcnv2_forward_packed_fp16(void *stream, const ebfi_dcn_geom *g,
+                                   const void *input, const float *weight, const float *bias,
+                                   const void *offset_mask, void *output, float *abs_offset_sum,
+                                   void *workspace, size_t workspace_bytes);
+int ebfi_dcnv2_backward_packed_fp16(void *stream, const ebfi_dcn_geom *g,
+                                    const void *input, const float *weight, const float *bias,
+                                    const void *offset_mask, const void *grad_output,
+                                    void *grad_input, void *grad_offset_mask,
+                                    float *grad_weight, float *grad_bias,
+                                    void *workspace, size_t workspace_bytes);
+
 /* ---- FAC KernelConv2D ------------------------------------------------------- */
 
 /* input  : (B, C, H+K-1, W+K-1)   already padded by the caller (KernelConv2D.py:82-86)
@@ -210,6 +237,15 @@ int ebfi_fac_backward(void *stream, const float *input, const float *kernel,
 int ebfi_fac_forward_bf16(void *stream, const void *input, const void *kernel, void *output,
                           int batch, int channels, int height_out, int width_out, int kernel_size);
 int ebfi_fac_backward_bf16(void *stream, const void *input, const void *kernel, const void *grad_output,
+                           void *grad_input, void *grad_kernel,
+                           int batch, int channels, int height_out, int width_out, int kernel_size,
+                           void *workspace, size_t workspace_bytes);
+
+/* fp16 storage variants: as the bf16 ones, with every tensor `__half*`. A result beyond the fp16 range is stored as
+ * +-inf, as a cast to fp16 gives; NaN stays NaN. */
+int ebfi_fac_forward_fp16(void *stream, const void *input, const void *kernel, void *output,
+                          int batch, int channels, int height_out, int width_out, int kernel_size);
+int ebfi_fac_backward_fp16(void *stream, const void *input, const void *kernel, const void *grad_output,
                            void *grad_input, void *grad_kernel,
                            int batch, int channels, int height_out, int width_out, int kernel_size,
                            void *workspace, size_t workspace_bytes);
@@ -262,6 +298,20 @@ int ebfi_kpn_fused_forward_bf16(void *stream, const void *event_feat, const void
                                 void *output, int batch, int channels_event, int channels_frame,
                                 int height, int width, int kernel_size, void *workspace, size_t workspace_bytes);
 int ebfi_kpn_fused_backward_bf16(void *stream, const void *event_feat, const void *frame_feat,
+                                 const float *conv_weight, const float *conv_bias, float negative_slope,
+                                 const void *grad_output, void *grad_pre, float *grad_event_fac, float *grad_bias,
+                                 int batch, int channels_event, int channels_frame, int height, int width,
+                                 int kernel_size, void *workspace, size_t workspace_bytes);
+
+/* fp16 activation variants: the two *_bf16 entries above with `__half*` in place of `__nv_bfloat16*`, same arguments
+ * and workspaces. The conv operands are rounded to bf16 as in the fp32 and bf16 entries, so on fp16-valued inputs
+ * output and grad_pre equal the fp32 entries' results rounded once to fp16 (+-inf beyond the fp16 range), and
+ * grad_event_fac and grad_bias are equal. */
+int ebfi_kpn_fused_forward_fp16(void *stream, const void *event_feat, const void *frame_feat,
+                                const float *conv_weight, const float *conv_bias, float negative_slope,
+                                void *output, int batch, int channels_event, int channels_frame,
+                                int height, int width, int kernel_size, void *workspace, size_t workspace_bytes);
+int ebfi_kpn_fused_backward_fp16(void *stream, const void *event_feat, const void *frame_feat,
                                  const float *conv_weight, const float *conv_bias, float negative_slope,
                                  const void *grad_output, void *grad_pre, float *grad_event_fac, float *grad_bias,
                                  int batch, int channels_event, int channels_frame, int height, int width,
@@ -396,6 +446,13 @@ int ebfi_dcnv2_backward_dp(void *stream, const ebfi_dcn_geom *g,
 /* The same with bf16 activations, as ebfi_dcnv2_backward_bf16 (EBFI_ERR_UNSUPPORTED: take ebfi_dcnv2_backward_dp on
  * widened copies). grad_weight / grad_bias are fp32, exchanged exactly as above. */
 int ebfi_dcnv2_backward_dp_bf16(void *stream, const ebfi_dcn_geom *g,
+                                const void *input, const float *weight, const float *bias,
+                                const void *offset, const void *mask, const void *grad_output,
+                                void *grad_input, void *grad_offset, void *grad_mask,
+                                float *grad_weight, float *grad_bias,
+                                void *workspace, size_t workspace_bytes, const ebfi_dp_comm *comm, int defer);
+/* The same with fp16 activations, as ebfi_dcnv2_backward_fp16. */
+int ebfi_dcnv2_backward_dp_fp16(void *stream, const ebfi_dcn_geom *g,
                                 const void *input, const float *weight, const float *bias,
                                 const void *offset, const void *mask, const void *grad_output,
                                 void *grad_input, void *grad_offset, void *grad_mask,

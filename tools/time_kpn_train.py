@@ -8,12 +8,12 @@ channels, 256x256, K=5) and the cfg5 block shape (B=8, 128x128). Prints one JSON
   *_peak_mb         torch.cuda.max_memory_allocated over forward + backward, above what was allocated before
 and the device name and power limit read in the same run.
 
---bf16 times the same two workloads in mixed precision: bf16 event / frame tensors and fp32 parameters under
-torch.autocast(dtype=torch.bfloat16), the autocast op sequence (bf16 cuDNN conv, bf16 LeakyReLU and FAC) against
-fused_backward=True (KernelConvFACBF16Function: bf16 fused kernels + bf16 cuDNN dgrad/wgrad of the bf16 grad_pre);
-the reference_* keys then hold the autocast sequence.
+--dtype bf16 / fp16 times the same two workloads in mixed precision: 16-bit event / frame tensors and fp32
+parameters under torch.autocast with that dtype, the autocast op sequence (16-bit cuDNN conv, LeakyReLU and FAC)
+against fused_backward=True (KernelConvFACBF16Function: 16-bit fused kernels + 16-bit cuDNN dgrad/wgrad of the 16-bit
+grad_pre); the reference_* keys then hold the autocast sequence. --bf16 is short for --dtype bf16.
 
-    python tools/time_kpn_train.py [--reps 15] [--bf16]
+    python tools/time_kpn_train.py [--reps 15] [--dtype fp32|bf16|fp16]
 """
 import argparse
 import contextlib
@@ -38,8 +38,12 @@ def device_info():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=15)
-    ap.add_argument("--bf16", action="store_true", help="bf16 activations under torch.autocast (mixed precision)")
+    ap.add_argument("--dtype", choices=("fp32", "bf16", "fp16"), default="fp32",
+                    help="activation dtype; bf16 / fp16 run under torch.autocast (mixed precision)")
+    ap.add_argument("--bf16", action="store_true", help="same as --dtype bf16")
     args = ap.parse_args()
+    if args.bf16:
+        args.dtype = "bf16"
     if not torch.cuda.is_available():
         raise SystemExit("time_kpn_train.py needs a CUDA device")
     dev = torch.device("cuda:0")
@@ -59,8 +63,9 @@ def main():
         return ts[len(ts) // 2]
 
     info = device_info()
-    act = torch.bfloat16 if args.bf16 else torch.float32
-    amp = (lambda: torch.autocast("cuda", dtype=torch.bfloat16)) if args.bf16 else contextlib.nullcontext
+    act = {"fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}[args.dtype]
+    half = act != torch.float32
+    amp = (lambda: torch.autocast("cuda", dtype=act)) if half else contextlib.nullcontext
     for (B, H, W) in [(4, 256, 256), (8, 128, 128)]:
         C, K = 64, 5
         torch.manual_seed(0)
@@ -97,11 +102,11 @@ def main():
             peak[fused] = (torch.cuda.max_memory_allocated() - base) / 2 ** 20
 
         # backward pieces of the fused path, each alone
-        # (bf16: the calls KernelConvFACBF16Function makes — bf16 activations, fp32 weights for the fused kernels,
-        # bf16 weights for cuDNN's convolution backward)
+        # (16-bit: the calls KernelConvFACBF16Function makes — 16-bit activations, fp32 weights for the fused kernels,
+        # 16-bit weights for cuDNN's convolution backward)
         evd, frd, w, b = ev.detach(), fr.detach(), conv.weight.detach(), conv.bias.detach()
         x, wc = torch.cat([evd, frd], 1), w.to(act)
-        fused_bwd = modification.kernelconv_fac_fused_backward_bf16 if args.bf16 else \
+        fused_bwd = modification.kernelconv_fac_fused_backward_bf16 if half else \
             modification.kernelconv_fac_fused_backward
         gpre = fused_bwd(evd, frd, w, b, K, 0.01, G)[0]
         pieces = {
@@ -128,7 +133,7 @@ def main():
         del gpre, x
 
         res = {"workload": f"B={B} Ce=Cf={C} K={K} {H}x{W}",
-               "precision": "bf16 activations, fp32 parameters, autocast" if args.bf16 else "fp32",
+               "precision": f"{args.dtype} activations, fp32 parameters, autocast" if half else "fp32",
                "reference_fwd_bwd_ms": round(median(ts[False]), 4), "fused_fwd_bwd_ms": round(median(ts[True]), 4),
                "bwd_breakdown_ms": breakdown, "kpn_kernels_ms": kernels,
                "reference_peak_mb": round(peak[False], 1), "fused_peak_mb": round(peak[True], 1),
