@@ -15,6 +15,7 @@ import kpn_train_oracle as KO
 import test_kpn_train_gpu as TG
 from conftest import rel_err
 from test_dcn_bf16_gpu import FALLBACKS, TC_SHAPES, _box_path, _forward, _fwd_bwd, _module, _rel_l2
+from test_kpn_gpu import PIPELINE_SHAPES as KPN_PIPELINE_SHAPES
 from test_kpn_gpu import SHAPES as KPN_SHAPES
 from test_kpn_gpu import _case as _kpn_case
 
@@ -126,7 +127,7 @@ def test_fac_row_segments_round_the_seam_rows_twice():
     assert float((gi - want[1]).abs().max()) <= 2.0 ** -10 * float(want[1].abs().max())
 
 
-@pytest.mark.parametrize("shape", KPN_SHAPES)
+@pytest.mark.parametrize("shape", KPN_SHAPES + KPN_PIPELINE_SHAPES)
 def test_kpn_bit_identical_to_fp32_kernels(mod, shape):
     from gpu_util import t
     B, Ce, Cf, H, W, K = shape

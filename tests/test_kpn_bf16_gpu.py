@@ -11,7 +11,7 @@ import kpn_train_oracle as KO
 import test_kpn_train_gpu as TG
 from conftest import rel_err
 from oracle.oracle import _bf16_round
-from test_kpn_gpu import SHAPES, _case
+from test_kpn_gpu import PIPELINE_SHAPES, SHAPES, _case
 
 pytestmark = pytest.mark.gpu
 
@@ -29,7 +29,7 @@ def _autocast():
     return torch.autocast("cuda", dtype=BF16)
 
 
-@pytest.mark.parametrize("shape", SHAPES)
+@pytest.mark.parametrize("shape", SHAPES + PIPELINE_SHAPES)
 def test_forward_bit_identical_to_fp32_kernel(mod, shape):
     from gpu_util import t
     B, Ce, Cf, H, W, K = shape
@@ -46,7 +46,7 @@ def test_forward_bit_identical_to_fp32_kernel(mod, shape):
         assert torch.equal(pub, mod._fused_forward(evb.float(), frb.float(), wb.float(), bb.float(), K, SLOPE).to(BF16))
 
 
-@pytest.mark.parametrize("shape", SHAPES)
+@pytest.mark.parametrize("shape", SHAPES + PIPELINE_SHAPES)
 def test_backward_bit_identical_to_fp32_kernel(mod, shape):
     from gpu_util import t
     B, Ce, Cf, H, W, K = shape

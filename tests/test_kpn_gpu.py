@@ -32,8 +32,52 @@ SHAPES = [(1, 64, 64, 16, 8, 5),      # exactly one tile
           (1, 16, 16, 20, 20, 5),     # 32 input channels; last slice has a single channel
           (1, 64, 0, 18, 10, 1)]      # no frame features, 1x1 FAC
 
+# Shapes at which a CTA of the persistent kernel walks several items: its accumulator and halo-part barrier phases
+# wrap, parts are refilled while others compute, its range crosses weight slices and samples. Comments give Cin / 32
+# halo parts, channels in the last weight slice and items per CTA at 148 SMs (kpn_work_split; the coverage is
+# asserted at the device's SM count in test_kpn_pipeline_gpu.py).
+PIPELINE_SHAPES = [(2, 48, 48, 21, 33, 5),    # 3 parts, last slice full, 3 items per CTA, crosses slice and sample
+                   (3, 96, 0, 33, 20, 3),     # 3 parts, K = 3, 6 items, no frame features
+                   (2, 32, 64, 29, 43, 1),    # 3 parts, K = 1
+                   (2, 64, 32, 64, 64, 5),    # 3 parts, 10 items
+                   (2, 33, 31, 40, 40, 5),    # odd Ce: an 8-channel input chunk mixes event and frame channels
+                   (1, 128, 0, 17, 9, 5),     # 4 parts, no frame features, H % 16 = 1
+                   (2, 64, 64, 17, 25, 1),    # 4 parts, K = 1, W % 8 = 1
+                   (2, 64, 64, 17, 29, 5),    # 4 parts, 3 items, crosses slice and sample
+                   (2, 16, 16, 49, 49, 5),    # 1 part, 3 items
+                   (2, 32, 32, 80, 56, 3),    # 2 parts, 6 items
+                   (3, 32, 32, 3, 70, 5),     # H < K: a window reaches past both image borders
+                   (4, 16, 16, 7, 5, 3),      # W < 8, H < 16: a single partial tile per sample
+                   (2, 32, 0, 1, 1, 5),       # H = W = 1: the whole replication pad folds onto one pixel
+                   (5, 64, 64, 2, 2, 5),      # 4 parts, 2 x 2 images
+                   (2, 96, 32, 36, 50, 3)]    # 4 parts, last slice full, 10 items
 
-@pytest.mark.parametrize("shape", SHAPES)
+
+def kpn_work_split(shape, sms, backward=False):
+    """The work split of csrc/kpn.cu (`fill` and the launch arithmetic of kpn_forward / kpn_backward) for
+    shape = (B, Ce, Cf, H, W, K) on `sms` SMs. Items are (weight slice of 3 FAC channels, 16 x 8 pixel tile) in
+    slice-major order, tiles in (sample, tile row, tile column) order; CTA k walks items [k * per, (k + 1) * per).
+    Returns npart (halo parts = Cin / 32), last (FAC channels in the last slice), tiles_x, tiles_y, ntile (tiles per
+    slice), nslice, per, ctas, crosses_slice / crosses_sample (some CTA's range holds items of two slices / two
+    samples)."""
+    B, Ce, Cf, H, W, K = shape
+    nslice = -(-Ce // 3)
+    tiles_x, tiles_y = -(-W // 8), -(-H // 16)
+    tiles_per_sample = tiles_x * tiles_y
+    ntile = B * tiles_per_sample
+    total = nslice * ntile
+    grid = min(total, sms, 1024) if backward else min(total, sms)      # 1024: BWD_MAX_GRID
+    per = -(-total // grid)
+    ctas = -(-total // per)
+    first = np.arange(ctas) * per
+    last = np.minimum(first + per, total) - 1
+    return dict(npart=(Ce + Cf) // 32, last=Ce - 3 * (nslice - 1), tiles_x=tiles_x, tiles_y=tiles_y, ntile=ntile,
+                nslice=nslice, per=per, ctas=ctas,
+                crosses_slice=bool((first // ntile != last // ntile).any()),
+                crosses_sample=B > 1 and bool((first // tiles_per_sample != last // tiles_per_sample).any()))
+
+
+@pytest.mark.parametrize("shape", SHAPES + PIPELINE_SHAPES)
 def test_fused_against_oracle(mod, oracle, shape):
     from gpu_util import n, t
     B, Ce, Cf, H, W, K = shape
