@@ -70,6 +70,12 @@ SIGNATURES = {
     "ebfi_fac_backward_bf16": (c_int, [c_void] * 6 + [c_int] * 5 + [c_void, c_size]),
     "ebfi_fac_forward_fp16": (c_int, [c_void] * 4 + [c_int] * 5),
     "ebfi_fac_backward_fp16": (c_int, [c_void] * 6 + [c_int] * 5 + [c_void, c_size]),
+    "ebfi_fac_replpad_forward": (c_int, [c_void] * 4 + [c_int] * 5),
+    "ebfi_fac_replpad_backward": (c_int, [c_void] * 6 + [c_int] * 5 + [c_void, c_size]),
+    "ebfi_fac_replpad_forward_bf16": (c_int, [c_void] * 4 + [c_int] * 5),
+    "ebfi_fac_replpad_backward_bf16": (c_int, [c_void] * 6 + [c_int] * 5 + [c_void, c_size]),
+    "ebfi_fac_replpad_forward_fp16": (c_int, [c_void] * 4 + [c_int] * 5),
+    "ebfi_fac_replpad_backward_fp16": (c_int, [c_void] * 6 + [c_int] * 5 + [c_void, c_size]),
     "ebfi_kpn_fused_workspace_bytes": (c_size, [c_int] * 6),
     "ebfi_kpn_fused_forward": (c_int, [c_void] * 5 + [ctypes.c_float, c_void] + [c_int] * 6 + [c_void, c_size]),
     "ebfi_kpn_fused_backward_workspace_bytes": (c_size, [c_int] * 6),

@@ -250,6 +250,32 @@ int ebfi_fac_backward_fp16(void *stream, const void *input, const void *kernel, 
                            int batch, int channels, int height_out, int width_out, int kernel_size,
                            void *workspace, size_t workspace_bytes);
 
+/* ReplicationPad2d((K-1)/2) followed by FAC as one op (the KernelConv2D module, KernelConv2D.py:77-87): the
+ * arguments of the entries above, except that input and grad_input are the unpadded (B, C, H, W) tensors.
+ * The pad is folded into the kernels, so no padded copy is written or read. The forward and grad_kernel are
+ * bit-identical to the padded entries on the replication-padded input. grad_input sums the padded cells each
+ * input element is replicated to in a fixed order in fp32 (no atomics) and rounds 16-bit results once; an
+ * element outside the first and last row and column is bit-identical to its padded counterpart. The backward
+ * takes exactly ebfi_fac_backward_workspace_bytes(B, C, H, W, K) bytes of workspace. K = 1 is the plain op. */
+int ebfi_fac_replpad_forward(void *stream, const float *input, const float *kernel, float *output,
+                             int batch, int channels, int height_out, int width_out, int kernel_size);
+int ebfi_fac_replpad_backward(void *stream, const float *input, const float *kernel,
+                              const float *grad_output, float *grad_input, float *grad_kernel,
+                              int batch, int channels, int height_out, int width_out, int kernel_size,
+                              void *workspace, size_t workspace_bytes);
+int ebfi_fac_replpad_forward_bf16(void *stream, const void *input, const void *kernel, void *output,
+                                  int batch, int channels, int height_out, int width_out, int kernel_size);
+int ebfi_fac_replpad_backward_bf16(void *stream, const void *input, const void *kernel, const void *grad_output,
+                                   void *grad_input, void *grad_kernel,
+                                   int batch, int channels, int height_out, int width_out, int kernel_size,
+                                   void *workspace, size_t workspace_bytes);
+int ebfi_fac_replpad_forward_fp16(void *stream, const void *input, const void *kernel, void *output,
+                                  int batch, int channels, int height_out, int width_out, int kernel_size);
+int ebfi_fac_replpad_backward_fp16(void *stream, const void *input, const void *kernel, const void *grad_output,
+                                   void *grad_input, void *grad_kernel,
+                                   int batch, int channels, int height_out, int width_out, int kernel_size,
+                                   void *workspace, size_t workspace_bytes);
+
 /* ---- KernelConv producer -> FAC fusion (forward; SURVEY 8f rank 1) ------------- */
 
 /* models/Ours/model_singleframe.py:145-146,159-162 (class Modification) as ONE op:
