@@ -480,6 +480,8 @@ size_t ebfi_dcnv2_blocked_input_offset(const ebfi_dcn_geom *q)
     DcnDims d{};
     if (fill_dims(q, d) != EBFI_OK) return 0;
     d.det = 0;
+    const char *impl = getenv("EBFI_DCN_IMPL");
+    if (impl && impl[0] == 's') return 0;                // the CUDA-core kernels run: no copy is made or read
     if (backward_box_splits(d) == 0) return 0;           // the backward could not use it
     return forward_tc_blocked_offset(d);
 }

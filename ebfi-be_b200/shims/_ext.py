@@ -61,12 +61,14 @@ def _remember_blocked(lib, g, input, ws):
                                               input.untyped_storage())
 
 
-def _blocked_input_ptr(g, input):
-    """Before a backward: the forward's blocked copy of this very tensor if it is still alive (sets the geometry flag),
-    else the tensor itself."""
+def _blocked_input_ptr(g, input, grad_output):
+    """Before a backward: the forward's blocked copy of this very tensor if it is still alive and this backward runs the
+    box kernel that reads it (sets the geometry flag), else the tensor itself. The box kernel needs a 16-byte aligned
+    grad_output and no EBFI_DCN_IMPL=simt, which may have changed since the forward."""
     hit = _blocked_cache.get(input.device.index)
     if (hit is not None and not g.flags and hit[0] == _blocked_key(input, g)
-            and hit[3] == torch.cuda.current_stream(input.device)):
+            and hit[3] == torch.cuda.current_stream(input.device) and grad_output.data_ptr() % 16 == 0
+            and L.load().ebfi_dcnv2_blocked_input_offset(g) == hit[2]):
         g.flags |= L.EBFI_DCN_INPUT_BLOCKED
         return L.c_void(hit[1].data_ptr() + hit[2])
     return L.ptr(input)
@@ -205,7 +207,7 @@ def dcn_v2_backward(input, weight, bias, offset, mask, grad_output, kernel_h, ke
         grads = [torch.empty_like(t) for t in (input, offset, mask, weight, bias)]
         nbytes = lib.ebfi_dcnv2_backward_workspace_bytes(g)
         ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
-        in_ptr = _blocked_input_ptr(g, input)
+        in_ptr = _blocked_input_ptr(g, input, grad_output)
         args = (L.stream_ptr(input.device), g, in_ptr, L.ptr(weight), L.ptr(bias), L.ptr(offset), L.ptr(mask),
                 L.ptr(grad_output), *(L.ptr(t) for t in grads), L.ptr(ws), nbytes)
         if not half:
@@ -298,7 +300,7 @@ def dcn_v2_backward_packed(input, weight, bias, offset_mask, grad_output, kernel
         grads = [torch.empty_like(t) for t in (input, offset_mask, weight, bias)]
         nbytes = lib.ebfi_dcnv2_backward_workspace_bytes(g)
         ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
-        in_ptr = _blocked_input_ptr(g, input)
+        in_ptr = _blocked_input_ptr(g, input, grad_output)
         args = (L.stream_ptr(input.device), g, in_ptr, L.ptr(weight), L.ptr(bias), L.ptr(offset_mask),
                 L.ptr(grad_output), *(L.ptr(t) for t in grads), L.ptr(ws), nbytes)
         if not half:

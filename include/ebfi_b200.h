@@ -100,7 +100,8 @@ size_t ebfi_dcnv2_backward_workspace_bytes(const ebfi_dcn_geom *g);
 size_t ebfi_dcnv2_forward_workspace_bytes(const ebfi_dcn_geom *g);
 
 /* Byte offset of the group-blocked input copy inside the forward workspace after ebfi_dcnv2_forward, or 0 when this
- * geometry does not produce / the backward cannot consume one (see EBFI_DCN_INPUT_BLOCKED). */
+ * geometry does not produce / the backward cannot consume one, or EBFI_DCN_IMPL=simt is set in the environment (the
+ * CUDA-core kernels neither write nor read it) (see EBFI_DCN_INPUT_BLOCKED). */
 size_t ebfi_dcnv2_blocked_input_offset(const ebfi_dcn_geom *g);
 
 /* out[b,co,h,w] = bias[co] + sum_{c,i,j} weight[co,c,i,j] * mask * bilinear(input[b,c], ...)

@@ -250,6 +250,37 @@ def test_backward_reuses_the_forwards_blocked_input(dcn, monkeypatch):
         assert torch.equal(a, c)
 
 
+def test_blocked_copy_only_goes_to_the_box_backward(monkeypatch):
+    """The CUDA-core kernels (EBFI_DCN_IMPL=simt, for the forward and backward or only for the backward) and a grad_output
+    that is not 16-byte aligned run backwards that read the NCHW input: they get it, not a forward's blocked copy, and
+    give the results of the same backward on a tensor no forward has seen (grad_input to the order of its float atomics)."""
+    from gpu_util import dev
+    from ebfi_be_b200.shims import _ext
+    torch.manual_seed(10)
+    B, C, H, W, dg = 2, 64, 24, 40, 8
+    x = torch.randn(B, C, H, W, device=dev())
+    off = 2 * torch.randn(B, 2 * dg * 9, H, W, device=dev())
+    msk = torch.sigmoid(torch.randn(B, dg * 9, H, W, device=dev()))
+    w = torch.randn(64, C, 3, 3, device=dev()) / 24
+    b = torch.randn(64, device=dev())
+    go = torch.randn(B, 64, H, W, device=dev())
+    go_mis = torch.empty(go.numel() + 1, device=dev())[1:].view(go.shape).copy_(go)
+    geom = (3, 3, 1, 1, 1, 1, 1, 1, dg)
+    for fwd_env, bwd_env, g in ((None, None, go_mis), ("simt", "simt", go), (None, "simt", go)):
+        for name, env in (("fwd", fwd_env), ("bwd", bwd_env)):
+            if env:
+                monkeypatch.setenv("EBFI_DCN_IMPL", env)
+            else:
+                monkeypatch.delenv("EBFI_DCN_IMPL", raising=False)
+            if name == "fwd":
+                _ext.dcn_v2_forward(x, w, b, off, msk, *geom)
+        want = _ext.dcn_v2_backward(x.clone(), w, b, off, msk, g, *geom)
+        got = _ext.dcn_v2_backward(x, w, b, off, msk, g, *geom)
+        assert rel_err(got[0].cpu().numpy(), want[0].cpu().numpy()) < 1e-6, (fwd_env, bwd_env)
+        for a, c in zip(got[1:], want[1:]):
+            assert torch.equal(a, c), (fwd_env, bwd_env)
+
+
 def test_reductions_are_bit_reproducible(dcn):
     """grad_offset / grad_mask / grad_weight / grad_bias use fixed-order reductions."""
     from gpu_util import dev
