@@ -356,15 +356,22 @@ __global__ void dcn_reduce_partials(const float *__restrict__ gw_part, const flo
 }
 
 // ---- deterministic mode (EBFI_DCN_DETERMINISTIC): bound of a single grad_input contribution ----
+// max that keeps a NaN (fmaxf drops it): a NaN in grad_output, weight or mask makes the bound NaN, hence non-finite
+__device__ __forceinline__ float max_nan(float a, float b) { return (b > a || b != b) ? b : a; }
+
 __device__ __forceinline__ void atomic_max_nonneg(float *dst, float v)
 {
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<int *>(dst), __float_as_int(v));   // v >= 0: int order == float order
+    for (int o = 16; o > 0; o >>= 1) v = max_nan(v, __shfl_xor_sync(0xffffffffu, v, o));
+    // v >= 0 or a positive NaN: int order == float order, and a NaN's bits exceed every other value's
+    if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<int *>(dst), __float_as_int(v));
 }
 
-__global__ void dcn_det_bound(const float *__restrict__ gout, const float *__restrict__ weight,
-                              const float *__restrict__ mask, float *__restrict__ bound, DcnDims d)
+// T = the activation type of grad_output and mask, read as T and widened exactly: a 16-bit call gets the bound of the
+// fp32 call on the widened values, hence the same fixed-point scale
+template <typename T>
+__global__ void dcn_det_bound(const T *__restrict__ gout, const float *__restrict__ weight,
+                              const T *__restrict__ mask, float *__restrict__ bound, DcnDims d)
 {
     const size_t plane = (size_t)d.Ho * d.Wo, tid = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
     const size_t nthr = (size_t)gridDim.x * blockDim.x;
@@ -372,12 +379,12 @@ __global__ void dcn_det_bound(const float *__restrict__ gout, const float *__res
     for (size_t i = tid; i < (size_t)d.B * plane; i += nthr) {      // max over pixels of sum_co |gO|
         const size_t b = i / plane, pix = i - b * plane;
         float a = 0.f;
-        for (int co = 0; co < d.Co; ++co) a += fabsf(__ldg(gout + (b * d.Co + co) * plane + pix));
-        m0 = fmaxf(m0, a);
+        for (int co = 0; co < d.Co; ++co) a += fabsf(ld_act(gout + (b * d.Co + co) * plane + pix));
+        m0 = max_nan(m0, a);
     }
-    for (size_t i = tid; i < (size_t)d.Co * d.C * d.KK; i += nthr) m1 = fmaxf(m1, fabsf(__ldg(weight + i)));
+    for (size_t i = tid; i < (size_t)d.Co * d.C * d.KK; i += nthr) m1 = max_nan(m1, fabsf(__ldg(weight + i)));
     if (!d.packed)
-        for (size_t i = tid; i < (size_t)d.B * d.mask_bs; i += nthr) m2 = fmaxf(m2, fabsf(__ldg(mask + i)));
+        for (size_t i = tid; i < (size_t)d.B * d.mask_bs; i += nthr) m2 = max_nan(m2, fabsf(ld_act(mask + i)));
     atomic_max_nonneg(bound + 0, m0);
     atomic_max_nonneg(bound + 1, m1);
     atomic_max_nonneg(bound + 2, m2);
@@ -470,16 +477,16 @@ size_t ebfi_dcnv2_backward_workspace_bytes(const ebfi_dcn_geom *q)
     DcnDims d{};
     if (fill_dims(q, d) != EBFI_OK) return 0;
     const size_t S = (size_t)std::max({bwd_splits(d), backward_tc_splits(d), backward_box_splits(d)});
-    const size_t det = d.det ? 256 + (size_t)d.B * d.C * d.H * d.W * sizeof(long long) : 0;   // bound + CUDA-core int64 copy
+    const size_t det = d.det ? (size_t)d.B * d.C * d.H * d.W * sizeof(long long) : 0;   // CUDA-core int64 copy
+    const size_t bound = d.det ? 256 : 0;                                                  // 3-float bound, every path
     return ebfi::round_up(S * ((size_t)d.Co * d.C * d.KK + d.Co) * sizeof(float), (size_t)256) +
-           std::max({backward_tc_scratch_bytes(d), backward_box_scratch_bytes(d), det}) + 512;
+           std::max({backward_tc_scratch_bytes(d), backward_box_scratch_bytes(d), det}) + bound + 512;
 }
 
 size_t ebfi_dcnv2_blocked_input_offset(const ebfi_dcn_geom *q)
 {
     DcnDims d{};
     if (fill_dims(q, d) != EBFI_OK) return 0;
-    d.det = 0;
     const char *impl = getenv("EBFI_DCN_IMPL");
     if (impl && impl[0] == 's') return 0;                // the CUDA-core kernels run: no copy is made or read
     if (backward_box_splits(d) == 0) return 0;           // the backward could not use it
@@ -551,16 +558,17 @@ static int run_backward(void *stream, const DcnDims &d_in, const T *input, const
     // the tensor-core backward stages grad_output with 128-bit loads (8 pixels: two for fp32, one for bf16 / fp16, when a
     // row is a whole number of 16-byte words): it needs a 16-byte aligned base for either element size
     const bool tc_ok = !(impl && impl[0] == 's') && ebfi::aligned16(grad_output);
-    // box kernel (dcn_bwd_box.cu) first; the group-specialised kernel (dcn_bwd_tc.cu) serves the deterministic flag
+    // box kernel (dcn_bwd_box.cu) first, in both modes; the group-specialised kernel (dcn_bwd_tc.cu) takes cpg 8 /
+    // Cout 64 footprints beyond the box, the CUDA-core kernel everything else
     const int S_box = tc_ok ? backward_box_splits(d) : 0;
     if (!std::is_same_v<T, float> && S_box == 0)
-        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_backward_%s: no box backward for this call (shape, flags or alignment)",
+        return ebfi::fail(EBFI_ERR_UNSUPPORTED, "dcn_backward_%s: no box backward for this call (shape or alignment)",
                           act_name<T>());
     const int S_tc = S_box > 0 ? S_box : (tc_ok ? backward_tc_splits(d) : 0);
     const int S = S_tc > 0 ? S_tc : bwd_splits(d);
     if (d.in_blocked) {
-        EBFI_REQUIRE(S_box > 0, "dcn_backward: EBFI_DCN_INPUT_BLOCKED needs the box path (ebfi_dcnv2_blocked_input_offset() != 0 "
-                                "and no EBFI_DCN_DETERMINISTIC)");
+        EBFI_REQUIRE(S_box > 0, "dcn_backward: EBFI_DCN_INPUT_BLOCKED needs the box path (ebfi_dcnv2_blocked_input_offset() != 0, "
+                                "a 16-byte aligned grad_output, no EBFI_DCN_IMPL=simt)");
         EBFI_REQUIRE((reinterpret_cast<uintptr_t>(input) & 31u) == 0, "dcn_backward: the blocked input must be 32-byte aligned");
     }
     const size_t n_w = (size_t)d.Co * d.C * d.KK, n_b = (size_t)d.Co;
@@ -578,6 +586,14 @@ static int run_backward(void *stream, const DcnDims &d_in, const T *input, const
     float *gw_part = static_cast<float *>(workspace);
     float *gb_part = gw_part + (size_t)S * n_w;
     char *scratch = static_cast<char *>(workspace) + part_bytes;
+    if (d.det) {
+        // bound of a single grad_input contribution -> the int64 fixed-point scale (box path: far samples only)
+        float *bound = reinterpret_cast<float *>(scratch + scratch_bytes);
+        EBFI_CUDA_OK(cudaMemsetAsync(bound, 0, 3 * sizeof(float), st));
+        dcn_det_bound<T><<<ebfi::sm_count() * 4, 256, 0, st>>>(grad_output, weight, mask, bound, d);
+        EBFI_LAUNCH_OK("dcn_det_bound");
+        d.det_bound = bound;
+    }
     if (S_box > 0) {
         // writes all five gradients, including its own fixed-order reduction of the weight-gradient partials
         return backward_box<T>(st, d, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,
@@ -586,13 +602,6 @@ static int run_backward(void *stream, const DcnDims &d_in, const T *input, const
     if constexpr (!std::is_same_v<T, float>) {
         return EBFI_ERR_UNSUPPORTED;      // not reached: a 16-bit call without the box path returned above
     } else {
-        if (d.det) {
-            float *bound = reinterpret_cast<float *>(scratch + scratch_bytes);
-            EBFI_CUDA_OK(cudaMemsetAsync(bound, 0, 3 * sizeof(float), st));
-            dcn_det_bound<<<ebfi::sm_count() * 4, 256, 0, st>>>(grad_output, weight, mask, bound, d);
-            EBFI_LAUNCH_OK("dcn_det_bound");
-            d.det_bound = bound;
-        }
         if (S_tc > 0) {
             // tensor-core path (dcn_bwd_tc.cu): cpg == 8, Cout == 64
             if (int rc = backward_tc(st, d, input, weight, offset, mask, grad_output, grad_input, grad_offset, grad_mask,

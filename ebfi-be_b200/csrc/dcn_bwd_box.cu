@@ -29,7 +29,10 @@
 //     atomics, no order dependence: grad_input is bit-identical run to run, by default.
 //   * samples whose corners leave the box (|offset| beyond ~7 pixels) fall back to 256-bit global loads and
 //     red.global.add.v4.f32 into a blocked fp32 buffer that dcn_gin_collect adds last (order-dependent only then, like
-//     the reference's atomicAdd, im2col_cuda.cu:249).
+//     the reference's atomicAdd, im2col_cuda.cu:249). With EBFI_DCN_DETERMINISTIC (the DET instantiations) those samples
+//     instead add each product, rounded once to int64 fixed point (det_add, scale from dcn_det_bound), into a blocked
+//     int64 buffer that dcn_gin_collect converts to its starting value: every result is then bit-reproducible, and equal
+//     to the default mode's bits wherever no sample leaves its box (the int64 buffer is 0 -> +0.0f).
 // Non-finite gradients: a NaN/Inf anywhere in the (tile, group) makes the scale undefined; the box is then written as NaN
 // so that overflow checks on grad_input (AMP GradScaler) still fire.
 // Activation type T (float | __nv_bfloat16 | __half, the *_bf16 / *_fp16 entries): offsets, masks and grad_output are
@@ -109,6 +112,14 @@ __device__ __forceinline__ void red_add_v4(float *addr, float a, float b, float 
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(e) : "memory");
 }
 
+// det_add (dcn_common.cuh) as one asm statement: each conversion stays next to its reduction, so a far sample keeps
+// one 64-bit temporary live instead of eight
+__device__ __forceinline__ void red_add_fixed(long long *addr, float v_scaled)
+{
+    asm volatile("{\n\t.reg .s64 t;\n\tcvt.rni.s64.f32 t, %1;\n\tred.global.add.u64 [%0], t;\n\t}"
+                 ::"l"(addr), "f"(v_scaled) : "memory");
+}
+
 __device__ __forceinline__ void atoms_add(uint32_t saddr, int v)
 {
     asm volatile("red.shared.add.s32 [%0], %1;" ::"r"(saddr), "r"(v) : "memory");
@@ -145,10 +156,11 @@ struct SampleCtx {
     int ho, wo, by0, bx0, bxq0;
     uint32_t box_s, acc_s;
     const float *ib;     // blocked input plane of (sample, group): far-sample gathers
-    float *gb;           // blocked far-sample accumulator of (sample, group)
+    float *gb;           // blocked far-sample accumulator of (sample, group); DET: int64 elements
     float scale;
 };
-template <bool PACKED>
+__shared__ float s_det_scale;    // DET: fixed-point scale of the far-sample accumulator, set once per CTA
+template <bool PACKED, bool DET>
 __device__ __forceinline__ void sample_bwd(const DcnDims &d, const SampleCtx &sc, const float (&gc)[8], float dy, float dx, float m,
                                            int ti, int tj, int lane, uint32_t wrot, float (&colv)[8], float &g_y, float &g_x, float &g_m)
 {
@@ -276,19 +288,40 @@ __device__ __forceinline__ void sample_bwd(const DcnDims &d, const SampleCtx &sc
     } else if (q_inside) {
         const Tap tq = make_tap(y, xs, d.H, d.W);
         const float q1 = tq.hy * tq.hx, q2 = tq.hy * tq.lx, q3 = tq.ly * tq.hx, q4 = tq.ly * tq.lx;
+        if constexpr (DET) {
+            // the same products as below, each rounded once to the int64 fixed-point grid: order-independent sums.
+            // Corners in a rolled loop and the scale from shared memory: the far path adds no live registers.
+            long long *g64 = reinterpret_cast<long long *>(gb);
+#pragma unroll 1
+            for (int c = 0; c < 4; ++c) {
+                const bool ok = c == 0 ? tq.c00 : c == 1 ? tq.c01 : c == 2 ? tq.c10 : tq.c11;
+                if (!ok) continue;
+                const float qc = c == 0 ? q1 : c == 1 ? q2 : c == 2 ? q3 : q4;
+                long long *pc = g64 + (size_t)(tq.i00 + (c & 1) + (c >> 1) * d.W) * CS;
+                const float ds = s_det_scale;
 #pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-            const float *tt = (hf == (odd ? 1 : 0)) ? ta : tb;      // natural half hf
-            if (tq.c00) red_add_v4(gb + (size_t)tq.i00 * CS + 4 * hf, q1 * tt[0], q1 * tt[1], q1 * tt[2], q1 * tt[3]);
-            if (tq.c01) red_add_v4(gb + (size_t)tq.i01 * CS + 4 * hf, q2 * tt[0], q2 * tt[1], q2 * tt[2], q2 * tt[3]);
-            if (tq.c10) red_add_v4(gb + (size_t)tq.i10 * CS + 4 * hf, q3 * tt[0], q3 * tt[1], q3 * tt[2], q3 * tt[3]);
-            if (tq.c11) red_add_v4(gb + (size_t)tq.i11 * CS + 4 * hf, q4 * tt[0], q4 * tt[1], q4 * tt[2], q4 * tt[3]);
+                for (int hf = 0; hf < 2; ++hf) {
+                    const float *tt = (hf == (odd ? 1 : 0)) ? ta : tb;      // natural half hf
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) red_add_fixed(pc + 4 * hf + j, qc * tt[j] * ds);
+                }
+            }
+        } else {
+#pragma unroll
+            for (int hf = 0; hf < 2; ++hf) {
+                const float *tt = (hf == (odd ? 1 : 0)) ? ta : tb;      // natural half hf
+                if (tq.c00) red_add_v4(gb + (size_t)tq.i00 * CS + 4 * hf, q1 * tt[0], q1 * tt[1], q1 * tt[2], q1 * tt[3]);
+                if (tq.c01) red_add_v4(gb + (size_t)tq.i01 * CS + 4 * hf, q2 * tt[0], q2 * tt[1], q2 * tt[2], q2 * tt[3]);
+                if (tq.c10) red_add_v4(gb + (size_t)tq.i10 * CS + 4 * hf, q3 * tt[0], q3 * tt[1], q3 * tt[2], q3 * tt[3]);
+                if (tq.c11) red_add_v4(gb + (size_t)tq.i11 * CS + 4 * hf, q4 * tt[0], q4 * tt[1], q4 * tt[2], q4 * tt[3]);
+            }
         }
     }
 }
 
 // MULTI: more than one 8-channel unit per deformable group (the group's offset / mask gradients accumulate over its units)
-template <bool PACKED, bool MULTI, typename T>
+// DET (EBFI_DCN_DETERMINISTIC): `gin_blk` is the int64 fixed-point far-sample accumulator, scaled by d.det_bound
+template <bool PACKED, bool MULTI, bool DET, typename T>
 __global__ void __launch_bounds__(NTHR, 1)
 dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__restrict__ wimg,
                    const T *__restrict__ offset, const T *__restrict__ mask,
@@ -334,6 +367,7 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
         umma::mbar_fence_init();
         tile_max[0] = tile_max[1] = 0u;
         w_max[0] = w_max[1] = 0;
+        if constexpr (DET) s_det_scale = ldexpf(1.f, det_scale_exp(d));
     }
     for (int c = tid; c < BOX_F / 4; c += NTHR) acc4[c] = make_int4(0, 0, 0, 0);
     for (int c = tid; c < 2 * CNT_PAD / 4; c += NTHR) cnt[c] = 0;
@@ -632,7 +666,7 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
             sc.by0 = cur.ty0 * d.sh - d.ph - pl.my; sc.bx0 = cur.tx0 * d.sw - d.pw - pl.mx; sc.bxq0 = cur.tx0 * d.sw - d.ph - pl.mx;
             sc.box_s = umma::smem_u32(boxes + bb * box::BYTES); sc.acc_s = acc_s;
             sc.ib = in_blk + ((size_t)cur.b * pl.units + cur.g) * in_plane * CS;
-            sc.gb = gin_blk + ((size_t)cur.b * pl.units + cur.g) * in_plane * CS;
+            sc.gb = gin_blk + ((size_t)cur.b * pl.units + cur.g) * in_plane * CS * (DET ? 2 : 1);
             sc.scale = ldexpf(1.f, k2);
             const T *om = oms + bb * (pl.om_bytes / (int)sizeof(T));
             const T *off_g = offset + (size_t)cur.b * d.off_bs + (size_t)(MULTI ? cur.g >> pl.ncs_shift : cur.g) * 2 * d.KK * plane;
@@ -666,7 +700,7 @@ dcn_bwd_box_kernel(const float *__restrict__ in_blk, const unsigned char *__rest
                         tap_read(off_g, mask_g, uplane, (unsigned)t, (unsigned)cur.pix, dy, dx, m);
                     }
                     float g_y, g_x, g_m;
-                    sample_bwd<PACKED>(d, sc, gc, dy, dx, m, ti, tj, lane, wrot, colv, g_y, g_x, g_m);
+                    sample_bwd<PACKED, DET>(d, sc, gc, dy, dx, m, ti, tj, lane, wrot, colv, g_y, g_x, g_m);
                     // more than 8 channels per deformable group: the group's units follow each other in this CTA and the
                     // same thread owns the element in each of them -> plain read-modify-write, fixed order
                     T *gy = goff_g + (2u * (unsigned)t * uplane + (unsigned)cur.pix);
@@ -824,19 +858,31 @@ __global__ void dcn_bwd_prep_weights(const float *__restrict__ weight, unsigned 
 
 // grad_input[b][g*8 + c][y][x] = sum, in a fixed order, over the boxes that cover (y, x) + the far-sample buffer.
 // One thread per (b, g, y, x): 32 contiguous bytes per box, coalesced along x; NCHW plane stores.
-template <typename T>
+// DET: the far-sample buffer holds int64 fixed point (64 bytes per pixel); its value converted by one rounding, or NaN
+// when the bound is not finite, is the starting value. Without far samples that is +0.0f, as in the float buffer, so
+// both modes then give the same bits.
+template <typename T, bool DET>
 __global__ void dcn_gin_collect(const float *__restrict__ pbox, const float *__restrict__ gin_blk, T *__restrict__ gin,
                                 DcnDims d, BoxBwdPlan pl)
 {
     const int HW = d.H * d.W;
     const size_t n = (size_t)d.B * pl.units * HW;
     const int sy = TH * d.sh, sx = TW * d.sw;
+    const float inv = DET ? (det_bound_nonfinite(d) ? __uint_as_float(0x7FC00000u) : ldexpf(1.f, -det_scale_exp(d))) : 0.f;
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         const size_t bg = i / HW;
         const int px = (int)(i - bg * HW), b = (int)(bg / pl.units), g = (int)(bg - (size_t)b * pl.units);
         const int y = px / d.W, x = px - y * d.W;
-        const float4 *fp = reinterpret_cast<const float4 *>(gin_blk + i * CS);
-        float4 a0 = __ldg(fp), a1 = __ldg(fp + 1);
+        float4 a0, a1;
+        if constexpr (DET) {
+            const longlong2 *lp = reinterpret_cast<const longlong2 *>(gin_blk) + i * (CS / 2);
+            const longlong2 v0 = __ldg(lp), v1 = __ldg(lp + 1), v2 = __ldg(lp + 2), v3 = __ldg(lp + 3);
+            a0 = make_float4(__ll2float_rn(v0.x) * inv, __ll2float_rn(v0.y) * inv, __ll2float_rn(v1.x) * inv, __ll2float_rn(v1.y) * inv);
+            a1 = make_float4(__ll2float_rn(v2.x) * inv, __ll2float_rn(v2.y) * inv, __ll2float_rn(v3.x) * inv, __ll2float_rn(v3.y) * inv);
+        } else {
+            const float4 *fp = reinterpret_cast<const float4 *>(gin_blk + i * CS);
+            a0 = __ldg(fp); a1 = __ldg(fp + 1);
+        }
         // box of tile (ty, tx): rows [ty*sy - ph - my, +BH), pixels [tx*sx - ph - mx, +BW)   (pad_h for x too, :368)
         const int ny = y + d.ph + pl.my, nx = x + d.ph + pl.mx;
         const int ty_hi = min(pl.tiles_y - 1, ny / sy), tx_hi = min(pl.tiles_x - 1, nx / sx);
@@ -874,7 +920,7 @@ __global__ void dcn_gin_collect(const float *__restrict__ pbox, const float *__r
 // row alignment; with 2 (bf16 outputs) and several units per group the owners' fp32 running sums take the bytes saved.
 bool make_plan(const DcnDims &d, BoxBwdPlan &pl, int act_bytes = 4)
 {
-    if (d.cpg % CS != 0 || d.Co != CO || d.det) return false;
+    if (d.cpg % CS != 0 || d.Co != CO) return false;
     pl.units = d.C / CS;
     pl.ncs = d.cpg / CS;
     if (pl.ncs & (pl.ncs - 1)) return false;             // units per group: a power of two (1, 2, 4)
@@ -930,13 +976,15 @@ int backward_box_splits(const DcnDims &d)
     return 2 * box_splits(d, pl);
 }
 
-// scratch: blocked input | blocked far-sample accumulator | W^T images | dense partial boxes
+// scratch: blocked input | blocked far-sample accumulator (fp32, int64 under EBFI_DCN_DETERMINISTIC) | W^T images |
+// dense partial boxes
 size_t backward_box_scratch_bytes(const DcnDims &d)
 {
     BoxBwdPlan pl{};
     if (!make_plan(d, pl)) return 0;
     const size_t n = (size_t)d.B * d.C * d.H * d.W;
-    return 2 * n * sizeof(float) + ebfi::round_up((size_t)pl.units * pl.wt_bytes, (size_t)256) +
+    return n * sizeof(float) + n * (d.det ? sizeof(long long) : sizeof(float)) +
+           ebfi::round_up((size_t)pl.units * pl.wt_bytes, (size_t)256) +
            (size_t)d.B * pl.ntiles * pl.units * box::BYTES;
 }
 
@@ -948,15 +996,16 @@ int backward_box(cudaStream_t st, const DcnDims &d, const T *input, const float 
     BoxBwdPlan pl{};
     if (!make_plan(d, pl, (int)sizeof(T))) return EBFI_ERR_UNSUPPORTED;
     const size_t n = (size_t)d.B * d.C * d.H * d.W;
+    const size_t far_bytes = n * (d.det ? sizeof(long long) : sizeof(float));
     float *in_blk = static_cast<float *>(scratch), *gin_blk = in_blk + n;
-    unsigned char *wimg = reinterpret_cast<unsigned char *>(gin_blk + n);
+    unsigned char *wimg = reinterpret_cast<unsigned char *>(gin_blk) + far_bytes;
     float *pbox = reinterpret_cast<float *>(wimg + ebfi::round_up((size_t)pl.units * pl.wt_bytes, (size_t)256));
     const int BG = d.B * pl.units, HW = d.H * d.W;
     if (d.in_blocked) {
         // the caller kept the forward's blocked copy (EBFI_DCN_INPUT_BLOCKED): only the far-sample accumulator is cleared
         in_blk = const_cast<float *>(reinterpret_cast<const float *>(input));
-        EBFI_CUDA_OK(cudaMemsetAsync(gin_blk, 0, n * sizeof(float), st));
-    } else if (int rc = launch_nchw_to_blocked(st, input, in_blk, BG, HW, gin_blk, 2)) {
+        EBFI_CUDA_OK(cudaMemsetAsync(gin_blk, 0, far_bytes, st));
+    } else if (int rc = launch_nchw_to_blocked(st, input, in_blk, BG, HW, gin_blk, d.det ? 4 : 2)) {
         return rc;       // blocked copy of the input + zero fill of the far-sample accumulator in one pass
     }
     dcn_bwd_prep_weights<<<ceil_div(pl.units * pl.N1 * CO, 256), 256, 0, st>>>(weight, reinterpret_cast<unsigned short *>(wimg), d, pl);
@@ -980,18 +1029,25 @@ int backward_box(cudaStream_t st, const DcnDims &d, const T *input, const float 
         if (int rc = tma::encode_3d(tm_mask, mask, om_type, dims_m, str, box_m)) return rc;
     }
     dim3 grid(box_splits(d, pl), pl.NH);
-#define EBFI_BWD_BOX(P, M)                                                                                             \
+#define EBFI_BWD_BOX(P, M, D)                                                                                          \
     do {                                                                                                               \
-        EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_box_kernel<P, M, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
-        dcn_bwd_box_kernel<P, M, T><<<grid, NTHR, pl.smem, st>>>(in_blk, wimg, offset, mask, gout, gin_blk, pbox, goff, gmask, \
-                                                                 gw_part, gb_part, d, pl, tm_box, tm_off, tm_mask);    \
+        EBFI_CUDA_OK(cudaFuncSetAttribute(dcn_bwd_box_kernel<P, M, D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem)); \
+        dcn_bwd_box_kernel<P, M, D, T><<<grid, NTHR, pl.smem, st>>>(in_blk, wimg, offset, mask, gout, gin_blk, pbox, goff, gmask, \
+                                                                    gw_part, gb_part, d, pl, tm_box, tm_off, tm_mask); \
     } while (0)
-    if (pl.ncs > 1) { if (d.packed) EBFI_BWD_BOX(true, true); else EBFI_BWD_BOX(false, true); }
-    else            { if (d.packed) EBFI_BWD_BOX(true, false); else EBFI_BWD_BOX(false, false); }
+#define EBFI_BWD_BOX_PM(D)                                                                                             \
+    do {                                                                                                               \
+        if (pl.ncs > 1) { if (d.packed) EBFI_BWD_BOX(true, true, D); else EBFI_BWD_BOX(false, true, D); }             \
+        else            { if (d.packed) EBFI_BWD_BOX(true, false, D); else EBFI_BWD_BOX(false, false, D); }           \
+    } while (0)
+    if (d.det) EBFI_BWD_BOX_PM(true);
+    else       EBFI_BWD_BOX_PM(false);
+#undef EBFI_BWD_BOX_PM
 #undef EBFI_BWD_BOX
     EBFI_LAUNCH_OK("dcn_bwd_box_kernel");
     const unsigned cgrid = (unsigned)std::min<size_t>(ceil_div((size_t)BG * HW, (size_t)256), (size_t)ebfi::sm_count() * 16);
-    dcn_gin_collect<T><<<cgrid, 256, 0, st>>>(pbox, gin_blk, gin, d, pl);
+    if (d.det) dcn_gin_collect<T, true><<<cgrid, 256, 0, st>>>(pbox, gin_blk, gin, d, pl);
+    else       dcn_gin_collect<T, false><<<cgrid, 256, 0, st>>>(pbox, gin_blk, gin, d, pl);
     EBFI_LAUNCH_OK("dcn_gin_collect");
     const int Kdim = d.C * d.KK;
     const int rblocks = ceil_div(Kdim * CO + CO, 64);

@@ -26,8 +26,9 @@ struct DcnDims {
     int off_bp, mask_bp;      // the same batch strides in planes (off_bs / (Ho*Wo), ...), for TMA plane coordinates
     int packed;
     float *abs_sum;   // packed forward only, nullable: += sum |offset| (DCN_sep's `offset_mean` warning, :221-223)
-    // EBFI_DCN_DETERMINISTIC (backward): grad_input is accumulated as int64 fixed point. det_bound -> 3 device
-    // floats {max_px sum_co |gO|, max |weight|, max |mask|} whose product bounds every single contribution;
+    // EBFI_DCN_DETERMINISTIC (backward): grad_input is accumulated as int64 fixed point (by the box kernel: its far
+    // samples only). det_bound -> 3 device floats {max_px sum_co |gO|, max |weight|, max |mask|} whose product bounds
+    // every single contribution;
     // det_head = 62 - bits(max contributions per element): sums stay below 2^62 for scale = 2^(det_head - e),
     // bound < 2^e.
     int det, det_head;

@@ -8,8 +8,9 @@ Differences, all deliberate:
     grad_output) of one 16-bit type — all of them, or some with the rest fp32, as under torch.autocast — run in that
     type: fp32 activations are rounded to it once (autocast's own cast). weight / bias may then be fp32 or of that type
     and are used as fp32. Outputs and activation gradients have the 16-bit type, grad_weight / grad_bias the
-    parameter's dtype. The tensor-core kernels read and write the 16-bit activations directly; every other call (other
-    shapes, EBFI_DCN_DETERMINISTIC, EBFI_DCN_IMPL=simt, a misaligned grad_output) converts at this boundary
+    parameter's dtype. The tensor-core kernels read and write the 16-bit activations directly, the backward's box
+    kernel in the deterministic mode too; every other call (the CUDA-core kernels: other shapes or EBFI_DCN_IMPL=simt;
+    the deterministic backward of footprints beyond the box; a misaligned grad_output) converts at this boundary
     (_via_fp32) with the same result dtypes. Both give the bits of the fp32 kernels on the widened values, rounded
     once; an fp16 result beyond the fp16 range is inf, as tensor.half() gives. bf16 mixed with fp16 raises. With fp32
     activations everything must be fp32, as in the reference.
@@ -63,10 +64,10 @@ def _remember_blocked(lib, g, input, ws):
 
 def _blocked_input_ptr(g, input, grad_output):
     """Before a backward: the forward's blocked copy of this very tensor if it is still alive and this backward runs the
-    box kernel that reads it (sets the geometry flag), else the tensor itself. The box kernel needs a 16-byte aligned
-    grad_output and no EBFI_DCN_IMPL=simt, which may have changed since the forward."""
+    box kernel that reads it (sets the geometry flag), else the tensor itself. The box kernel runs in both modes; it
+    needs a 16-byte aligned grad_output and no EBFI_DCN_IMPL=simt, which may have changed since the forward."""
     hit = _blocked_cache.get(input.device.index)
-    if (hit is not None and not g.flags and hit[0] == _blocked_key(input, g)
+    if (hit is not None and g.flags in (0, L.EBFI_DCN_DETERMINISTIC) and hit[0] == _blocked_key(input, g)
             and hit[3] == torch.cuda.current_stream(input.device) and grad_output.data_ptr() % 16 == 0
             and L.load().ebfi_dcnv2_blocked_input_offset(g) == hit[2]):
         g.flags |= L.EBFI_DCN_INPUT_BLOCKED
@@ -123,7 +124,8 @@ def _via_fp32(dtype, fn, tensors, ints, out_dtypes=None):
     """16-bit activations at the boundary: the fp32 entry `fn` on exactly widened copies, results rounded once to
     `dtype` (or converted to `out_dtypes`, one per result). This is what a bf16 / fp16 call runs where the kernels have
     no native 16-bit I/O: the CUDA-core kernels (shapes outside the tensor-core ones, EBFI_DCN_IMPL=simt), the
-    deterministic backward, and a grad_output that is not 16-byte aligned. It costs extra elementwise passes, and the
+    deterministic backward where the box kernel does not run (dcn_bwd_tc.cu), and a grad_output that is not 16-byte
+    aligned. It costs extra elementwise passes, and the
     widened input is a new tensor, so a backward through here re-blocks it."""
     out = fn(*(t.float() for t in tensors), *ints)
     if torch.is_tensor(out):

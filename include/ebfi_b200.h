@@ -67,21 +67,25 @@ typedef struct ebfi_dcn_geom {
     int flags;                            /* 0, or EBFI_DCN_DETERMINISTIC (new; not in the reference's argument list) */
 } ebfi_dcn_geom;
 
-/* Backward only: accumulate grad_input in 64-bit fixed point in global memory (integer atomics are associative), so
- * that ALL five gradients are bit-reproducible run to run for ANY offsets. The reference's col2im uses float
+/* Backward only: ALL five gradients bit-reproducible run to run for ANY offsets. The reference's col2im uses float
  * atomicAdd (dcn_v2_im2col_cuda.cu:249) and is not. The DEFAULT mode (no flag) is already bit-reproducible on the
- * tensor-core path (8, 16 or 32 channels per deformable group, 64 outputs) for every sample whose four corners lie within ~7 pixels of its
- * tile's undeformed footprint: those accumulate in shared-memory fixed point and the per-tile boxes are summed in a
- * fixed order (csrc/dcn_bwd_box.cu); only samples beyond that use float red.global.add. This flag removes that last
- * order dependence (and covers the CUDA-core path) at ~3x the cost. The fixed-point scale is a power of two derived on
- * the device from max|grad_output|, max|weight| and max|mask| such that no sum can overflow; resolution is at least
- * 2^-20 of the largest possible single contribution. A non-finite gradient yields NaN (never a silent zero). */
+ * box kernel (csrc/dcn_bwd_box.cu: 8, 16 or 32 channels per deformable group, 64 outputs, a tile footprint that fits
+ * its box) for every sample whose four corners lie within ~7 pixels of its tile's undeformed footprint: those
+ * accumulate in shared-memory fixed point and the per-tile boxes are summed in a fixed order; only samples beyond
+ * that ("far" samples) use float red.global.add. With this flag the same box kernel runs, and its far samples add
+ * into a 64-bit fixed-point buffer instead (integer atomics are associative): one extra pass over grad_output for the
+ * scale, and the same bits as the default mode wherever no sample is far. Shapes the box kernel does not cover
+ * accumulate ALL of grad_input in 64-bit fixed point: csrc/dcn_bwd_tc.cu for 8 channels per group and 64 outputs
+ * (e.g. stride 2 in W), the CUDA-core kernel otherwise. The fixed-point scale, a power of two derived on the device
+ * from max|grad_output|, max|weight| and max|mask| such that no sum can overflow, applies to those 64-bit sums only
+ * (on the box kernel: the far samples); its resolution is at least 2^-20 of the largest possible single
+ * contribution. A non-finite gradient yields NaN (never a silent zero). */
 #define EBFI_DCN_DETERMINISTIC 1
 
 /* Backward only: `input` is not the NCHW tensor but its group-blocked copy [B][C/8][H][W][8 channels] (32-byte aligned)
  * that ebfi_dcnv2_forward left in its workspace at byte offset ebfi_dcnv2_blocked_input_offset(g) — a caller that keeps
  * the forward workspace alive until the backward (an autograd context) saves the re-blocking pass. Only valid when
- * that offset is non-zero and EBFI_DCN_DETERMINISTIC is not set. */
+ * that offset is non-zero (with or without EBFI_DCN_DETERMINISTIC). */
 #define EBFI_DCN_INPUT_BLOCKED 2
 
 /* Output spatial size, formula of dcn_v2_cuda.cu:64-65. Returns EBFI_ERR_INVALID
@@ -155,7 +159,8 @@ int ebfi_dcnv2_backward_packed(void *stream, const ebfi_dcn_geom *g,
  * bf16, and grad_weight / grad_bias are equal.
  * They run only where the tensor-core kernels run: the forward for Cout a multiple of 16 up to 128, channels per group
  * a multiple of 8 and up to 12 taps, with a workspace of ebfi_dcnv2_forward_workspace_bytes; the backward for
- * Cout == 64, 8 / 16 / 32 channels per group, no EBFI_DCN_DETERMINISTIC and a 16-byte aligned grad_output; neither
+ * Cout == 64, 8 / 16 / 32 channels per group, a tile footprint that fits the box and a 16-byte aligned grad_output, in
+ * both modes of EBFI_DCN_DETERMINISTIC (the bound of the deterministic scale is taken on the widened values); neither
  * under EBFI_DCN_IMPL=simt. Anything else returns EBFI_ERR_UNSUPPORTED before any work is enqueued: take the fp32 entry
  * on widened copies. ebfi_dcnv2_backward_dp_bf16 is declared with the data-parallel entries below. */
 int ebfi_dcnv2_forward_bf16(void *stream, const ebfi_dcn_geom *g,
