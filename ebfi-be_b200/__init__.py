@@ -12,13 +12,16 @@ sm_100a kernels in lib/libebfi_b200.so through the C ABI of include/ebfi_b200.h:
     ebfi_be_b200.shims         modules named `_ext` and `kernelconv2d_cuda`, so the reference's
                                own, unmodified wrappers import and run on these kernels
     ebfi_be_b200.parallel      batch sharding + weight-gradient all-reduce helpers
+    ebfi_be_b200.ops           the ops a model's forward and backward call, as torch custom operators
+                               (torch.ops.ebfi_b200.*) for torch.compile and torch.export
 
 There is no CPU fallback: every op raises if the CUDA library is missing or the tensors are
 not on a CUDA device.
 """
 from . import _lib  # noqa: F401
+from . import ops  # noqa: F401  (registers torch.ops.ebfi_b200.*, which the modules call under torch.compile)
 
-__all__ = ["_lib", "dcn_v2", "kernelconv2d", "encodings", "shims", "parallel", "install_shims"]
+__all__ = ["_lib", "ops", "dcn_v2", "kernelconv2d", "encodings", "shims", "parallel", "install_shims"]
 
 
 def install_shims():

@@ -206,7 +206,8 @@ class _OffsetWatch:
 
 class DCN_sep(_DCNWithOffsetConv):
     """Offsets and masks come from a second feature map `fea` (dcn_v2.py:197-227). `fused=False` runs
-    the reference's op sequence including its per-call host sync."""
+    the reference's op sequence including its per-call host sync. Under torch.compile the fused path does not
+    evaluate the `offset mean > 100` warning: its pinned copies and events are host work outside the graph."""
     fused = True
 
     def __init__(self, *args, **kwargs):
@@ -219,6 +220,9 @@ class DCN_sep(_DCNWithOffsetConv):
     def forward(self, input, fea):
         if self.fused and input.is_cuda:
             om = self.conv_offset_mask(fea)
+            if torch.compiler.is_compiling():
+                return dcn_v2_conv_packed(input, om, self.weight, self.bias, self.stride, self.padding,
+                                          self.dilation, self.deformable_groups)
             self._watch.poll()
             stat = torch.empty(1, dtype=torch.float32, device=input.device)
             out = dcn_v2_conv_packed(input, om, self.weight, self.bias, self.stride, self.padding,

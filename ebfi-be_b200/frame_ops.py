@@ -17,6 +17,8 @@ def _frames(ims):
 
 def Frame2DCP(ims, sz=35):
     """Dark-channel prior map: min over channels, then a sz x sz minimum filter (cv2.erode). Bx3xHxW -> Bx1xHxW."""
+    if torch.compiler.is_compiling():
+        return torch.ops.ebfi_b200.frame_to_dcp(ims, int(sz))
     x = _frames(ims)
     B, _, H, W = x.shape
     with torch.cuda.device(x.device):
@@ -29,6 +31,8 @@ def Frame2DCP(ims, sz=35):
 
 def Frame2Lap(ims):
     """Laplacian of the 8-bit gray image (cv2.cvtColor BGR2GRAY + cv2.Laplacian). Bx3xHxW in [0, 1] -> Bx1xHxW."""
+    if torch.compiler.is_compiling():
+        return torch.ops.ebfi_b200.frame_to_lap(ims)
     x = _frames(ims)
     B, _, H, W = x.shape
     with torch.cuda.device(x.device):

@@ -12,6 +12,8 @@ input is written, saved or read, and the backward sums the pad's gradient in a f
 CUDA pad backward accumulates with atomics and raises under torch.use_deterministic_algorithms(True)), so the
 module trains bit-reproducibly, with or without that switch.
 """
+import contextlib
+
 import torch
 from torch import nn
 from torch.autograd import Function
@@ -19,6 +21,12 @@ from torch.autograd import Function
 from . import _lib as L
 from .shims import kernelconv2d_cuda
 from .shims.kernelconv2d_cuda import _SUFFIX
+
+
+def _device_of(t):
+    """torch.cuda.device_of(t). Dynamo cannot trace that context; under torch.compile the ops take the device from
+    their tensors."""
+    return contextlib.nullcontext() if torch.compiler.is_compiling() else torch.cuda.device_of(t)
 
 
 class KernelConv2DFunction(Function):
@@ -33,7 +41,7 @@ class KernelConv2DFunction(Function):
             raise NotImplementedError()      # CPU VERSION NOT IMPLEMENTED (KernelConv2D.py:38-39)
         ctx.kernel_size = kernel_size
         ctx.save_for_backward(input, kernel)
-        with torch.cuda.device_of(input):
+        with _device_of(input):
             output = torch.empty((input.size(0), input.size(1), kernel.size(2), kernel.size(3)),
                                  dtype=input.dtype, device=input.device)
             kernelconv2d_cuda.forward(input, kernel, kernel_size, output)
@@ -45,7 +53,7 @@ class KernelConv2DFunction(Function):
         grad_output = grad_output.contiguous()
         if not grad_output.is_cuda:
             raise NotImplementedError()      # KernelConv2D.py:55-56
-        with torch.cuda.device_of(input):
+        with _device_of(input):
             grad_input, grad_kernel = torch.empty_like(input), torch.empty_like(kernel)
             kernelconv2d_cuda.backward(input, kernel, ctx.kernel_size, grad_output, grad_input, grad_kernel)
         return grad_input, grad_kernel, None
@@ -63,6 +71,43 @@ def _replpad_dims(input, kernel, kernel_size):
     return (*input.shape, K)
 
 
+def _replpad_forward(input, kernel, kernel_size):
+    """ebfi_fac_replpad_forward on CUDA tensors: FAC of ReplicationPad2d((K-1)/2)(input) with `kernel`."""
+    input, kernel = input.contiguous(), kernel.contiguous()
+    B, C, H, W, K = _replpad_dims(input, kernel, kernel_size)
+    lib = L.load()
+    with torch.cuda.device_of(input):
+        output = torch.empty((B, C, H, W), dtype=input.dtype, device=input.device)
+        fn = getattr(lib, "ebfi_fac_replpad_forward" + _SUFFIX[input.dtype])
+        L.check(fn(L.stream_ptr(input.device), L.ptr(input), L.ptr(kernel), L.ptr(output), B, C, H, W, K),
+                "ebfi_fac_replpad_forward")
+    return output
+
+
+def _check_replpad_grad(input, grad_output):
+    if grad_output.dtype != input.dtype:
+        raise RuntimeError(f"KernelConv2D: grad_output is {grad_output.dtype}, the input {input.dtype}")
+    if grad_output.shape != input.shape:
+        raise RuntimeError(f"KernelConv2D: grad_output is {tuple(grad_output.shape)}, the input {tuple(input.shape)}")
+
+
+def _replpad_backward(input, kernel, kernel_size, grad_output):
+    """ebfi_fac_replpad_backward on CUDA tensors -> (grad_input, grad_kernel) of _replpad_forward."""
+    grad_output = grad_output.contiguous()
+    _check_replpad_grad(input, grad_output)
+    B, C, H, W, K = _replpad_dims(input, kernel, kernel_size)
+    lib = L.load()
+    with torch.cuda.device_of(input):
+        grad_input, grad_kernel = torch.empty_like(input), torch.empty_like(kernel)
+        nbytes = lib.ebfi_fac_backward_workspace_bytes(B, C, H, W, K)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
+        fn = getattr(lib, "ebfi_fac_replpad_backward" + _SUFFIX[input.dtype])
+        L.check(fn(L.stream_ptr(input.device), L.ptr(input), L.ptr(kernel), L.ptr(grad_output),
+                   L.ptr(grad_input), L.ptr(grad_kernel), B, C, H, W, K, L.ptr(ws), nbytes),
+                "ebfi_fac_replpad_backward")
+    return grad_input, grad_kernel
+
+
 class KernelConv2DReplPadFunction(Function):
     """ReplicationPad2d((K-1)/2)(input) followed by KernelConv2DFunction, with the pad folded into the kernels:
     input (B, C, H, W), kernel (B, C*K*K, H, W). Saves only input and kernel. Forward and grad_kernel are
@@ -73,35 +118,22 @@ class KernelConv2DReplPadFunction(Function):
         if not (input.is_cuda and kernel.is_cuda):
             raise NotImplementedError()      # CPU VERSION NOT IMPLEMENTED (KernelConv2D.py:38-39)
         input, kernel = input.contiguous(), kernel.contiguous()
-        B, C, H, W, K = _replpad_dims(input, kernel, kernel_size)
-        ctx.kernel_size = K
+        ctx.kernel_size = int(kernel_size)
         ctx.save_for_backward(input, kernel)
-        lib = L.load()
-        with torch.cuda.device_of(input):
-            output = torch.empty((B, C, H, W), dtype=input.dtype, device=input.device)
-            fn = getattr(lib, "ebfi_fac_replpad_forward" + _SUFFIX[input.dtype])
-            L.check(fn(L.stream_ptr(input.device), L.ptr(input), L.ptr(kernel), L.ptr(output), B, C, H, W, K),
-                    "ebfi_fac_replpad_forward")
-        return output
+        if torch.compiler.is_compiling():
+            return torch.ops.ebfi_b200.fac_replpad_forward(input, kernel, ctx.kernel_size)
+        return _replpad_forward(input, kernel, ctx.kernel_size)
 
     @staticmethod
     def backward(ctx, grad_output):
         input, kernel = ctx.saved_tensors
         if not grad_output.is_cuda:
             raise NotImplementedError()      # KernelConv2D.py:55-56
-        grad_output = grad_output.contiguous()
-        if grad_output.dtype != input.dtype:
-            raise RuntimeError(f"KernelConv2D: grad_output is {grad_output.dtype}, the input {input.dtype}")
-        B, C, H, W, K = _replpad_dims(input, kernel, ctx.kernel_size)
-        lib = L.load()
-        with torch.cuda.device_of(input):
-            grad_input, grad_kernel = torch.empty_like(input), torch.empty_like(kernel)
-            nbytes = lib.ebfi_fac_backward_workspace_bytes(B, C, H, W, K)
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
-            fn = getattr(lib, "ebfi_fac_replpad_backward" + _SUFFIX[input.dtype])
-            L.check(fn(L.stream_ptr(input.device), L.ptr(input), L.ptr(kernel), L.ptr(grad_output),
-                       L.ptr(grad_input), L.ptr(grad_kernel), B, C, H, W, K, L.ptr(ws), nbytes),
-                    "ebfi_fac_replpad_backward")
+        if torch.compiler.is_compiling():
+            grad_input, grad_kernel = torch.ops.ebfi_b200.fac_replpad_backward(input, kernel, ctx.kernel_size,
+                                                                                grad_output)
+        else:
+            grad_input, grad_kernel = _replpad_backward(input, kernel, ctx.kernel_size, grad_output)
         return grad_input, grad_kernel, None
 
 

@@ -55,6 +55,9 @@ def _fused_forward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, 
     """ebfi_kpn_fused_forward (fp32 activations) or its _bf16 / _fp16 variant (16-bit activations) on CUDA tensors
     with fp32 weight and bias: the one forward of kernelconv_fac_fused, KernelConvFACFunction and
     KernelConvFACBF16Function. The output has the activations' dtype."""
+    if torch.compiler.is_compiling():
+        return torch.ops.ebfi_b200.kpn_fused_forward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size,
+                                                     negative_slope)
     B, Ce, Cf, H, W, K = _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, "kernelconv_fac_fused")
     event_feat, frame_feat, conv_weight, conv_bias = (t.contiguous() for t in (event_feat, frame_feat, conv_weight, conv_bias))
     lib = L.load()
@@ -111,6 +114,9 @@ def _require_half_io(what, activations, parameters):
 
 def _fused_backward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, negative_slope, grad_output, what):
     """ebfi_kpn_fused_backward or its _bf16 / _fp16 variant, chosen by the activations' dtype; fp32 weight and bias."""
+    if torch.compiler.is_compiling():
+        return torch.ops.ebfi_b200.kpn_fused_backward(event_feat, frame_feat, conv_weight, conv_bias, kernel_size,
+                                                      negative_slope, grad_output)
     B, Ce, Cf, H, W, K = _block_dims(event_feat, frame_feat, conv_weight, conv_bias, kernel_size, what)
     if tuple(grad_output.shape) != tuple(event_feat.shape):
         raise RuntimeError(f"{what}: grad_output must have the event features' shape")

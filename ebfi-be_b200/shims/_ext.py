@@ -52,8 +52,10 @@ def _blocked_key(input, g):
             g.pad_h, g.pad_w, g.dilation_h, g.dilation_w, g.deformable_group)
 
 
-def _remember_blocked(lib, g, input, ws):
+def _remember_blocked(lib, g, input, ws, reuse_blocked):
     """After a forward: note where its workspace holds the group-blocked copy of `input`."""
+    if not reuse_blocked:
+        return
     off_blk = lib.ebfi_dcnv2_blocked_input_offset(g)
     if off_blk and os.environ.get("EBFI_DCN_NO_BLOCKED_REUSE") != "1":
         # keeps `ws` alive until the next forward on this device; the stream that runs the backward is the one that
@@ -62,11 +64,11 @@ def _remember_blocked(lib, g, input, ws):
                                               input.untyped_storage())
 
 
-def _blocked_input_ptr(g, input, grad_output):
+def _blocked_input_ptr(g, input, grad_output, reuse_blocked):
     """Before a backward: the forward's blocked copy of this very tensor if it is still alive and this backward runs the
     box kernel that reads it (sets the geometry flag), else the tensor itself. The box kernel runs in both modes; it
     needs a 16-byte aligned grad_output and no EBFI_DCN_IMPL=simt, which may have changed since the forward."""
-    hit = _blocked_cache.get(input.device.index)
+    hit = _blocked_cache.get(input.device.index) if reuse_blocked else None
     if (hit is not None and g.flags in (0, L.EBFI_DCN_DETERMINISTIC) and hit[0] == _blocked_key(input, g)
             and hit[3] == torch.cuda.current_stream(input.device) and grad_output.data_ptr() % 16 == 0
             and L.load().ebfi_dcnv2_blocked_input_offset(g) == hit[2]):
@@ -75,11 +77,10 @@ def _blocked_input_ptr(g, input, grad_output):
     return L.ptr(input)
 
 
-def _geom(input, weight, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
-          dilation_h, dilation_w, deformable_group, flags=0):
+def _check_weight(input, weight, kernel_h, kernel_w):
     if input.dim() != 4 or weight.dim() != 4:
         raise RuntimeError("dcn_v2: input and weight must be 4-D")
-    channels_out, channels_kernel, kh_, kw_ = weight.shape
+    _, channels_kernel, kh_, kw_ = weight.shape
     # same two shape checks as dcn_v2_cuda.cu:58-62
     if kh_ != kernel_h or kw_ != kernel_w:
         raise RuntimeError("Input shape and kernel shape wont match: (%d x %d vs %d x %d)."
@@ -87,7 +88,12 @@ def _geom(input, weight, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
     if input.shape[1] != channels_kernel:
         raise RuntimeError("Input shape and kernel channels wont match: (%d vs %d)."
                            % (input.shape[1], channels_kernel))
-    g = L.DcnGeom(input.shape[0], input.shape[1], input.shape[2], input.shape[3], channels_out,
+
+
+def _geom(input, weight, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+          dilation_h, dilation_w, deformable_group, flags=0):
+    _check_weight(input, weight, kernel_h, kernel_w)
+    g = L.DcnGeom(input.shape[0], input.shape[1], input.shape[2], input.shape[3], weight.shape[0],
                   kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
                   deformable_group, flags)
     ho, wo = L.c_int(), L.c_int()
@@ -154,8 +160,12 @@ def _check_offset_mask(g, ho, wo, offset, mask):
 
 
 def dcn_v2_forward(input, weight, bias, offset, mask, kernel_h, kernel_w, stride_h, stride_w,
-                   pad_h, pad_w, dilation_h, dilation_w, deformable_group):
-    """dcn_v2_cuda_forward (src/cuda/dcn_v2_cuda.cu:20-95). Returns a new (B, Cout, Ho, Wo) tensor."""
+                   pad_h, pad_w, dilation_h, dilation_w, deformable_group, *, reuse_blocked=True):
+    """dcn_v2_cuda_forward (src/cuda/dcn_v2_cuda.cu:20-95). Returns a new (B, Cout, Ho, Wo) tensor.
+    reuse_blocked=False: leave the blocked copy of `input` to no later backward (what torch.ops.ebfi_b200 runs)."""
+    if torch.compiler.is_compiling():
+        return torch.ops.ebfi_b200.dcn_v2_forward(input, weight, bias, offset, mask, kernel_h, kernel_w, stride_h,
+                                                  stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group)
     dt = _check_cuda(input=input, weight=weight, bias=bias, offset=offset, mask=mask)
     half = _HALF.get(dt)
     ints = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group)
@@ -175,18 +185,26 @@ def dcn_v2_forward(input, weight, bias, offset, mask, kernel_h, kernel_w, stride
         if not half:
             L.check(lib.ebfi_dcnv2_forward(*args), "dcn_v2_forward")
         elif not _ran_native(getattr(lib, "ebfi_dcnv2_forward" + half)(*args), "dcn_v2_forward" + half):
-            return _via_fp32(dt, dcn_v2_forward, (input, weight, bias, offset, mask), ints)
-        _remember_blocked(lib, g, input, ws)
+            return _via_fp32(dt, functools.partial(dcn_v2_forward, reuse_blocked=reuse_blocked),
+                             (input, weight, bias, offset, mask), ints)
+        _remember_blocked(lib, g, input, ws, reuse_blocked)
     return output
 
 
 def dcn_v2_backward(input, weight, bias, offset, mask, grad_output, kernel_h, kernel_w, stride_h,
-                    stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group, comm=None, defer=False):
+                    stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group, comm=None, defer=False, *,
+                    reuse_blocked=True):
     """dcn_v2_cuda_backward (dcn_v2_cuda.cu:97-216).
     Returns [grad_input, grad_offset, grad_mask, grad_weight, grad_bias].
     comm (new, optional): a parallel.GradComm — grad_weight / grad_bias then come back summed over its ranks, the
     exchange fused into the kernel that reduces them (ebfi_dcnv2_backward_dp). defer=True: the kernel only publishes
-    this rank's sums; `comm.complete(grad_weight, grad_bias)` finishes the exchange where the sums are needed."""
+    this rank's sums; `comm.complete(grad_weight, grad_bias)` finishes the exchange where the sums are needed. A call
+    with `comm` runs eagerly only (a graph break under torch.compile).
+    reuse_blocked=False: re-block `input` rather than read a forward's blocked copy (what torch.ops.ebfi_b200 runs)."""
+    if comm is None and torch.compiler.is_compiling():
+        return list(torch.ops.ebfi_b200.dcn_v2_backward(input, weight, bias, offset, mask, grad_output, kernel_h,
+                                                        kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                                                        dilation_w, deformable_group))
     # THArgCheck(input.is_contiguous()) / (weight.is_contiguous()), dcn_v2_cuda.cu:110-111
     if not input.is_contiguous():
         raise RuntimeError("input tensor has to be contiguous")
@@ -209,7 +227,7 @@ def dcn_v2_backward(input, weight, bias, offset, mask, grad_output, kernel_h, ke
         grads = [torch.empty_like(t) for t in (input, offset, mask, weight, bias)]
         nbytes = lib.ebfi_dcnv2_backward_workspace_bytes(g)
         ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
-        in_ptr = _blocked_input_ptr(g, input, grad_output)
+        in_ptr = _blocked_input_ptr(g, input, grad_output, reuse_blocked)
         args = (L.stream_ptr(input.device), g, in_ptr, L.ptr(weight), L.ptr(bias), L.ptr(offset), L.ptr(mask),
                 L.ptr(grad_output), *(L.ptr(t) for t in grads), L.ptr(ws), nbytes)
         if not half:
@@ -225,8 +243,8 @@ def dcn_v2_backward(input, weight, bias, offset, mask, grad_output, kernel_h, ke
                               "dcn_v2_backward_dp" + half)
     out_dtypes = [dt] * 3 + param_dtypes
     if not ran:
-        return _via_fp32(dt, dcn_v2_backward, (input, weight, bias, offset, mask, grad_output), ints + (comm, defer),
-                         out_dtypes)
+        return _via_fp32(dt, functools.partial(dcn_v2_backward, reuse_blocked=reuse_blocked),
+                         (input, weight, bias, offset, mask, grad_output), ints + (comm, defer), out_dtypes)
     return [t.to(dt) for t, dt in zip(grads, out_dtypes)]
 
 
@@ -245,11 +263,19 @@ def _check_packed(g, ho, wo, offset_mask):
 
 
 def dcn_v2_forward_packed(input, weight, bias, offset_mask, kernel_h, kernel_w, stride_h, stride_w,
-                          pad_h, pad_w, dilation_h, dilation_w, deformable_group, abs_offset_sum=None):
+                          pad_h, pad_w, dilation_h, dilation_w, deformable_group, abs_offset_sum=None, *,
+                          reuse_blocked=True):
     """NEW (no reference counterpart in `_ext`): dcn_v2_forward fed with the raw `conv_offset_mask`
     output, i.e. chunk / cat / sigmoid of DCN.forward / DCN_sep.forward (dcn_v2.py:179-187, :217-227)
     folded into the kernel. `abs_offset_sum`: optional 1-element fp32 CUDA tensor that receives
-    sum |offset| (for the `offset_mean > 100` warning, :221-223)."""
+    sum |offset| (for the `offset_mean > 100` warning, :221-223). reuse_blocked as in dcn_v2_forward."""
+    if torch.compiler.is_compiling():
+        # inductor (torch 2.11) fails to lower the op with its optional written argument left None: pass a scratch sum
+        if abs_offset_sum is None:
+            abs_offset_sum = torch.empty(1, dtype=torch.float32, device=input.device)
+        return torch.ops.ebfi_b200.dcn_v2_forward_packed(input, weight, bias, offset_mask, kernel_h, kernel_w,
+                                                         stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                                                         deformable_group, abs_offset_sum)
     dt = _check_cuda(input=input, weight=weight, bias=bias, offset_mask=offset_mask)
     half = _HALF.get(dt)
     ints = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group)
@@ -272,15 +298,21 @@ def dcn_v2_forward_packed(input, weight, bias, offset_mask, kernel_h, kernel_w, 
         if not half:
             L.check(lib.ebfi_dcnv2_forward_packed(*args), "dcn_v2_forward_packed")
         elif not _ran_native(getattr(lib, "ebfi_dcnv2_forward_packed" + half)(*args), "dcn_v2_forward_packed" + half):
-            return _via_fp32(dt, dcn_v2_forward_packed, (input, weight, bias, offset_mask), ints + (abs_offset_sum,))
-        _remember_blocked(lib, g, input, ws)
+            return _via_fp32(dt, functools.partial(dcn_v2_forward_packed, reuse_blocked=reuse_blocked),
+                             (input, weight, bias, offset_mask), ints + (abs_offset_sum,))
+        _remember_blocked(lib, g, input, ws, reuse_blocked)
     return output
 
 
 def dcn_v2_backward_packed(input, weight, bias, offset_mask, grad_output, kernel_h, kernel_w, stride_h,
-                           stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group):
+                           stride_w, pad_h, pad_w, dilation_h, dilation_w, deformable_group, *, reuse_blocked=True):
     """Backward of dcn_v2_forward_packed. Returns [grad_input, grad_offset_mask, grad_weight, grad_bias];
-    grad_offset_mask has the layout of offset_mask, its last third already multiplied by sigmoid'."""
+    grad_offset_mask has the layout of offset_mask, its last third already multiplied by sigmoid'.
+    reuse_blocked as in dcn_v2_backward."""
+    if torch.compiler.is_compiling():
+        return list(torch.ops.ebfi_b200.dcn_v2_backward_packed(input, weight, bias, offset_mask, grad_output,
+                                                               kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w,
+                                                               dilation_h, dilation_w, deformable_group))
     if not input.is_contiguous():
         raise RuntimeError("input tensor has to be contiguous")
     if not weight.is_contiguous():
@@ -302,7 +334,7 @@ def dcn_v2_backward_packed(input, weight, bias, offset_mask, grad_output, kernel
         grads = [torch.empty_like(t) for t in (input, offset_mask, weight, bias)]
         nbytes = lib.ebfi_dcnv2_backward_workspace_bytes(g)
         ws = torch.empty(nbytes, dtype=torch.uint8, device=input.device)
-        in_ptr = _blocked_input_ptr(g, input, grad_output)
+        in_ptr = _blocked_input_ptr(g, input, grad_output, reuse_blocked)
         args = (L.stream_ptr(input.device), g, in_ptr, L.ptr(weight), L.ptr(bias), L.ptr(offset_mask),
                 L.ptr(grad_output), *(L.ptr(t) for t in grads), L.ptr(ws), nbytes)
         if not half:
@@ -311,7 +343,8 @@ def dcn_v2_backward_packed(input, weight, bias, offset_mask, grad_output, kernel
         ran = _ran_native(getattr(lib, "ebfi_dcnv2_backward_packed" + half)(*args), "dcn_v2_backward_packed" + half)
     out_dtypes = [dt] * 2 + param_dtypes
     if not ran:
-        return _via_fp32(dt, dcn_v2_backward_packed, (input, weight, bias, offset_mask, grad_output), ints, out_dtypes)
+        return _via_fp32(dt, functools.partial(dcn_v2_backward_packed, reuse_blocked=reuse_blocked),
+                         (input, weight, bias, offset_mask, grad_output), ints, out_dtypes)
     return [t.to(dt) for t, dt in zip(grads, out_dtypes)]
 
 

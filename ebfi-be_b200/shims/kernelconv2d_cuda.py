@@ -4,7 +4,8 @@
 forward(input, kernel, kernel_size, output) -> 1 and
 backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel) -> 1 write into the
 caller-allocated tensors like the reference; a failing launch raises RuntimeError (the
-reference's AT_ERROR("CUDA call failed"), KernelConv2D_cuda.cpp:26-28).
+reference's AT_ERROR("CUDA call failed"), KernelConv2D_cuda.cpp:26-28). Under torch.compile they run as
+torch.ops.ebfi_b200.fac_forward / fac_backward, which declare those writes.
 """
 import torch
 
@@ -39,10 +40,18 @@ def _dims(input, kernel, kernel_size, what):
     return B, C, H, W, K
 
 
-def forward(input, kernel, kernel_size, output):
+def _check_forward(input, kernel, kernel_size, output):
     B, C, H, W, K = _dims(input, kernel, kernel_size, "kernelconv2d_cuda.forward")
     if tuple(output.shape) != (B, C, H, W) or not output.is_contiguous() or output.dtype != input.dtype:
         raise RuntimeError("kernelconv2d_cuda.forward: output must be a contiguous (B, C, H, W) tensor of the input dtype")
+    return B, C, H, W, K
+
+
+def forward(input, kernel, kernel_size, output):
+    if torch.compiler.is_compiling():
+        torch.ops.ebfi_b200.fac_forward(input, kernel, kernel_size, output)
+        return 1
+    B, C, H, W, K = _check_forward(input, kernel, kernel_size, output)
     lib = L.load()
     fn = getattr(lib, "ebfi_fac_forward" + _SUFFIX[input.dtype])
     with torch.cuda.device(input.device):
@@ -50,7 +59,7 @@ def forward(input, kernel, kernel_size, output):
     return 1
 
 
-def backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel):
+def _check_backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel):
     B, C, H, W, K = _dims(input, kernel, kernel_size, "kernelconv2d_cuda.backward")
     L.require_cuda(grad_output, grad_input, grad_kernel)
     if tuple(grad_output.shape) != (B, C, H, W) or not grad_output.is_contiguous() or grad_output.dtype != input.dtype:
@@ -60,6 +69,14 @@ def backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel):
     if grad_input.shape != input.shape or grad_kernel.shape != kernel.shape or \
             not grad_input.is_contiguous() or not grad_kernel.is_contiguous():
         raise RuntimeError("kernelconv2d_cuda.backward: grad_input / grad_kernel must match input / kernel")
+    return B, C, H, W, K
+
+
+def backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel):
+    if torch.compiler.is_compiling():
+        torch.ops.ebfi_b200.fac_backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel)
+        return 1
+    B, C, H, W, K = _check_backward(input, kernel, kernel_size, grad_output, grad_input, grad_kernel)
     lib = L.load()
     with torch.cuda.device(input.device):
         nbytes = lib.ebfi_fac_backward_workspace_bytes(B, C, H, W, K)
